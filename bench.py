@@ -5,6 +5,7 @@ raw scramble throughput, 2^24 cubes x 100 random moves, 20x24 representation, pe
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
   python bench.py --impl reference --gpus N ...            # the reference's numpy algorithm on the host cores
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's states to DIR/states.npy
 
 One JSON line on stdout (rank 0).  A "step" is one pass of the scramble kernel over the whole batch of
 host-supplied action sequences already resident in HBM (`value`), and the same pass through the host-buffer C-ABI
@@ -31,6 +32,7 @@ BYTES_PER_CUBE = DEPTH + 20          # uint8 actions in + int8[20] state out (SU
 # ncu --set full capture of the shipped scramble kernel (one 2^24-cube launch), summarised by tools/ncu_summary.py: bench.py reads
 # `roofline.traffic` (dram read + write) and the limiter percentages from this file at run time.
 NCU_SUMMARY = os.path.join(ROOT, "profiles", "r2_scramble_macro3_ncu.json")
+DUMP_ROWS = 1 << 19          # --dump-outputs: a fixed sample of the final states (2^19 x 20 float32 = 40 MB)
 METRIC, UNIT = "cube_moves_per_sec", "moves/s"
 WORKLOAD = "raw scramble: 2^24 cubes x 100 random moves per GPU, 20x24 rep, packed int8 (BASELINE configs[1])"
 
@@ -276,6 +278,13 @@ def run_gpu(args):
 			ev[k + 1].record()
 		barrier()
 	launches = N.lib.rb_launch_count() - launches0
+	if args.dump_outputs and rank == 0:
+		# the states the last timed step returned (`out` is reused further down): the same seeded rows on every run, so that two
+		# builds can be compared output for output
+		rows = np.sort(np.random.RandomState(0).choice(n, min(n, DUMP_ROWS), replace=False))
+		states = out[torch.from_numpy(rows).to(dev)].cpu().numpy().astype(np.float32)
+		os.makedirs(args.dump_outputs, exist_ok=True)
+		np.save(os.path.join(args.dump_outputs, "states.npy"), states)
 	ms_total = ev[0].elapsed_time(ev[-1])
 	per_launch_ms = [ev[k].elapsed_time(ev[k + 1]) for k in range(args.steps)]
 	t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
@@ -461,7 +470,14 @@ def main():
 	ap.add_argument("--warmup", type=int, default=3)
 	ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
 	ap.add_argument("--cubes", type=int, default=N_CUBES, help="cubes per GPU (default 2^24, the BASELINE size)")
+	ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+					help="after the timed steps, write the int8[20] states of the last step as float32 to DIR/states.npy: "
+						 f"rank 0's cubes, at most {DUMP_ROWS} rows drawn with a fixed seed, in cube order")
 	args = ap.parse_args()
+	if args.steps < 1:
+		ap.error("--steps must be at least 1")
+	if args.dump_outputs and args.impl == "reference":
+		ap.error("--dump-outputs applies to the CUDA arm (--impl b200)")
 	if args.impl == "reference":
 		run_reference(args)
 		return
@@ -471,6 +487,8 @@ def main():
 		cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}", "--master-addr", "127.0.0.1",
 			   "--master-port", os.environ.get("MASTER_PORT", "29531"), os.path.abspath(__file__), "--gpus", str(args.gpus),
 			   "--steps", str(args.steps), "--warmup", str(args.warmup), "--cubes", str(args.cubes)]
+		if args.dump_outputs:
+			cmd += ["--dump-outputs", os.path.abspath(args.dump_outputs)]
 		sys.exit(subprocess.call(cmd))
 	run_gpu(args)
 
