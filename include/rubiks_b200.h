@@ -66,6 +66,11 @@ int rb_get_perm686(uint8_t* perm);
 int rb_get_macro_table(uint32_t* rows);
 /* The fused 3-move table of the same kernel's 3-moves-per-row variant: uint32[12*12*12][5], row index a0 + 12 a1 + 144 a2. */
 int rb_get_macro3_table(uint32_t* rows);
+/* The deduplicated form of that table the kernel stages in shared memory: elems uint32[1080][4], the distinct 16-byte parts
+ * (selector words) of the rows; remap uint32[2372][2] = {twist|flip word, element index}.  remap index a0 + 12 a1 + 144 a2
+ * (4-bit actions, up to 2355) stands for the row of the INVERSE moves (a0 ^ 1, a1 ^ 1, a2 ^ 1), invalid indices for element 0
+ * with no twist or flip; index 2356 + a (a < 16) for the single inverse move a ^ 1 (a >= 12: element 0 again). */
+int rb_get_macro3_dedup(uint32_t* elems, uint32_t* remap);
 /* Sticker view used to render a 6x8x6 state from the 20x24 state of the same move sequence (fast 6x8x6 scramble):
  * corner_home uint8[8][3], corner_dst uint8[8][24][3], edge_home uint8[12][2], edge_dst uint8[12][24][2]: sticker k of a
  * cubie sits in 6x8x6 slot *_home[c][k] when solved and in slot *_dst[c][v][k] when the cubie's 20x24 value is v.

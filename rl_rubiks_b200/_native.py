@@ -33,6 +33,7 @@ SIGNATURES = {
 	"rb_get_perm686": (C.c_int, [_p]),
 	"rb_get_macro_table": (C.c_int, [_p]),
 	"rb_get_macro3_table": (C.c_int, [_p]),
+	"rb_get_macro3_dedup": (C.c_int, [_p, _p]),
 	"rb_get_stickers686": (C.c_int, [_p, _p, _p, _p]),
 	"rb_get_solved": (C.c_int, [C.c_int, _p]),
 	"rb_multi_rotate": (C.c_int, [C.c_int, _p, _p, _p, _p, _i64, _p]),

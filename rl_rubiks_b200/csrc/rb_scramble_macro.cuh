@@ -10,9 +10,10 @@
 // Permutation + additive orientation is closed under composition, so k consecutive moves are fused into one table row of
 // five words: corner selectors, three edge selector words and one word carrying the 8 twist increments and 12 flip bits.
 //
-//   k_scramble_macro3 (the one that runs for depth <= 400): rows of THREE moves (12^3), four copies of the 16-byte part,
-//     the product taken backwards (inverse moves, reverse order) so that the registers end up cubie-major -- see the
-//     comments at the kernel.  0.83 ms for 2^24 x 100 moves, at the shared-memory bound of this table design.
+//   k_scramble_macro3 (the one that runs for depth <= 400): rows of THREE moves (12^3), the product taken backwards (inverse
+//     moves, reverse order) so that the registers end up cubie-major -- see the comments at the kernel.  Up to depth 195 the
+//     table is deduplicated to its 1080 distinct elements in 8 conflict-free copies (0.757 ms for 2^24 x 100 moves), for
+//     longer sequences it is the 1728 rows in four copies of the 16-byte part (0.82 ms at depth 100).
 //   k_scramble_macro (fallback for longer sequences): rows of TWO moves (13^2 with identity padding), the table replicated
 //     so that every fetch is bank-conflict free (64 KB), forward product, scatter to cubie-major at the end.
 //
@@ -28,6 +29,8 @@
 #include "rb_tables.cuh"
 #include <cuda.h>              // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint)
 #include <stdlib.h>
+#include <array>
+#include <map>
 
 namespace rbs {
 
@@ -115,11 +118,28 @@ static void encode(const Elem& e, uint32_t* row) {
 
 constexpr int kRows3 = 12 * 12 * 12;            // 3-move rows, index a0 + 12 a1 + 144 a2 (no identity padding: the tail uses the 2-move table)
 
+// Deduplicated 3-move table (k_scramble_macro3 for depths up to 195, see launch()): a row is a function of the group element its three moves
+// multiply to, and the 1728 sequences give only 1080 elements (1068 at distance 3, plus the 12 single moves: x x x = x^-1).
+// The 16-byte part of each element is stored once per lane of a quarter-warp phase (8 copies, [element][copy], copy = lane % 8:
+// conflict-free LDS.128); a remap indexed like g_macro3 gives {twist|flip word, element}.  Entries past the 1728 valid indices
+// (4-bit masked invalid actions, up to kIdxMax3) point at element 0 with no twist or flip; entries kSingle3 + a (a = 0..15, the
+// raw action masked to 4 bits) are the single inverse move a ^ 1 for the depth % 3 tail (a >= 12: element 0 again).
+constexpr int kElems3 = 1080;
+constexpr int kRepDedup = 8;
+constexpr int kSingle3 = 15 + 12 * 15 + 144 * 15 + 1;          // 2356 = kIdxMax3 + 1
+constexpr int kRemap3 = kSingle3 + 16;                          // 2372
+constexpr int kElemBytes3 = kElems3 * kRepDedup * 16;           // 138,240
+constexpr int kImageBytes3 = kElemBytes3 + kRemap3 * 8;          // 157,216: staged with one bulk copy (multiple of 16)
+__device__ __align__(16) uint32_t g_macro3_image[kImageBytes3 / 4];       // Host::image3
+
 struct Host {
 	uint32_t rows[kRows * kRowWords + 3];
 	uint32_t rows3[kRows3 * kRowWords + 3];
 	uint32_t rows3_inv[kRows3 * kRowWords + 3];          // rows3 re-indexed by the inverse actions (device layout of g_macro3)
 	uint32_t rows_inv[kRows * kRowWords + 3];             // rows re-indexed likewise (identity 12 stays 12): g_macro_tail_inv
+	uint32_t elems3[kElems3 * 4];                         // distinct 16-byte parts of rows3_inv
+	uint32_t remap3[kRemap3 * 2];                         // {twist|flip word, element index}, indexed like rows3_inv, then kSingle3 + a
+	uint32_t image3[kImageBytes3 / 4];                    // shared-memory image of the deduplicated table (8 copies | remap)
 	bool ok;
 };
 
@@ -153,6 +173,39 @@ static const Host& host() {
 			const int j = inv(i % kA) + kA * inv(i / kA);
 			memcpy(h.rows_inv + i * kRowWords, h.rows + j * kRowWords, sizeof(uint32_t) * kRowWords);
 		}
+
+		std::map<std::array<uint32_t, 4>, uint32_t> elem;
+		auto element_of = [&](const uint32_t* r) {                        // index of r's 16-byte part, appended when new
+			const std::array<uint32_t, 4> key{r[0], r[1], r[2], r[3]};
+			auto it = elem.find(key);
+			if (it != elem.end()) return it->second;
+			const uint32_t e = (uint32_t)elem.size();
+			if (e < (uint32_t)kElems3) memcpy(h.elems3 + 4 * e, r, 16);
+			elem.emplace(key, e);
+			return e;
+		};
+		for (int i = 0; i < kRows3; ++i) {
+			const uint32_t* r = h.rows3_inv + i * kRowWords;
+			h.remap3[2 * i] = r[4];
+			h.remap3[2 * i + 1] = element_of(r);
+		}
+		for (int a = 0; a < 12; ++a) {
+			uint32_t r[kRowWords];
+			encode(s[a ^ 1], r);
+			h.remap3[2 * (kSingle3 + a)] = r[4];
+			h.remap3[2 * (kSingle3 + a) + 1] = element_of(r);
+		}
+		h.ok = h.ok && elem.size() == (size_t)kElems3;
+		// every index the kernel can form reproduces the row it stands for, word for word
+		auto same = [&](int i, const uint32_t* r) {
+			const uint32_t e = h.remap3[2 * i + 1];
+			return e < (uint32_t)kElems3 && memcmp(h.elems3 + 4 * e, r, 16) == 0 && h.remap3[2 * i] == r[4];
+		};
+		for (int i = 0; i < kRows3; ++i) h.ok = h.ok && same(i, h.rows3_inv + i * kRowWords);
+		for (int a = 0; a < 12; ++a) h.ok = h.ok && same(kSingle3 + a, h.rows_inv + (a + kA * 12) * kRowWords);
+		for (int e = 0; e < kElems3; ++e)
+			for (int c = 0; c < kRepDedup; ++c) memcpy(h.image3 + (e * kRepDedup + c) * 4, h.elems3 + 4 * e, 16);
+		memcpy(h.image3 + kElemBytes3 / 4, h.remap3, sizeof(h.remap3));
 	});
 	return h;
 }
@@ -392,6 +445,8 @@ k_scramble_macro(const uint8_t* __restrict__ actions, int8_t* __restrict__ out, 
 // bank groups {k, k + 4}, so within one quarter-warp phase of the LDS.128 only the two lanes that share a copy can collide
 // (when their rows have the same parity): ~1.9 wavefronts per phase instead of 2.6 for an unreplicated table.  The 4-byte
 // twist|flip word comes from a second array with R2 copies.  Trailing depth % 3 moves use the 2-move table (one copy).
+// Where the action buffers leave room for it, the deduplicated table (Host::image3, kDedup) replaces both arrays: 8 copies fit
+// for 1080 elements, and the depth % 3 moves are single-move rows of the same table.
 // Action bytes are masked to 4 bits, so an out-of-range action forms a row index <= kIdxMax3 that still lies inside the
 // CTA's shared memory (the launch always requests at least that much): an unspecified but memory-safe result.
 constexpr int kRep1 = 4;
@@ -416,6 +471,11 @@ __device__ __forceinline__ uint4 lds128(uint32_t a) {
 __device__ __forceinline__ uint32_t lds32(uint32_t a) {
 	uint32_t v;
 	asm("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a));
+	return v;
+}
+__device__ __forceinline__ uint2 lds64(uint32_t a) {
+	uint2 v;
+	asm("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(a));
 	return v;
 }
 
@@ -453,19 +513,25 @@ __device__ __forceinline__ void cubie_major(const Slots& s, uint32_t (&w)[5]) {
 // kMode: 0 = any depth (unaligned rows, funnel-shifted words), 1 = depth % 4 == 0 (word loads), 2 = depth % 16 == 0 (16-byte
 // loads in the main loop), 3 = depth % 128 == 0 (16-byte loads from padded rows).  Separate instantiations keep the common
 // mode-1 kernel (depth 100) free of the other modes' code.
-// n_work <= blockDim.x / 32 warps take chunks (small n is spread over all SMs); the whole CTA stages the table.
-template <int kMode, int R2>
+// n_work <= blockDim.x / 32 warps take chunks (small n is spread over all SMs).
+// kDedup: the deduplicated table (kImageBytes3, see Host::image3), staged by one bulk copy; a row is an LDS.64 of the remap
+// {twist|flip, element} and an LDS.128 of the element's copy for this lane, both conflict free in the element part: 4 + ~6
+// wavefronts per row against 7.75 + 3.5 for the 4-copy table, whose rows are two independent loads.  Otherwise the 4-copy
+// table (R2 copies of the twist|flip word), staged by the whole CTA.
+template <int kMode, int R2, bool kDedup>
 __global__ void __launch_bounds__(kMaxThreads, 1)
 k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out, int64_t n, int depth, int out_pitch,
-                  uint32_t p2_stride, uint32_t n_work) {
-	// p2_stride = 4 * R2 arrives as a kernel argument so that the twist|flip word's address is an IMAD (FMA pipe) rather than
-	// the LEA (ALU pipe, the binding one) ptxas emits for a power-of-two constant
+                  uint32_t p1_stride, uint32_t p2_stride, uint32_t n_work) {
+	// p2_stride = 4 * R2 (8 for kDedup: the remap entry) and p1_stride = 128 (kDedup: the element stride) arrive as kernel
+	// arguments so that the addresses are IMADs (FMA pipe) rather than the LEA (ALU pipe, the binding one) ptxas emits for a
+	// power-of-two constant
 	constexpr bool kWordAligned = kMode >= 1;
 	extern __shared__ __align__(128) uint8_t smem[];
 	constexpr int kP2Bytes3 = kP2Rows3 * 4 * R2;
 	uint8_t* table = smem;                                              // [P1 | P2 | tail | mbarriers | action buffers]
-	uint8_t* tail = smem + kP1Bytes3 + kP2Bytes3;
-	uint64_t* bars = reinterpret_cast<uint64_t*>(tail + kTailBytes);
+	uint8_t* tail = smem + kP1Bytes3 + kP2Bytes3;                       // kDedup: [elements | remap | table mbarrier | mbarriers | ...]
+	uint64_t* tbar = reinterpret_cast<uint64_t*>(smem + kImageBytes3);
+	uint64_t* bars = reinterpret_cast<uint64_t*>(kDedup ? smem + kImageBytes3 + 16 : tail + kTailBytes);
 	const uint32_t lane = threadIdx.x & 31, wib = threadIdx.x >> 5, n_warps = n_work;
 	const int chunk_bytes = 32 * depth;
 	// depth % 16 == 0: the main loop reads the action rows with 16-byte loads (a16).  depth % 128 == 0: the rows are 128 bytes
@@ -477,7 +543,8 @@ k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out,
 	const int pitch = depth + (pad16 ? 16 : 0);
 	uint8_t* buf = reinterpret_cast<uint8_t*>(bars) + kMaxThreads / 32 * 8 + (size_t)wib * (32 * pitch);
 	uint64_t* bar = &bars[wib];
-	const uint32_t off1 = smem_u32(table) + (lane & (kRep1 - 1)) * 16u, off2 = smem_u32(table) + (uint32_t)kP1Bytes3 + (lane & (R2 - 1)) * 4u;
+	const uint32_t off1 = smem_u32(table) + (lane & ((kDedup ? kRepDedup : kRep1) - 1)) * 16u;
+	const uint32_t off2 = smem_u32(table) + (kDedup ? (uint32_t)kElemBytes3 : (uint32_t)kP1Bytes3 + (lane & (R2 - 1)) * 4u);
 
 	const int64_t n_chunks = (n + 31) / 32;
 	const int64_t stride = (int64_t)gridDim.x * n_warps;
@@ -498,27 +565,35 @@ k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out,
 			}
 		}
 	};
+	if (kDedup && threadIdx.x == 0) mbar_init(tbar, 1);
 	if (lane == 0) mbar_init(bar, 1);
 	asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 	__syncwarp();
+	if (kDedup && threadIdx.x == 0) {
+		mbar_expect_tx(tbar, (uint32_t)kImageBytes3);
+		bulk_g2s(table, g_macro3_image, (uint32_t)kImageBytes3, tbar);
+	}
 	if (wib < n_work) issue(chunk);
-	for (int i = threadIdx.x; i < kP2Rows3 * kRep1; i += blockDim.x) {
-		const int row = i / kRep1, c = i % kRep1;
-		if (row < kRows3) {
-			const uint32_t* r = g_macro3 + row * kRowWords;
-			*reinterpret_cast<uint4*>(table + (row * kRep1 + c) * 16) = make_uint4(r[0], r[1], r[2], r[3]);
-			if (c < R2) *reinterpret_cast<uint32_t*>(table + kP1Bytes3 + (row * R2 + c) * 4) = r[4];
-		} else if (c < R2) {
-			*reinterpret_cast<uint32_t*>(table + kP1Bytes3 + (row * R2 + c) * 4) = 0u;
+	if (!kDedup) {
+		for (int i = threadIdx.x; i < kP2Rows3 * kRep1; i += blockDim.x) {
+			const int row = i / kRep1, c = i % kRep1;
+			if (row < kRows3) {
+				const uint32_t* r = g_macro3 + row * kRowWords;
+				*reinterpret_cast<uint4*>(table + (row * kRep1 + c) * 16) = make_uint4(r[0], r[1], r[2], r[3]);
+				if (c < R2) *reinterpret_cast<uint32_t*>(table + kP1Bytes3 + (row * R2 + c) * 4) = r[4];
+			} else if (c < R2) {
+				*reinterpret_cast<uint32_t*>(table + kP1Bytes3 + (row * R2 + c) * 4) = 0u;
+			}
+		}
+		for (int i = threadIdx.x; i < kDevRows; i += blockDim.x) {
+			const uint32_t* r = g_macro_tail_inv + (i < kRows ? i : kRows - 1) * kRowWords;
+			*reinterpret_cast<uint4*>(tail + i * 32) = make_uint4(r[0], r[1], r[2], r[3]);
+			*reinterpret_cast<uint32_t*>(tail + i * 32 + 16) = r[4];
 		}
 	}
-	for (int i = threadIdx.x; i < kDevRows; i += blockDim.x) {
-		const uint32_t* r = g_macro_tail_inv + (i < kRows ? i : kRows - 1) * kRowWords;
-		*reinterpret_cast<uint4*>(tail + i * 32) = make_uint4(r[0], r[1], r[2], r[3]);
-		*reinterpret_cast<uint32_t*>(tail + i * 32 + 16) = r[4];
-	}
-	__syncthreads();
+	__syncthreads();                                                    // kDedup: the table mbarrier is initialised for every warp
 	if (wib >= n_work) return;
+	if (kDedup) mbar_wait(tbar, 0);
 
 	uint32_t parity = 0;
 	for (; chunk < n_chunks; chunk += stride) {
@@ -544,9 +619,15 @@ k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out,
 				return __funnelshift_r(arow[m >> 2], arow[(m >> 2) + 1], ashift);
 			};
 			auto apply3 = [&](uint32_t r) {
-				const uint32_t o1 = mad_u32(r, 16u * kRep1, off1), o2 = mad_u32(r, p2_stride, off2);
-				apply_row(lds128(o1), lds32(o2), s);
+				if (kDedup) {
+					const uint2 e = lds64(mad_u32(r, p2_stride, off2));                 // {twist|flip, element}
+					apply_row(lds128(mad_u32(e.y, p1_stride, off1)), e.x, s);
+				} else {
+					const uint32_t o1 = mad_u32(r, 16u * kRep1, off1), o2 = mad_u32(r, p2_stride, off2);
+					apply_row(lds128(o1), lds32(o2), s);
+				}
 			};
+			auto apply1 = [&](uint32_t a) { apply3((uint32_t)kSingle3 + a); };     // kDedup: single inverse move a ^ 1 (a 4-bit masked)
 			// The kernel multiplies the INVERSE moves in REVERSE order: the slot-major product is then the inverse group element,
 			// whose byte q holds the position (and minus the twist) of CUBIE q -- the reference's cubie-major state up to a per-byte
 			// formula, so the result needs no scatter by cubie id (20 conflicting STS.U8 per cube otherwise).
@@ -570,12 +651,14 @@ k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out,
 				wa &= 0x0f0f0f0fu; wb &= 0x0f0f0f0fu;
 				apply3(__dp4a(wb, 0x010C9000u, 0u));
 				apply3(__dp4a(wb, 0x00000001u, __dp4a(wa, 0x0C900000u, 0u)));
-				apply_tail(__dp4a(wa, 0x0000010Du, 0u));
+				if (kDedup) { apply1((wa >> 8) & 0xffu); apply1(wa & 0xffu); }
+				else apply_tail(__dp4a(wa, 0x0000010Du, 0u));
 			};
 			auto rem4 = [&](uint32_t wa) {                                     // 4 moves, bytes 3..0: (3,2,1) then the single move 0
 				wa &= 0x0f0f0f0fu;
 				apply3(__dp4a(wa, 0x010C9000u, 0u));
-				apply_tail((wa & 0xffu) + 13u * 12u);
+				if (kDedup) apply1(wa & 0xffu);
+				else apply_tail((wa & 0xffu) + 13u * 12u);
 			};
 			auto fold = [&]() { s.C0 = fold_twists(s.C0); s.C1 = fold_twists(s.C1); };
 			auto group24w = [&](uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3, uint32_t w4, uint32_t w5) {
@@ -621,7 +704,11 @@ k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out,
 						else if (pos - 4 >= M) rem4(word_at(pos - 4));
 					} else {
 						for (; pos - 3 >= M; pos -= 3) apply3(inv_at(pos - 1) + 12u * inv_at(pos - 2) + 144u * inv_at(pos - 3));
-						if (pos > M) apply_tail(inv_at(pos - 1) + 13u * (pos - 2 >= M ? inv_at(pos - 2) : 12u));
+						if (kDedup) {
+							for (; pos > M; --pos) apply1(inv_at(pos - 1));
+						} else if (pos > M) {
+							apply_tail(inv_at(pos - 1) + 13u * (pos - 2 >= M ? inv_at(pos - 2) : 12u));
+						}
 					}
 					fold();
 				}
@@ -858,16 +945,21 @@ static int ensure_device() {
 	if (dev < 0 || dev >= 64) return rb_fail(RB_ERR_BAD_ARG, "device ordinal out of range%s%s");
 	if (done[dev]) return RB_OK;
 	const Host& h = host();
-	if (!h.ok) return rb_fail(RB_ERR_BAD_ARG, "macro-move table: corner twist is not additive for these move tables%s%s");
+	if (!h.ok) return rb_fail(RB_ERR_BAD_ARG, "macro-move tables: a host check failed (twist additivity or the deduplicated 3-move table)%s%s");
 	RB_CUDA(cudaMemcpyToSymbol(g_macro, h.rows, sizeof(h.rows)));
 	RB_CUDA(cudaMemcpyToSymbol(g_macro3, h.rows3_inv, sizeof(h.rows3_inv)));
 	RB_CUDA(cudaMemcpyToSymbol(g_macro_tail_inv, h.rows_inv, sizeof(h.rows_inv)));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<3, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaMemcpyToSymbol(g_macro3_image, h.image3, sizeof(h.image3)));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<0, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<2, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<3, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<0, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<2, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<3, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, 4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
 	RB_CUDA(cudaFuncSetAttribute(k_scramble_mm<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
 	RB_CUDA(cudaFuncSetAttribute(k_scramble_mm<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
 	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
@@ -893,10 +985,17 @@ static int64_t fixed_smem3(int r2) { return (int64_t)kP1Bytes3 + (int64_t)kP2Row
 constexpr int kStageThreads = 1024;             // threads that fill the table, whatever the number of working warps
 // row pitch of the action buffers (see the kernel): depth % 128 == 0 rows are padded by 16 bytes
 static int pitch3(int depth) { return depth % 128 == 0 ? depth + 16 : depth; }
+constexpr int64_t kFixedSmemDedup = kImageBytes3 + 16 + kMaxThreads / 32 * 8;   // image + table mbarrier + one per warp
+// Warps per CTA that the shared memory beside the table holds (r2 = 0: the deduplicated table, in multiples of 4 so that the
+// four sub-partitions get equal shares -- 2^24 x 100 moves on B200: 23 warps 0.771 ms, 20 warps 0.757 ms).
+static int64_t smem_warps3(int depth, int r2) {
+	const int64_t w = (kSmemBudget - 16 - (r2 ? fixed_smem3(r2) : kFixedSmemDedup)) / (32 * (int64_t)pitch3(depth));
+	return r2 ? w : w & ~3;
+}
 static int warps_for3(int64_t n, int depth, int r2) {
 	if (depth < 20) return 0;
-	int64_t w = (kSmemBudget - 16 - fixed_smem3(r2)) / (32 * (int64_t)pitch3(depth));
-	if (w > max_threads() / 32) w = max_threads() / 32;
+	int64_t w = smem_warps3(depth, r2);
+	if (w > max_threads() / 32) w = r2 ? max_threads() / 32 : max_threads() / 128 * 4;
 	if (w < 8) return 0;                         // long sequences: too few resident warps to hide the table latency
 	const int64_t spread = ((n + 31) / 32 + RB_NUM_SMS - 1) / RB_NUM_SMS;
 	if (w > spread) w = spread;
@@ -970,8 +1069,24 @@ static int launch(const uint8_t* actions, int8_t* out, int64_t n, int depth, cud
 	int rc = ensure_device();
 	if (rc != RB_OK) return rc;
 	static const int rows_per = env_int("RB_SCRAMBLE_MOVES_PER_ROW", 3), r2_env = env_int("RB_SCRAMBLE_R2", 1);
-	const int r2 = (depth % 4 == 0 && depth % 16 != 0 && (r2_env == 2 || r2_env == 4)) ? r2_env : 1;
+	// The deduplicated table where it leaves room for at least 12 warps (pitch <= 195: every depth from 20 to 195), else the
+	// 4-copy table.  2^24 cubes on B200, deduplicated / 4-copy: depth 100 (20 warps) 0.757 / 0.818 ms, 144 (16) 1.059 / 1.172,
+	// 176 (12) 1.319 / 1.450; with 8 warps it loses at some depths (200: 1.737 / 1.655, 256: 2.222 / 2.170).
+	const bool dedup = smem_warps3(depth, 0) >= 12;
+	const int r2 = dedup ? 0 : (depth % 4 == 0 && depth % 16 != 0 && (r2_env == 2 || r2_env == 4)) ? r2_env : 1;
 	const int W3 = rows_per == 3 ? warps_for3(n, depth, r2) : 0;
+	if (W3 > 0 && dedup) {
+		const int64_t ctas = ((n + 31) / 32 + W3 - 1) / W3;
+		const int grid = (int)(ctas < RB_NUM_SMS ? ctas : RB_NUM_SMS);
+		const size_t smem = (size_t)kFixedSmemDedup + (size_t)W3 * 32 * pitch3(depth) + 16;
+		const uint32_t nw = (uint32_t)W3, es = kRepDedup * 16;
+		if (depth % 4 != 0) k_scramble_macro3<0, 1, true><<<grid, W3 * 32, smem, st>>>(actions, out, n, depth, out_pitch, es, 8u, nw);
+		else if (depth % 128 == 0) k_scramble_macro3<3, 1, true><<<grid, W3 * 32, smem, st>>>(actions, out, n, depth, out_pitch, es, 8u, nw);
+		else if (depth % 16 == 0) k_scramble_macro3<2, 1, true><<<grid, W3 * 32, smem, st>>>(actions, out, n, depth, out_pitch, es, 8u, nw);
+		else k_scramble_macro3<1, 1, true><<<grid, W3 * 32, smem, st>>>(actions, out, n, depth, out_pitch, es, 8u, nw);
+		RB_LAUNCHED("scramble_macro3_2024");
+		return RB_OK;
+	}
 	if (W3 > 0) {
 		const int64_t ctas = ((n + 31) / 32 + W3 - 1) / W3;
 		const int grid = (int)(ctas < RB_NUM_SMS ? ctas : RB_NUM_SMS);
@@ -980,12 +1095,12 @@ static int launch(const uint8_t* actions, int8_t* out, int64_t n, int depth, cud
 		size_t smem = (size_t)fixed_smem3(r2) + (size_t)W3 * 32 * pitch3(depth) + 16;
 		if (smem < (size_t)kMinSmem3) smem = kMinSmem3;
 		const uint32_t nw = (uint32_t)W3;
-		if (depth % 4 != 0) k_scramble_macro3<0, 1><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 4u, nw);
-		else if (depth % 128 == 0) k_scramble_macro3<3, 1><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 4u, nw);
-		else if (depth % 16 == 0) k_scramble_macro3<2, 1><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 4u, nw);
-		else if (r2 == 2) k_scramble_macro3<1, 2><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 8u, nw);
-		else if (r2 == 4) k_scramble_macro3<1, 4><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 16u, nw);
-		else k_scramble_macro3<1, 1><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 4u, nw);
+		if (depth % 4 != 0) k_scramble_macro3<0, 1, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 4u, nw);
+		else if (depth % 128 == 0) k_scramble_macro3<3, 1, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 4u, nw);
+		else if (depth % 16 == 0) k_scramble_macro3<2, 1, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 4u, nw);
+		else if (r2 == 2) k_scramble_macro3<1, 2, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 8u, nw);
+		else if (r2 == 4) k_scramble_macro3<1, 4, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 16u, nw);
+		else k_scramble_macro3<1, 1, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 4u, nw);
 		RB_LAUNCHED("scramble_macro3_2024");
 		return RB_OK;
 	}

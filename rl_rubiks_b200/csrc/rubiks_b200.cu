@@ -45,15 +45,23 @@ int rb_get_perm686(uint8_t* perm) {
 int rb_get_macro_table(uint32_t* rows) {
 	RB_REQUIRE(rows, "null output");
 	const rbs::Host& h = rbs::host();
-	if (!h.ok) return rb_fail(RB_ERR_BAD_ARG, "macro-move table: corner twist is not additive for these move tables%s%s");
+	if (!h.ok) return rb_fail(RB_ERR_BAD_ARG, "macro-move tables: a host check failed (twist additivity or the deduplicated 3-move table)%s%s");
 	memcpy(rows, h.rows, sizeof(uint32_t) * rbs::kRows * rbs::kRowWords);
 	return RB_OK;
 }
 int rb_get_macro3_table(uint32_t* rows) {
 	RB_REQUIRE(rows, "null output");
 	const rbs::Host& h = rbs::host();
-	if (!h.ok) return rb_fail(RB_ERR_BAD_ARG, "macro-move table: corner twist is not additive for these move tables%s%s");
+	if (!h.ok) return rb_fail(RB_ERR_BAD_ARG, "macro-move tables: a host check failed (twist additivity or the deduplicated 3-move table)%s%s");
 	memcpy(rows, h.rows3, sizeof(uint32_t) * rbs::kRows3 * rbs::kRowWords);
+	return RB_OK;
+}
+int rb_get_macro3_dedup(uint32_t* elems, uint32_t* remap) {
+	RB_REQUIRE(elems && remap, "null output");
+	const rbs::Host& h = rbs::host();
+	if (!h.ok) return rb_fail(RB_ERR_BAD_ARG, "macro-move tables: a host check failed (twist additivity or the deduplicated 3-move table)%s%s");
+	memcpy(elems, h.elems3, sizeof(h.elems3));
+	memcpy(remap, h.remap3, sizeof(h.remap3));
 	return RB_OK;
 }
 int rb_get_stickers686(uint8_t* corner_home, uint8_t* corner_dst, uint8_t* edge_home, uint8_t* edge_dst) {
