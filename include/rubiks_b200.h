@@ -248,7 +248,7 @@ typedef struct rb_astar_view {
 	uint8_t* won;                 /* [K] */
 	int32_t* solved_index;        /* [K] */
 	void*    table;               /* shared seen-set, rb_hashset_bytes(capacity) bytes, cleared with rb_hashset_clear */
-	int64_t  capacity;            /* power of two, >= 2 K M */
+	int64_t  capacity;            /* power of two, >= 2 K M (checked: RB_ERR_CAPACITY below that) */
 	void*    scratch;             /* rb_astar_scratch_bytes(K, N) bytes */
 } rb_astar_view;
 int64_t rb_astar_scratch_bytes(int32_t K, int32_t N);

@@ -585,6 +585,10 @@ static int astar_view(const rb_astar_view* a, rba::View& v) {
 	RB_REQUIRE(a->states && a->G && a->parents && a->parent_actions && a->cost && a->in_open && a->count && a->n_sel && a->sel && a->won &&
 	           a->solved_index && a->table && a->scratch, "null buffer in view");
 	RB_REQUIRE_TABLE(a->table, a->capacity);
+	// a full table drops a child without an error word (k_probe stores slot -1): at least 2 K M slots keep every search's
+	// M states at load <= 1/2
+	if (a->capacity < 2 * (int64_t)a->K * a->M)
+		return rb_fail(RB_ERR_CAPACITY, "A* table capacity must be at least 2 K M slots%s%s");
 	RB_REQUIRE(aligned(a->scratch, 16) && aligned(a->states, 4) && aligned(a->G, 8) && aligned(a->cost, 8), "misaligned buffer");
 	const int64_t K = a->K, P = 12 * (int64_t)a->N, nbx = (P + rba::kThreads - 1) / rba::kThreads;
 	v.K = a->K; v.M = a->M; v.N = a->N;

@@ -119,3 +119,14 @@ def test_hashset_capacity_limits_are_errors():
 	assert N.lib.rb_hashset_clear(fake, (1 << 20) + 1, None) == N.RB_ERR_BAD_ARG
 	assert N.lib.rb_hashset_clear(ctypes.c_void_p((1 << 20) + 16), 1 << 20, None) == N.RB_ERR_BAD_ARG
 	assert N.lib.rb_hashset_rehash(fake, 1 << 10, fake, 1 << 31, None) == N.RB_ERR_CAPACITY
+	# A* shares one table among K searches of up to M states: below 2 K M slots a full table would drop children silently.
+	# roots / new_states / values are NULL, so no call can get past its argument checks to a launch.
+	K, M, Nx = 3, 1000, 4
+	v = N.AStarView(K, M, Nx, *([fake] * 12), 2048, fake)              # 2048 < 2 K M = 6000
+	out = [fake] * 4
+	assert N.lib.rb_astar_init(ctypes.byref(v), None, None) == N.RB_ERR_CAPACITY
+	assert N.lib.rb_astar_expand(ctypes.byref(v), M - 1, None, *out, None) == N.RB_ERR_CAPACITY
+	assert N.lib.rb_astar_commit(ctypes.byref(v), None, 0.5, *out[:3], None) == N.RB_ERR_CAPACITY
+	v.K, v.M = 65535, 1 << 14                                           # 2 K M overflows 32 bits
+	v.capacity = 1 << 30
+	assert N.lib.rb_astar_init(ctypes.byref(v), None, None) == N.RB_ERR_CAPACITY
