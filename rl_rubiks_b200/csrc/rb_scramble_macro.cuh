@@ -28,7 +28,6 @@
 #include "rb_common.cuh"
 #include "rb_tables.cuh"
 #include <cuda.h>              // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint)
-#include <stdlib.h>
 #include <array>
 #include <map>
 
@@ -266,13 +265,9 @@ __device__ __forceinline__ uint32_t shr_fma(uint32_t x) {
 
 // x >> 16 as a 2-way dot product (IDP.2A: x.hi16 * 1 + x.lo16 * 0): half the pipe time of the quarter-rate IMAD.HI
 __device__ __forceinline__ uint32_t shr16(uint32_t x) {
-#ifdef RB_SHR16_IMADHI
-	return shr_fma<16>(x);
-#else
 	uint32_t r;
 	asm("dp2a.hi.u32.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(x), "r"(0x01000000u), "r"(0u));
 	return r;
-#endif
 }
 
 // One table row applied to the slot-major state.  p1 = {corner selectors, edge selectors 0..2}, tf = twists | flips.
@@ -444,7 +439,7 @@ k_scramble_macro(const uint8_t* __restrict__ actions, int8_t* __restrict__ out, 
 // part would need 221 KB, so it is kept in kRep1 = 4 copies laid out row-major [row][copy] -- copy k = lane % 4 lives in
 // bank groups {k, k + 4}, so within one quarter-warp phase of the LDS.128 only the two lanes that share a copy can collide
 // (when their rows have the same parity): ~1.9 wavefronts per phase instead of 2.6 for an unreplicated table.  The 4-byte
-// twist|flip word comes from a second array with R2 copies.  Trailing depth % 3 moves use the 2-move table (one copy).
+// twist|flip word comes from a second array, one per row.  Trailing depth % 3 moves use the 2-move table (one copy).
 // Where the action buffers leave room for it, the deduplicated table (Host::image3, kDedup) replaces both arrays: 8 copies fit
 // for 1080 elements, and the depth % 3 moves are single-move rows of the same table.
 // Action bytes are masked to 4 bits, so an out-of-range action forms a row index <= kIdxMax3 that still lies inside the
@@ -453,7 +448,9 @@ constexpr int kRep1 = 4;
 constexpr int kIdxMax3 = 15 + 12 * 15 + 144 * 15;           // 2355
 constexpr int kP1Bytes3 = kRows3 * kRep1 * 16;              // 110,592
 constexpr int kP2Rows3 = 2368;                              // > kIdxMax3
+constexpr int kP2Bytes3 = kP2Rows3 * 4;                     // one twist|flip word per row
 constexpr int kTailBytes = kDevRows * 32;                   // 2-move rows padded to 32 bytes, one copy
+constexpr int kTableBytes3 = kP1Bytes3 + kP2Bytes3 + kTailBytes;      // the 4-copy table: [P1 | P2 | tail]
 constexpr int kMinSmem3 = (kIdxMax3 + 1) * kRep1 * 16 + 128;
 
 __device__ __forceinline__ uint32_t mad_u32(uint32_t a, uint32_t b, uint32_t c) {
@@ -479,6 +476,148 @@ __device__ __forceinline__ uint2 lds64(uint32_t a) {
 	return v;
 }
 
+// The 4-copy table, staged by the whole CTA (the caller synchronises): kRep1 copies of each row's 16-byte part, the rows'
+// twist|flip words (zero up to kP2Rows3), then the 2-move rows for the depth % 3 moves.
+__device__ __forceinline__ void stage_table3(uint8_t* table) {
+	for (int i = threadIdx.x; i < kP2Rows3 * kRep1; i += blockDim.x) {
+		const int row = i / kRep1, c = i % kRep1;
+		if (row < kRows3) {
+			const uint32_t* r = g_macro3 + row * kRowWords;
+			*reinterpret_cast<uint4*>(table + (row * kRep1 + c) * 16) = make_uint4(r[0], r[1], r[2], r[3]);
+			if (c == 0) *reinterpret_cast<uint32_t*>(table + kP1Bytes3 + row * 4) = r[4];
+		} else if (c == 0) {
+			*reinterpret_cast<uint32_t*>(table + kP1Bytes3 + row * 4) = 0u;
+		}
+	}
+	uint8_t* tail = table + kP1Bytes3 + kP2Bytes3;
+	for (int i = threadIdx.x; i < kDevRows; i += blockDim.x) {
+		const uint32_t* r = g_macro_tail_inv + (i < kRows ? i : kRows - 1) * kRowWords;
+		*reinterpret_cast<uint4*>(tail + i * 32) = make_uint4(r[0], r[1], r[2], r[3]);
+		*reinterpret_cast<uint32_t*>(tail + i * 32 + 16) = r[4];
+	}
+}
+
+__device__ __forceinline__ void fold(Slots& s) { s.C0 = fold_twists(s.C0); s.C1 = fold_twists(s.C1); }
+
+// The row primitives of the 3-move kernels on one lane's view of the table at `table` (the 4-copy table, or kDedup: the
+// deduplicated one).  p1_stride / p2_stride arrive as kernel arguments: see k_scramble_macro3.
+// The kernels multiply the INVERSE moves in REVERSE order: the slot-major product is then the inverse group element, whose
+// byte q holds the position (and minus the twist) of CUBIE q -- the reference's cubie-major state up to a per-byte formula,
+// so the result needs no scatter by cubie id (20 conflicting STS.U8 per cube otherwise).  The inversion a ^ 1 is folded into
+// the tables' layout, the action bytes are only masked to 4 bits; the row index a0 + 12 a1 + 144 a2 (a0 = the later move) is
+// one or two dp4a.
+template <bool kDedup>
+struct Rows3 {
+	uint32_t off1, off2, tail, p1_stride, p2_stride;
+
+	__device__ __forceinline__ Rows3(const uint8_t* table, uint32_t lane, uint32_t p1, uint32_t p2)
+		: off1(smem_u32(table) + (lane & ((kDedup ? kRepDedup : kRep1) - 1)) * 16u),
+		  off2(smem_u32(table) + (kDedup ? (uint32_t)kElemBytes3 : (uint32_t)kP1Bytes3)),
+		  tail(smem_u32(table + kP1Bytes3 + kP2Bytes3)), p1_stride(p1), p2_stride(p2) {}
+
+	__device__ __forceinline__ void apply3(Slots& s, uint32_t r) const {
+		if (kDedup) {
+			const uint2 e = lds64(mad_u32(r, p2_stride, off2));                 // {twist|flip, element}
+			apply_row(lds128(mad_u32(e.y, p1_stride, off1)), e.x, s);
+		} else {
+			const uint32_t o1 = mad_u32(r, 16u * kRep1, off1), o2 = mad_u32(r, p2_stride, off2);
+			apply_row(lds128(o1), lds32(o2), s);
+		}
+	}
+	// kDedup: the single inverse move a ^ 1 (a masked to 4 bits)
+	__device__ __forceinline__ void apply1(Slots& s, uint32_t a) const { apply3(s, (uint32_t)kSingle3 + a); }
+	// 4-copy table: a 2-move row (the second move may be the identity, 12)
+	__device__ __forceinline__ void apply_tail(Slots& s, uint32_t idx2) const {
+		const uint32_t r = tail + idx2 * 32u;
+		apply_row(lds128(r), lds32(r + 16u), s);
+	}
+	// 12 moves = 3 action words = 4 rows, last move first
+	__device__ __forceinline__ void apply_words(Slots& s, uint32_t w0, uint32_t w1, uint32_t w2) const {
+		w0 &= 0x0f0f0f0fu; w1 &= 0x0f0f0f0fu; w2 &= 0x0f0f0f0fu;
+		apply3(s, __dp4a(w2, 0x010C9000u, 0u));
+		apply3(s, __dp4a(w2, 0x00000001u, __dp4a(w1, 0x0C900000u, 0u)));
+		apply3(s, __dp4a(w1, 0x0000010Cu, __dp4a(w0, 0x90000000u, 0u)));
+		apply3(s, __dp4a(w0, 0x00010C90u, 0u));
+	}
+	// 8 moves, bytes 7..0: (7,6,5) (4,3,2) then the pair (1,0)
+	__device__ __forceinline__ void rem8(Slots& s, uint32_t wa, uint32_t wb) const {
+		wa &= 0x0f0f0f0fu; wb &= 0x0f0f0f0fu;
+		apply3(s, __dp4a(wb, 0x010C9000u, 0u));
+		apply3(s, __dp4a(wb, 0x00000001u, __dp4a(wa, 0x0C900000u, 0u)));
+		if (kDedup) { apply1(s, (wa >> 8) & 0xffu); apply1(s, wa & 0xffu); }
+		else apply_tail(s, __dp4a(wa, 0x0000010Du, 0u));
+	}
+	// 4 moves, bytes 3..0: (3,2,1) then the single move 0
+	__device__ __forceinline__ void rem4(Slots& s, uint32_t wa) const {
+		wa &= 0x0f0f0f0fu;
+		apply3(s, __dp4a(wa, 0x010C9000u, 0u));
+		if (kDedup) apply1(s, wa & 0xffu);
+		else apply_tail(s, (wa & 0xffu) + 13u * 12u);
+	}
+	// 24 moves: 8 rows add at most 16 to a twist accumulator <= 10
+	__device__ __forceinline__ void group24(Slots& s, uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3, uint32_t w4, uint32_t w5) const {
+		apply_words(s, w3, w4, w5); apply_words(s, w0, w1, w2);
+		fold(s);
+	}
+};
+
+// The whole sequence from word loads: word_at(m) = action bytes m .. m+3 (m % 4 == 0), inv_at(m) = action byte m masked to 4 bits
+// (the tables are indexed by the raw action).  The depth % 24 moves at the end of the sequence come first -- at most 4 + 3 + 1
+// rows, 8 byte-fetched rows when !kWords (depth % 4 != 0) -- then 24-move groups from the end, two (48 moves) per loop trip:
+// half the loop bookkeeping.
+template <bool kWords, bool kDedup, class WordAt, class InvAt>
+__device__ __forceinline__ void walk3(const Rows3<kDedup>& t, Slots& s, int depth, WordAt word_at, InvAt inv_at) {
+	const int M = depth - depth % 24;
+	int pos = depth;
+	if (pos > M) {
+		if (kWords) {                                               // 4, 8, ..., 20 moves: whole words, indices by dp4a
+			if (pos - 12 >= M) { t.apply_words(s, word_at(pos - 12), word_at(pos - 8), word_at(pos - 4)); pos -= 12; }
+			if (pos - 8 >= M) t.rem8(s, word_at(pos - 8), word_at(pos - 4));
+			else if (pos - 4 >= M) t.rem4(s, word_at(pos - 4));
+		} else {
+			for (; pos - 3 >= M; pos -= 3) t.apply3(s, inv_at(pos - 1) + 12u * inv_at(pos - 2) + 144u * inv_at(pos - 3));
+			if (kDedup) {
+				for (; pos > M; --pos) t.apply1(s, inv_at(pos - 1));
+			} else if (pos > M) {
+				t.apply_tail(s, inv_at(pos - 1) + 13u * (pos - 2 >= M ? inv_at(pos - 2) : 12u));
+			}
+		}
+		fold(s);
+	}
+	auto group24 = [&](int m) { t.group24(s, word_at(m), word_at(m + 4), word_at(m + 8), word_at(m + 12), word_at(m + 16), word_at(m + 20)); };
+	int m = M - 24;
+	for (; m >= 24; m -= 48) { group24(m); group24(m - 24); }
+	if (m >= 0) group24(m);
+}
+
+// Writes the packed [cube][20] results of cnt <= kCubes cubes starting at cube `first`: thread tid holds words tid + kCubes * t
+// of the span in w[t].  out_pitch = 20: contiguous in HBM; 288: each state parked at the head of a 6x8x6 row for the rb686
+// render; bytes where out or the pitch is not word aligned.
+template <int kCubes>
+__device__ __forceinline__ void store_results(int8_t* out, int64_t first, int out_pitch, int cnt, uint32_t tid, const uint32_t (&w)[5]) {
+	uint8_t* dst = reinterpret_cast<uint8_t*>(out) + first * out_pitch;
+	if (out_pitch == 20 && (reinterpret_cast<uintptr_t>(out) & 3u) == 0) {
+#pragma unroll
+		for (int t = 0; t < 5; ++t) {
+			const int j = (int)tid + kCubes * t;
+			if (j < cnt * 5) reinterpret_cast<uint32_t*>(dst)[j] = w[t];
+		}
+	} else if ((reinterpret_cast<uintptr_t>(out) & 3u) == 0 && (out_pitch & 3) == 0) {
+#pragma unroll
+		for (int t = 0; t < 5; ++t) {
+			const int j = (int)tid + kCubes * t, c = j / 5, k = j - 5 * c;
+			if (j < cnt * 5) *reinterpret_cast<uint32_t*>(dst + c * out_pitch + 4 * k) = w[t];
+		}
+	} else {
+#pragma unroll
+		for (int t = 0; t < 5; ++t) {
+			const int j = (int)tid + kCubes * t, c = j / 5, k = j - 5 * c;
+			if (j < cnt * 5)
+				for (int q = 0; q < 4; ++q) dst[c * out_pitch + 4 * k + q] = (uint8_t)(w[t] >> (8 * q));
+		}
+	}
+}
+
 // Per byte: twist accumulator (bits 0-4) -> its value mod 3, by base-4 digit folds (4 == 1 mod 3); other bits ignored.
 // The accumulators have just been folded (<= 10, fits 4 bits): two digit folds suffice.
 __device__ __forceinline__ uint32_t mod3_bytes_folded(uint32_t c) {
@@ -488,10 +627,10 @@ __device__ __forceinline__ uint32_t mod3_bytes_folded(uint32_t c) {
 	return t ^ (x * 3u);
 }
 
-// Inverse-element form (see k_scramble_macro3): byte q of the slot-major registers describes CUBIE q -- id field = its
-// position, twist accumulator = minus its twist, flip bits = its flip.  Per byte: corner value 3 * pos + ori with
-// ori = acc mod 3 where the position has negative chirality (0, 2, 5, 7: bit 0 == bit 2), its negation elsewhere;
-// edge value 2 * pos + flip.  The five words are the reference's int8[20] state.
+// Inverse-element form (see Rows3): byte q of the slot-major registers describes CUBIE q -- id field = its position, twist
+// accumulator = minus its twist, flip bits = its flip.  Per byte: corner value 3 * pos + ori with ori = acc mod 3 where the
+// position has negative chirality (0, 2, 5, 7: bit 0 == bit 2), its negation elsewhere; edge value 2 * pos + flip.  The five
+// words are the reference's int8[20] state.
 __device__ __forceinline__ void cubie_major(const Slots& s, uint32_t (&w)[5]) {
 #pragma unroll
 	for (int h = 0; h < 2; ++h) {
@@ -517,21 +656,19 @@ __device__ __forceinline__ void cubie_major(const Slots& s, uint32_t (&w)[5]) {
 // kDedup: the deduplicated table (kImageBytes3, see Host::image3), staged by one bulk copy; a row is an LDS.64 of the remap
 // {twist|flip, element} and an LDS.128 of the element's copy for this lane, both conflict free in the element part: 4 + ~6
 // wavefronts per row against 7.75 + 3.5 for the 4-copy table, whose rows are two independent loads.  Otherwise the 4-copy
-// table (R2 copies of the twist|flip word), staged by the whole CTA.
-template <int kMode, int R2, bool kDedup>
+// table, staged by the whole CTA.
+template <int kMode, bool kDedup>
 __global__ void __launch_bounds__(kMaxThreads, 1)
 k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out, int64_t n, int depth, int out_pitch,
                   uint32_t p1_stride, uint32_t p2_stride, uint32_t n_work) {
-	// p2_stride = 4 * R2 (8 for kDedup: the remap entry) and p1_stride = 128 (kDedup: the element stride) arrive as kernel
-	// arguments so that the addresses are IMADs (FMA pipe) rather than the LEA (ALU pipe, the binding one) ptxas emits for a
-	// power-of-two constant
+	// p2_stride = 4 (8 for kDedup: the remap entry) and p1_stride = 128 (kDedup: the element stride) arrive as kernel arguments
+	// so that the addresses are IMADs (FMA pipe) rather than the LEA (ALU pipe, the binding one) ptxas emits for a power-of-two
+	// constant
 	constexpr bool kWordAligned = kMode >= 1;
 	extern __shared__ __align__(128) uint8_t smem[];
-	constexpr int kP2Bytes3 = kP2Rows3 * 4 * R2;
 	uint8_t* table = smem;                                              // [P1 | P2 | tail | mbarriers | action buffers]
-	uint8_t* tail = smem + kP1Bytes3 + kP2Bytes3;                       // kDedup: [elements | remap | table mbarrier | mbarriers | ...]
-	uint64_t* tbar = reinterpret_cast<uint64_t*>(smem + kImageBytes3);
-	uint64_t* bars = reinterpret_cast<uint64_t*>(kDedup ? smem + kImageBytes3 + 16 : tail + kTailBytes);
+	uint64_t* tbar = reinterpret_cast<uint64_t*>(smem + kImageBytes3);  // kDedup: [elements | remap | table mbarrier | mbarriers | ...]
+	uint64_t* bars = reinterpret_cast<uint64_t*>(kDedup ? smem + kImageBytes3 + 16 : smem + kTableBytes3);
 	const uint32_t lane = threadIdx.x & 31, wib = threadIdx.x >> 5, n_warps = n_work;
 	const int chunk_bytes = 32 * depth;
 	// depth % 16 == 0: the main loop reads the action rows with 16-byte loads (a16).  depth % 128 == 0: the rows are 128 bytes
@@ -543,8 +680,7 @@ k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out,
 	const int pitch = depth + (pad16 ? 16 : 0);
 	uint8_t* buf = reinterpret_cast<uint8_t*>(bars) + kMaxThreads / 32 * 8 + (size_t)wib * (32 * pitch);
 	uint64_t* bar = &bars[wib];
-	const uint32_t off1 = smem_u32(table) + (lane & ((kDedup ? kRepDedup : kRep1) - 1)) * 16u;
-	const uint32_t off2 = smem_u32(table) + (kDedup ? (uint32_t)kElemBytes3 : (uint32_t)kP1Bytes3 + (lane & (R2 - 1)) * 4u);
+	const Rows3<kDedup> t(table, lane, p1_stride, p2_stride);
 
 	const int64_t n_chunks = (n + 31) / 32;
 	const int64_t stride = (int64_t)gridDim.x * n_warps;
@@ -574,23 +710,7 @@ k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out,
 		bulk_g2s(table, g_macro3_image, (uint32_t)kImageBytes3, tbar);
 	}
 	if (wib < n_work) issue(chunk);
-	if (!kDedup) {
-		for (int i = threadIdx.x; i < kP2Rows3 * kRep1; i += blockDim.x) {
-			const int row = i / kRep1, c = i % kRep1;
-			if (row < kRows3) {
-				const uint32_t* r = g_macro3 + row * kRowWords;
-				*reinterpret_cast<uint4*>(table + (row * kRep1 + c) * 16) = make_uint4(r[0], r[1], r[2], r[3]);
-				if (c < R2) *reinterpret_cast<uint32_t*>(table + kP1Bytes3 + (row * R2 + c) * 4) = r[4];
-			} else if (c < R2) {
-				*reinterpret_cast<uint32_t*>(table + kP1Bytes3 + (row * R2 + c) * 4) = 0u;
-			}
-		}
-		for (int i = threadIdx.x; i < kDevRows; i += blockDim.x) {
-			const uint32_t* r = g_macro_tail_inv + (i < kRows ? i : kRows - 1) * kRowWords;
-			*reinterpret_cast<uint4*>(tail + i * 32) = make_uint4(r[0], r[1], r[2], r[3]);
-			*reinterpret_cast<uint32_t*>(tail + i * 32 + 16) = r[4];
-		}
-	}
+	if (!kDedup) stage_table3(table);
 	__syncthreads();                                                    // kDedup: the table mbarrier is initialised for every warp
 	if (wib >= n_work) return;
 	if (kDedup) mbar_wait(tbar, 0);
@@ -618,103 +738,38 @@ k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out,
 				if (kWordAligned) return *reinterpret_cast<const uint32_t*>(row + m);
 				return __funnelshift_r(arow[m >> 2], arow[(m >> 2) + 1], ashift);
 			};
-			auto apply3 = [&](uint32_t r) {
-				if (kDedup) {
-					const uint2 e = lds64(mad_u32(r, p2_stride, off2));                 // {twist|flip, element}
-					apply_row(lds128(mad_u32(e.y, p1_stride, off1)), e.x, s);
-				} else {
-					const uint32_t o1 = mad_u32(r, 16u * kRep1, off1), o2 = mad_u32(r, p2_stride, off2);
-					apply_row(lds128(o1), lds32(o2), s);
-				}
-			};
-			auto apply1 = [&](uint32_t a) { apply3((uint32_t)kSingle3 + a); };     // kDedup: single inverse move a ^ 1 (a 4-bit masked)
-			// The kernel multiplies the INVERSE moves in REVERSE order: the slot-major product is then the inverse group element,
-			// whose byte q holds the position (and minus the twist) of CUBIE q -- the reference's cubie-major state up to a per-byte
-			// formula, so the result needs no scatter by cubie id (20 conflicting STS.U8 per cube otherwise).
-			// 12 moves = 3 action words = 4 rows, last move first; the inversion a ^ 1 is folded into the tables' layout, the action
-			// bytes are only masked to 4 bits; the row index a0 + 12 a1 + 144 a2 (a0 = the later move) is one or two dp4a.
-			auto apply_words = [&](uint32_t w0, uint32_t w1, uint32_t w2) {
-				w0 &= 0x0f0f0f0fu; w1 &= 0x0f0f0f0fu; w2 &= 0x0f0f0f0fu;
-				apply3(__dp4a(w2, 0x010C9000u, 0u));
-				apply3(__dp4a(w2, 0x00000001u, __dp4a(w1, 0x0C900000u, 0u)));
-				apply3(__dp4a(w1, 0x0000010Cu, __dp4a(w0, 0x90000000u, 0u)));
-				apply3(__dp4a(w0, 0x00010C90u, 0u));
-			};
-			auto inv_at = [&](int m) -> uint32_t { return row[m] & 15u; };     // raw action: the tables are indexed by it
-			// the depth % 24 moves at the end of the sequence come first: at most 4 + 3 + 1 rows (8 byte-fetched rows when unaligned)
-			const int M = depth - depth % 24;
-			auto apply_tail = [&](uint32_t idx2) {                             // 2-move row (second move may be the identity, 12)
-				const uint32_t r = smem_u32(tail) + idx2 * 32u;
-				apply_row(lds128(r), lds32(r + 16u), s);
-			};
-			auto rem8 = [&](uint32_t wa, uint32_t wb) {                        // 8 moves, bytes 7..0: (7,6,5) (4,3,2) then the pair (1,0)
-				wa &= 0x0f0f0f0fu; wb &= 0x0f0f0f0fu;
-				apply3(__dp4a(wb, 0x010C9000u, 0u));
-				apply3(__dp4a(wb, 0x00000001u, __dp4a(wa, 0x0C900000u, 0u)));
-				if (kDedup) { apply1((wa >> 8) & 0xffu); apply1(wa & 0xffu); }
-				else apply_tail(__dp4a(wa, 0x0000010Du, 0u));
-			};
-			auto rem4 = [&](uint32_t wa) {                                     // 4 moves, bytes 3..0: (3,2,1) then the single move 0
-				wa &= 0x0f0f0f0fu;
-				apply3(__dp4a(wa, 0x010C9000u, 0u));
-				if (kDedup) apply1(wa & 0xffu);
-				else apply_tail((wa & 0xffu) + 13u * 12u);
-			};
-			auto fold = [&]() { s.C0 = fold_twists(s.C0); s.C1 = fold_twists(s.C1); };
-			auto group24w = [&](uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3, uint32_t w4, uint32_t w5) {
-				apply_words(w3, w4, w5); apply_words(w0, w1, w2);              // 8 rows add at most 16 to a twist accumulator <= 10
-				fold();
-			};
-			auto group24 = [&](int m) { group24w(word_at(m), word_at(m + 4), word_at(m + 8), word_at(m + 12), word_at(m + 16), word_at(m + 20)); };
-			int m = M - 24;
 			if (a16) {
 				// depth % 16 == 0 (so depth % 24 is 0, 8 or 16): rows whose word stride is a multiple of 8 (depth 32, 64, 96, ...) would
 				// read single words with 8- to 32-way bank conflicts, 16-byte loads cut that four-fold.  Pairs of groups are anchored at
 				// multiples of 48 from the row start; what lies above them -- an odd group and / or the remainder -- is at most 40 bytes
 				// starting 16-byte aligned and is taken with two or three 16-byte loads as well (the last may run 8 bytes past the row).
+				const int M = depth - depth % 24;
+				int m = M - 24;
 				const int rem = depth - M, top = (M / 48) * 48;
 				const bool odd = (M / 24) & 1;
 				const uint4* q = reinterpret_cast<const uint4*>(row + top);
 				if (odd) {
 					const uint4 q0 = q[0], q1 = q[1];
-					if (rem == 8) { rem8(q1.z, q1.w); fold(); }
-					else if (rem == 16) { const uint4 q2 = q[2]; apply_words(q1.w, q2.x, q2.y); rem4(q1.z); fold(); }
-					group24w(q0.x, q0.y, q0.z, q0.w, q1.x, q1.y);
+					if (rem == 8) { t.rem8(s, q1.z, q1.w); fold(s); }
+					else if (rem == 16) { const uint4 q2 = q[2]; t.apply_words(s, q1.w, q2.x, q2.y); t.rem4(s, q1.z); fold(s); }
+					t.group24(s, q0.x, q0.y, q0.z, q0.w, q1.x, q1.y);
 					m -= 24;
 				} else if (rem) {
 					const uint4 q0 = q[0];
-					if (rem == 8) rem8(q0.x, q0.y);
-					else { apply_words(q0.y, q0.z, q0.w); rem4(q0.x); }
-					fold();
+					if (rem == 8) t.rem8(s, q0.x, q0.y);
+					else { t.apply_words(s, q0.y, q0.z, q0.w); t.rem4(s, q0.x); }
+					fold(s);
 				}
 				for (; m >= 24; m -= 48) {
 					const uint4* p = reinterpret_cast<const uint4*>(row + (m - 24));
 					const uint4 q0 = p[0], q1 = p[1], q2 = p[2];
-					apply_words(q2.y, q2.z, q2.w); apply_words(q1.z, q1.w, q2.x);
-					fold();
-					apply_words(q0.w, q1.x, q1.y); apply_words(q0.x, q0.y, q0.z);
-					fold();
+					t.apply_words(s, q2.y, q2.z, q2.w); t.apply_words(s, q1.z, q1.w, q2.x);
+					fold(s);
+					t.apply_words(s, q0.w, q1.x, q1.y); t.apply_words(s, q0.x, q0.y, q0.z);
+					fold(s);
 				}
 			} else {
-				int pos = depth;
-				if (pos > M) {
-					if (kWordAligned) {                                         // 4, 8, ..., 20 moves: whole words, indices by dp4a
-						if (pos - 12 >= M) { apply_words(word_at(pos - 12), word_at(pos - 8), word_at(pos - 4)); pos -= 12; }
-						if (pos - 8 >= M) rem8(word_at(pos - 8), word_at(pos - 4));
-						else if (pos - 4 >= M) rem4(word_at(pos - 4));
-					} else {
-						for (; pos - 3 >= M; pos -= 3) apply3(inv_at(pos - 1) + 12u * inv_at(pos - 2) + 144u * inv_at(pos - 3));
-						if (kDedup) {
-							for (; pos > M; --pos) apply1(inv_at(pos - 1));
-						} else if (pos > M) {
-							apply_tail(inv_at(pos - 1) + 13u * (pos - 2 >= M ? inv_at(pos - 2) : 12u));
-						}
-					}
-					fold();
-				}
-				// two groups (48 moves) per trip: half the loop bookkeeping
-				for (; m >= 24; m -= 48) { group24(m); group24(m - 24); }
-				if (m >= 0) group24(m);
+				walk3<kWordAligned>(t, s, depth, word_at, [&](int m) -> uint32_t { return row[m] & 15u; });
 			}
 			cubie_major(s, res);
 		}
@@ -727,41 +782,18 @@ k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out,
 		__syncwarp();
 		// 32 cubes = 640 contiguous bytes in shared memory: each lane takes its five words into registers, the buffer is then
 		// free for the bulk copy of the warp's next chunk, which is started BEFORE the results leave for HBM (the stores, and
-		// their completion, are off the path that refills the buffer).  out_pitch = 20: also contiguous in HBM (288: parked at
-		// the head of a 6x8x6 row for the rb686 render).
+		// their completion, are off the path that refills the buffer).
 		uint32_t outw[5];
 #pragma unroll
-		for (int t = 0; t < 5; ++t) {
-			const int j = lane + 32 * t;
-			outw[t] = j < cnt * 5 ? reinterpret_cast<const uint32_t*>(buf)[j] : 0u;
+		for (int k = 0; k < 5; ++k) {
+			const int j = lane + 32 * k;
+			outw[k] = j < cnt * 5 ? reinterpret_cast<const uint32_t*>(buf)[j] : 0u;
 		}
 		// generic-proxy reads / writes of the buffer are ordered before the async-proxy refill
 		asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 		__syncwarp();
 		issue(chunk + stride);
-		{
-			uint8_t* dst = reinterpret_cast<uint8_t*>(out) + chunk * 32 * out_pitch;
-			if (out_pitch == 20 && (reinterpret_cast<uintptr_t>(out) & 3u) == 0) {
-#pragma unroll
-				for (int t = 0; t < 5; ++t) {
-					const int j = lane + 32 * t;
-					if (j < cnt * 5) reinterpret_cast<uint32_t*>(dst)[j] = outw[t];
-				}
-			} else if ((reinterpret_cast<uintptr_t>(out) & 3u) == 0 && (out_pitch & 3) == 0) {
-#pragma unroll
-				for (int t = 0; t < 5; ++t) {
-					const int j = lane + 32 * t, c = j / 5, k = j - 5 * c;
-					if (j < cnt * 5) *reinterpret_cast<uint32_t*>(dst + c * out_pitch + 4 * k) = outw[t];
-				}
-			} else {
-#pragma unroll
-				for (int t = 0; t < 5; ++t) {
-					const int j = lane + 32 * t, c = j / 5, k = j - 5 * c;
-					if (j < cnt * 5)
-						for (int q = 0; q < 4; ++q) dst[c * out_pitch + 4 * k + q] = (uint8_t)(outw[t] >> (8 * q));
-				}
-			}
-		}
+		store_results<32>(out, chunk * 32, out_pitch, cnt, lane, outw);
 	}
 }
 
@@ -772,7 +804,7 @@ k_scramble_macro3(const uint8_t* __restrict__ actions, int8_t* __restrict__ out,
 // row request per ~8 clocks and cost 1.49 ms for 2^24 x 100 moves).  Shared-memory banks are the word COLUMN of the tile
 // whatever the row, so the conflict-free read is a whole row per instruction: lane l takes word l of rows m .. m+3 (four
 // LDS.32) and holds moves m .. m+3 of cubes 4 l .. 4 l + 3 as a 4 x 4 byte matrix; warp k of the quad transposes out column
-// k (three PRMT with warp-uniform selectors) and works on cube 4 l + k.  The rest is k_scramble_macro3's modes 0 / 1.
+// k (three PRMT with warp-uniform selectors) and works on cube 4 l + k.  The rest is walk3 on the 4-copy table.
 constexpr int kSpan = 128;
 __device__ __forceinline__ void quad_sync(uint32_t quad) {
 	asm volatile("bar.sync %0, 128;" ::"r"(quad + 1u) : "memory");
@@ -783,15 +815,13 @@ __global__ void __launch_bounds__(kMaxThreads, 1)
 k_scramble_mm(const __grid_constant__ CUtensorMap tmap, int8_t* __restrict__ out, int64_t n, int depth, int out_pitch, uint32_t p2_stride,
               uint32_t n_quads, int box_h) {
 	extern __shared__ __align__(128) uint8_t smem[];
-	constexpr int kP2Bytes3 = kP2Rows3 * 4;
 	uint8_t* table = smem;                                              // [P1 | P2 | tail | mbarriers | one tile per quad]
-	uint8_t* tail = smem + kP1Bytes3 + kP2Bytes3;
-	uint64_t* bars = reinterpret_cast<uint64_t*>(tail + kTailBytes);
+	uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kTableBytes3);
 	const uint32_t lane = threadIdx.x & 31, wib = threadIdx.x >> 5, quad = wib >> 2, k = wib & 3u, tq = threadIdx.x & 127u;
 	const int span_bytes = kSpan * depth;
 	uint8_t* tile = reinterpret_cast<uint8_t*>(bars) + kMaxThreads / 32 * 8 + (size_t)quad * span_bytes;
 	uint64_t* bar = &bars[quad];
-	const uint32_t off1 = smem_u32(table) + (lane & (kRep1 - 1)) * 16u, off2 = smem_u32(table) + (uint32_t)kP1Bytes3;
+	const Rows3<false> t(table, lane, 0u, p2_stride);
 	const int64_t n_spans = (n + kSpan - 1) / kSpan, stride = (int64_t)gridDim.x * n_quads;
 	int64_t span = (int64_t)blockIdx.x * n_quads + quad;
 
@@ -803,21 +833,7 @@ k_scramble_mm(const __grid_constant__ CUtensorMap tmap, int8_t* __restrict__ out
 	if (tq == 0) mbar_init(bar, 1);
 	asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 	if (tq == 0 && quad < n_quads) issue(span);                            // the thread that initialised the barrier; the others meet it after the block barrier
-	for (int i = threadIdx.x; i < kP2Rows3 * kRep1; i += blockDim.x) {
-		const int row = i / kRep1, c = i % kRep1;
-		if (row < kRows3) {
-			const uint32_t* r = g_macro3 + row * kRowWords;
-			*reinterpret_cast<uint4*>(table + (row * kRep1 + c) * 16) = make_uint4(r[0], r[1], r[2], r[3]);
-			if (c == 0) *reinterpret_cast<uint32_t*>(table + kP1Bytes3 + row * 4) = r[4];
-		} else if (c == 0) {
-			*reinterpret_cast<uint32_t*>(table + kP1Bytes3 + row * 4) = 0u;
-		}
-	}
-	for (int i = threadIdx.x; i < kDevRows; i += blockDim.x) {
-		const uint32_t* r = g_macro_tail_inv + (i < kRows ? i : kRows - 1) * kRowWords;
-		*reinterpret_cast<uint4*>(tail + i * 32) = make_uint4(r[0], r[1], r[2], r[3]);
-		*reinterpret_cast<uint32_t*>(tail + i * 32 + 16) = r[4];
-	}
+	stage_table3(table);
 	__syncthreads();
 	if (quad >= n_quads) return;
 
@@ -837,53 +853,7 @@ k_scramble_mm(const __grid_constant__ CUtensorMap tmap, int8_t* __restrict__ out
 				const uint32_t x = prmt(p[0], p[32], sel1), y = prmt(p[64], p[96], sel1);
 				return prmt(x, y, sel2);
 			};
-			auto inv_at = [&](int m) -> uint32_t { return tile[m * kSpan + (int)my_cube] & 15u; };
-			auto apply3 = [&](uint32_t r) {
-				const uint32_t o1 = mad_u32(r, 16u * kRep1, off1), o2 = mad_u32(r, p2_stride, off2);
-				apply_row(lds128(o1), lds32(o2), s);
-			};
-			auto apply_words = [&](uint32_t w0, uint32_t w1, uint32_t w2) {      // 12 moves, last first (see k_scramble_macro3)
-				w0 &= 0x0f0f0f0fu; w1 &= 0x0f0f0f0fu; w2 &= 0x0f0f0f0fu;
-				apply3(__dp4a(w2, 0x010C9000u, 0u));
-				apply3(__dp4a(w2, 0x00000001u, __dp4a(w1, 0x0C900000u, 0u)));
-				apply3(__dp4a(w1, 0x0000010Cu, __dp4a(w0, 0x90000000u, 0u)));
-				apply3(__dp4a(w0, 0x00010C90u, 0u));
-			};
-			auto apply_tail = [&](uint32_t idx2) {
-				const uint32_t r = smem_u32(tail) + idx2 * 32u;
-				apply_row(lds128(r), lds32(r + 16u), s);
-			};
-			auto rem8 = [&](uint32_t wa, uint32_t wb) {
-				wa &= 0x0f0f0f0fu; wb &= 0x0f0f0f0fu;
-				apply3(__dp4a(wb, 0x010C9000u, 0u));
-				apply3(__dp4a(wb, 0x00000001u, __dp4a(wa, 0x0C900000u, 0u)));
-				apply_tail(__dp4a(wa, 0x0000010Du, 0u));
-			};
-			auto rem4 = [&](uint32_t wa) {
-				wa &= 0x0f0f0f0fu;
-				apply3(__dp4a(wa, 0x010C9000u, 0u));
-				apply_tail((wa & 0xffu) + 13u * 12u);
-			};
-			auto fold = [&]() { s.C0 = fold_twists(s.C0); s.C1 = fold_twists(s.C1); };
-			auto group24 = [&](int m) {
-				const uint32_t w0 = word_at(m), w1 = word_at(m + 4), w2 = word_at(m + 8), w3 = word_at(m + 12), w4 = word_at(m + 16), w5 = word_at(m + 20);
-				apply_words(w3, w4, w5); apply_words(w0, w1, w2);
-				fold();
-			};
-			const int M = depth - depth % 24;
-			int pos = depth;
-			if (pos > M) {
-				if (kWords) {
-					if (pos - 12 >= M) { apply_words(word_at(pos - 12), word_at(pos - 8), word_at(pos - 4)); pos -= 12; }
-					if (pos - 8 >= M) rem8(word_at(pos - 8), word_at(pos - 4));
-					else if (pos - 4 >= M) rem4(word_at(pos - 4));
-				} else {
-					for (; pos - 3 >= M; pos -= 3) apply3(inv_at(pos - 1) + 12u * inv_at(pos - 2) + 144u * inv_at(pos - 3));
-					if (pos > M) apply_tail(inv_at(pos - 1) + 13u * (pos - 2 >= M ? inv_at(pos - 2) : 12u));
-				}
-				fold();
-			}
-			for (int m = M - 24; m >= 0; m -= 24) group24(m);
+			walk3<kWords>(t, s, depth, word_at, [&](int m) -> uint32_t { return tile[m * kSpan + (int)my_cube] & 15u; });
 			cubie_major(s, res);
 		}
 		quad_sync(quad);                                                  // the whole tile is consumed
@@ -895,46 +865,21 @@ k_scramble_mm(const __grid_constant__ CUtensorMap tmap, int8_t* __restrict__ out
 		quad_sync(quad);
 		uint32_t outw[5];
 #pragma unroll
-		for (int t = 0; t < 5; ++t) {
-			const int j = (int)tq + kSpan * t;
-			outw[t] = j < cnt * 5 ? tilew[j] : 0u;
+		for (int j = 0; j < 5; ++j) {
+			const int i = (int)tq + kSpan * j;
+			outw[j] = i < cnt * 5 ? tilew[i] : 0u;
 		}
 		asm volatile("fence.proxy.async.shared::cta;" ::: "memory");        // generic reads / writes of the tile before its async refill
 		quad_sync(quad);
 		if (tq == 0) issue(span + stride);
-		uint8_t* dst = reinterpret_cast<uint8_t*>(out) + span * kSpan * out_pitch;
-		if (out_pitch == 20 && (reinterpret_cast<uintptr_t>(out) & 3u) == 0) {
-#pragma unroll
-			for (int t = 0; t < 5; ++t) {
-				const int j = (int)tq + kSpan * t;
-				if (j < cnt * 5) reinterpret_cast<uint32_t*>(dst)[j] = outw[t];
-			}
-		} else {
-#pragma unroll
-			for (int t = 0; t < 5; ++t) {
-				const int j = (int)tq + kSpan * t, c = j / 5, q = j - 5 * c;
-				if (j < cnt * 5) {
-					if ((reinterpret_cast<uintptr_t>(out) & 3u) == 0 && (out_pitch & 3) == 0) *reinterpret_cast<uint32_t*>(dst + c * out_pitch + 4 * q) = outw[t];
-					else
-						for (int b = 0; b < 4; ++b) dst[c * out_pitch + 4 * q + b] = (uint8_t)(outw[t] >> (8 * b));
-				}
-			}
-		}
+		store_results<kSpan>(out, span * kSpan, out_pitch, cnt, tq, outw);
 	}
 }
 
-static int env_int(const char* name, int dflt) {
-	const char* e = getenv(name);
-	return e ? atoi(e) : dflt;
-}
-// Tuning knob: RB_SCRAMBLE_THREADS caps the threads per CTA (multiple of 32); default = the fastest measured on B200.
-static int max_threads() {
-	static int v = [] {
-		int t = env_int("RB_SCRAMBLE_THREADS", kMaxThreads);
-		return t >= 32 && t <= kMaxThreads ? t / 32 * 32 : kMaxThreads;
-	}();
-	return v;
-}
+// Defined in rb_scramble_seeded.cuh; its shared-memory attribute is set with the others in ensure_device().
+struct PhiloxKeys;
+__global__ void k_scramble_seeded(PhiloxKeys keys, uint64_t first_cube, int8_t* __restrict__ out, int64_t n, int depth, int out_pitch,
+                                  uint32_t p2_stride, uint32_t n_warps);
 
 static int ensure_device() {
 	static std::mutex mu;
@@ -950,20 +895,19 @@ static int ensure_device() {
 	RB_CUDA(cudaMemcpyToSymbol(g_macro3, h.rows3_inv, sizeof(h.rows3_inv)));
 	RB_CUDA(cudaMemcpyToSymbol(g_macro_tail_inv, h.rows_inv, sizeof(h.rows_inv)));
 	RB_CUDA(cudaMemcpyToSymbol(g_macro3_image, h.image3, sizeof(h.image3)));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<0, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<2, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<3, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<0, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<2, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<3, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
-	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, 4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro3<3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
 	RB_CUDA(cudaFuncSetAttribute(k_scramble_mm<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
 	RB_CUDA(cudaFuncSetAttribute(k_scramble_mm<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
 	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
 	RB_CUDA(cudaFuncSetAttribute(k_scramble_macro<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
+	RB_CUDA(cudaFuncSetAttribute(k_scramble_seeded, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBudget));
 	done[dev] = true;
 	return RB_OK;
 }
@@ -974,28 +918,29 @@ constexpr int64_t kFixedSmem = kTableBytes + kMaxThreads / 32 * 8;        // tab
 static int warps_for(int64_t n, int depth) {
 	if (depth < 20) return 0;                   // the result is written over the head of the 20+ byte action row
 	int64_t w = (kSmemBudget - 1024 - kFixedSmem) / (32 * (int64_t)depth);
-	if (w > max_threads() / 32) w = max_threads() / 32;
+	if (w > kMaxThreads / 32) w = kMaxThreads / 32;
 	const int64_t spread = ((n + 31) / 32 + RB_NUM_SMS - 1) / RB_NUM_SMS;      // small n: use every SM
 	if (w > spread) w = spread;
 	return (int)w;
 }
 
-// 3-move kernel: fixed shared memory and warps per CTA for a given depth (0: use the 2-move kernel)
-static int64_t fixed_smem3(int r2) { return (int64_t)kP1Bytes3 + (int64_t)kP2Rows3 * 4 * r2 + kTailBytes + kMaxThreads / 32 * 8; }
+// 3-move kernels: fixed shared memory (4-copy table + one mbarrier per warp) and warps per CTA for a given depth (0: use the
+// 2-move kernel)
+constexpr int64_t kFixedSmem3 = kTableBytes3 + kMaxThreads / 32 * 8;
 constexpr int kStageThreads = 1024;             // threads that fill the table, whatever the number of working warps
 // row pitch of the action buffers (see the kernel): depth % 128 == 0 rows are padded by 16 bytes
 static int pitch3(int depth) { return depth % 128 == 0 ? depth + 16 : depth; }
 constexpr int64_t kFixedSmemDedup = kImageBytes3 + 16 + kMaxThreads / 32 * 8;   // image + table mbarrier + one per warp
-// Warps per CTA that the shared memory beside the table holds (r2 = 0: the deduplicated table, in multiples of 4 so that the
-// four sub-partitions get equal shares -- 2^24 x 100 moves on B200: 23 warps 0.771 ms, 20 warps 0.757 ms).
-static int64_t smem_warps3(int depth, int r2) {
-	const int64_t w = (kSmemBudget - 16 - (r2 ? fixed_smem3(r2) : kFixedSmemDedup)) / (32 * (int64_t)pitch3(depth));
-	return r2 ? w : w & ~3;
+// Warps per CTA that the shared memory beside the table holds (the deduplicated table: in multiples of 4 so that the four
+// sub-partitions get equal shares -- 2^24 x 100 moves on B200: 23 warps 0.771 ms, 20 warps 0.757 ms).
+static int64_t smem_warps3(int depth, bool dedup) {
+	const int64_t w = (kSmemBudget - 16 - (dedup ? kFixedSmemDedup : kFixedSmem3)) / (32 * (int64_t)pitch3(depth));
+	return dedup ? w & ~3 : w;
 }
-static int warps_for3(int64_t n, int depth, int r2) {
+static int warps_for3(int64_t n, int depth, bool dedup) {
 	if (depth < 20) return 0;
-	int64_t w = smem_warps3(depth, r2);
-	if (w > max_threads() / 32) w = r2 ? max_threads() / 32 : max_threads() / 128 * 4;
+	int64_t w = smem_warps3(depth, dedup);
+	if (w > kMaxThreads / 32) w = kMaxThreads / 32;
 	if (w < 8) return 0;                         // long sequences: too few resident warps to hide the table latency
 	const int64_t spread = ((n + 31) / 32 + RB_NUM_SMS - 1) / RB_NUM_SMS;
 	if (w > spread) w = spread;
@@ -1033,7 +978,7 @@ static bool can_transposed(const uint8_t* actions, int64_t n, int depth) {
 // quads (tiles of 128 cubes x depth bytes) per CTA for the move-major kernel; 0 = does not apply
 static int quads_for(int64_t n, int depth) {
 	if (depth < 20) return 0;
-	int64_t q = (kSmemBudget - 16 - fixed_smem3(1)) / ((int64_t)kSpan * depth);
+	int64_t q = (kSmemBudget - 16 - kFixedSmem3) / ((int64_t)kSpan * depth);
 	if (q > kMaxThreads / 128) q = kMaxThreads / 128;
 	if (q < 2) return 0;
 	const int64_t spread = ((n + kSpan - 1) / kSpan + RB_NUM_SMS - 1) / RB_NUM_SMS;
@@ -1042,7 +987,7 @@ static int quads_for(int64_t n, int depth) {
 }
 
 // move-major actions uint8 [depth][n] (see can_transposed / quads_for)
-static int launch_mm(const uint8_t* actions, int8_t* out, int64_t n, int depth, cudaStream_t st, int out_pitch = 20) {
+static int launch_mm(const uint8_t* actions, int8_t* out, int64_t n, int depth, cudaStream_t st, int out_pitch) {
 	int rc = ensure_device();
 	if (rc != RB_OK) return rc;
 	const int Q = quads_for(n, depth), bh = box_height(depth);
@@ -1056,7 +1001,7 @@ static int launch_mm(const uint8_t* actions, int8_t* out, int64_t n, int depth, 
 	if (cr != CUDA_SUCCESS) return rb_fail(RB_ERR_CUDA, "cuTensorMapEncodeTiled failed for the move-major action array%s%s");
 	const int64_t spans = (n + kSpan - 1) / kSpan, ctas = (spans + Q - 1) / Q;
 	const int grid = (int)(ctas < RB_NUM_SMS ? ctas : RB_NUM_SMS);
-	size_t smem = (size_t)fixed_smem3(1) + (size_t)Q * kSpan * depth + 16;
+	size_t smem = (size_t)kFixedSmem3 + (size_t)Q * kSpan * depth + 16;
 	if (smem < (size_t)kMinSmem3) smem = kMinSmem3;
 	if (depth % 4 == 0) k_scramble_mm<true><<<grid, kStageThreads, smem, st>>>(tmap, out, n, depth, out_pitch, 4u, (uint32_t)Q, bh);
 	else k_scramble_mm<false><<<grid, kStageThreads, smem, st>>>(tmap, out, n, depth, out_pitch, 4u, (uint32_t)Q, bh);
@@ -1064,46 +1009,35 @@ static int launch_mm(const uint8_t* actions, int8_t* out, int64_t n, int depth, 
 	return RB_OK;
 }
 
+// The 3-move kernel on W3 warps per CTA, its mode picked by the depth.
+template <bool kDedup>
+static int launch3(const uint8_t* actions, int8_t* out, int64_t n, int depth, cudaStream_t st, int out_pitch, int W3) {
+	const int64_t ctas = ((n + 31) / 32 + W3 - 1) / W3;
+	const int grid = (int)(ctas < RB_NUM_SMS ? ctas : RB_NUM_SMS);
+	// the 4-copy table is staged by a full CTA however few warps have work (4096 cubes: 128 single-warp CTAs took 70 us to fill it)
+	const int threads = kDedup || W3 * 32 >= kStageThreads ? W3 * 32 : kStageThreads;
+	size_t smem = (size_t)(kDedup ? kFixedSmemDedup : kFixedSmem3) + (size_t)W3 * 32 * pitch3(depth) + 16;
+	if (smem < (size_t)kMinSmem3) smem = kMinSmem3;
+	// element / row stride and remap entry / twist|flip word stride (the 4-copy table's 16-byte stride is a constant)
+	const uint32_t p1 = kDedup ? kRepDedup * 16u : 0u, p2 = kDedup ? 8u : 4u, nw = (uint32_t)W3;
+	if (depth % 4 != 0) k_scramble_macro3<0, kDedup><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, p1, p2, nw);
+	else if (depth % 128 == 0) k_scramble_macro3<3, kDedup><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, p1, p2, nw);
+	else if (depth % 16 == 0) k_scramble_macro3<2, kDedup><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, p1, p2, nw);
+	else k_scramble_macro3<1, kDedup><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, p1, p2, nw);
+	RB_LAUNCHED("scramble_macro3_2024");
+	return RB_OK;
+}
+
 // actions: cube-major uint8 [n][depth]
-static int launch(const uint8_t* actions, int8_t* out, int64_t n, int depth, cudaStream_t st, int out_pitch = 20) {
+static int launch(const uint8_t* actions, int8_t* out, int64_t n, int depth, cudaStream_t st, int out_pitch) {
 	int rc = ensure_device();
 	if (rc != RB_OK) return rc;
-	static const int rows_per = env_int("RB_SCRAMBLE_MOVES_PER_ROW", 3), r2_env = env_int("RB_SCRAMBLE_R2", 1);
 	// The deduplicated table where it leaves room for at least 12 warps (pitch <= 195: every depth from 20 to 195), else the
 	// 4-copy table.  2^24 cubes on B200, deduplicated / 4-copy: depth 100 (20 warps) 0.757 / 0.818 ms, 144 (16) 1.059 / 1.172,
 	// 176 (12) 1.319 / 1.450; with 8 warps it loses at some depths (200: 1.737 / 1.655, 256: 2.222 / 2.170).
-	const bool dedup = smem_warps3(depth, 0) >= 12;
-	const int r2 = dedup ? 0 : (depth % 4 == 0 && depth % 16 != 0 && (r2_env == 2 || r2_env == 4)) ? r2_env : 1;
-	const int W3 = rows_per == 3 ? warps_for3(n, depth, r2) : 0;
-	if (W3 > 0 && dedup) {
-		const int64_t ctas = ((n + 31) / 32 + W3 - 1) / W3;
-		const int grid = (int)(ctas < RB_NUM_SMS ? ctas : RB_NUM_SMS);
-		const size_t smem = (size_t)kFixedSmemDedup + (size_t)W3 * 32 * pitch3(depth) + 16;
-		const uint32_t nw = (uint32_t)W3, es = kRepDedup * 16;
-		if (depth % 4 != 0) k_scramble_macro3<0, 1, true><<<grid, W3 * 32, smem, st>>>(actions, out, n, depth, out_pitch, es, 8u, nw);
-		else if (depth % 128 == 0) k_scramble_macro3<3, 1, true><<<grid, W3 * 32, smem, st>>>(actions, out, n, depth, out_pitch, es, 8u, nw);
-		else if (depth % 16 == 0) k_scramble_macro3<2, 1, true><<<grid, W3 * 32, smem, st>>>(actions, out, n, depth, out_pitch, es, 8u, nw);
-		else k_scramble_macro3<1, 1, true><<<grid, W3 * 32, smem, st>>>(actions, out, n, depth, out_pitch, es, 8u, nw);
-		RB_LAUNCHED("scramble_macro3_2024");
-		return RB_OK;
-	}
-	if (W3 > 0) {
-		const int64_t ctas = ((n + 31) / 32 + W3 - 1) / W3;
-		const int grid = (int)(ctas < RB_NUM_SMS ? ctas : RB_NUM_SMS);
-		// the table is staged by a full CTA however few warps have work (4096 cubes: 128 single-warp CTAs took 70 us to fill it)
-		const int threads = W3 * 32 < kStageThreads ? kStageThreads : W3 * 32;
-		size_t smem = (size_t)fixed_smem3(r2) + (size_t)W3 * 32 * pitch3(depth) + 16;
-		if (smem < (size_t)kMinSmem3) smem = kMinSmem3;
-		const uint32_t nw = (uint32_t)W3;
-		if (depth % 4 != 0) k_scramble_macro3<0, 1, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 4u, nw);
-		else if (depth % 128 == 0) k_scramble_macro3<3, 1, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 4u, nw);
-		else if (depth % 16 == 0) k_scramble_macro3<2, 1, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 4u, nw);
-		else if (r2 == 2) k_scramble_macro3<1, 2, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 8u, nw);
-		else if (r2 == 4) k_scramble_macro3<1, 4, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 16u, nw);
-		else k_scramble_macro3<1, 1, false><<<grid, threads, smem, st>>>(actions, out, n, depth, out_pitch, 0u, 4u, nw);
-		RB_LAUNCHED("scramble_macro3_2024");
-		return RB_OK;
-	}
+	const bool dedup = smem_warps3(depth, true) >= 12;
+	const int W3 = warps_for3(n, depth, dedup);
+	if (W3 > 0) return dedup ? launch3<true>(actions, out, n, depth, st, out_pitch, W3) : launch3<false>(actions, out, n, depth, st, out_pitch, W3);
 	const int W = warps_for(n, depth);
 	const int64_t ctas = ((n + 31) / 32 + W - 1) / W;
 	const int grid = (int)(ctas < RB_NUM_SMS ? ctas : RB_NUM_SMS);

@@ -15,7 +15,7 @@
 // oracle/cube_oracle.py restates the generator in numpy (pinned on the Random123 known-answer vectors).
 //
 // The kernel is the slot-major macro-move kernel without its action buffers: thread per cube, 32 consecutive cubes per
-// warp, table rows from 4 copies in shared memory, results staged per warp and written as 640 contiguous bytes.
+// warp, table rows from 4 copies in shared memory (Rows3), results staged per warp and written as 640 contiguous bytes.
 #pragma once
 #include "rb_scramble_macro.cuh"
 
@@ -73,8 +73,7 @@ k_seeded_actions(PhiloxKeys keys, uint64_t first_cube, uint8_t* __restrict__ act
 }
 
 constexpr int kSeedStage = 640;                  // result staging per warp: 32 cubes x 20 B
-constexpr int kSeedP2Bytes = kP2Rows3 * 4;
-constexpr int kSeedSmem = kP1Bytes3 + kSeedP2Bytes + kTailBytes + kMaxThreads / 32 * kSeedStage;
+constexpr int kSeedSmem = kTableBytes3 + kMaxThreads / 32 * kSeedStage;
 
 __global__ void __launch_bounds__(kMaxThreads, 1)
 k_scramble_seeded(PhiloxKeys keys, uint64_t first_cube, int8_t* __restrict__ out, int64_t n, int depth, int out_pitch, uint32_t p2_stride,
@@ -82,26 +81,11 @@ k_scramble_seeded(PhiloxKeys keys, uint64_t first_cube, int8_t* __restrict__ out
 	// n_warps <= blockDim.x / 32 warps work (small n is spread over all SMs); the whole CTA stages the table
 	extern __shared__ __align__(128) uint8_t smem[];
 	uint8_t* table = smem;                                              // [P1: 4 copies of the 16-byte part | P2 | 2-move tail | staging]
-	uint8_t* tail = smem + kP1Bytes3 + kSeedP2Bytes;
 	const uint32_t lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-	uint32_t* stage = reinterpret_cast<uint32_t*>(tail + kTailBytes + wib * kSeedStage);
-	const uint32_t off1 = smem_u32(table) + (lane & (kRep1 - 1)) * 16u, off2 = smem_u32(table) + (uint32_t)kP1Bytes3;
+	uint32_t* stage = reinterpret_cast<uint32_t*>(smem + kTableBytes3 + wib * kSeedStage);
+	const Rows3<false> t(table, lane, 0u, p2_stride);
 
-	for (int i = threadIdx.x; i < kP2Rows3 * kRep1; i += blockDim.x) {
-		const int row = i / kRep1, c = i % kRep1;
-		if (row < kRows3) {
-			const uint32_t* r = g_macro3 + row * kRowWords;
-			*reinterpret_cast<uint4*>(table + (row * kRep1 + c) * 16) = make_uint4(r[0], r[1], r[2], r[3]);
-			if (c == 0) *reinterpret_cast<uint32_t*>(table + kP1Bytes3 + row * 4) = r[4];
-		} else if (c == 0) {
-			*reinterpret_cast<uint32_t*>(table + kP1Bytes3 + row * 4) = 0u;
-		}
-	}
-	for (int i = threadIdx.x; i < kDevRows; i += blockDim.x) {
-		const uint32_t* r = g_macro_tail_inv + (i < kRows ? i : kRows - 1) * kRowWords;
-		*reinterpret_cast<uint4*>(tail + i * 32) = make_uint4(r[0], r[1], r[2], r[3]);
-		*reinterpret_cast<uint32_t*>(tail + i * 32 + 16) = r[4];
-	}
+	stage_table3(table);
 	__syncthreads();
 	if (wib >= n_warps) return;
 
@@ -115,11 +99,6 @@ k_scramble_seeded(PhiloxKeys keys, uint64_t first_cube, int8_t* __restrict__ out
 			const uint64_t cube = first_cube + (uint64_t)(chunk * 32 + lane);
 			const uint32_t c2 = (uint32_t)cube, c3 = (uint32_t)(cube >> 32);
 			Slots s{0x60402000u, 0xe0c0a080u, 0x03020100u, 0x07060504u, 0x0b0a0908u};
-			auto apply3 = [&](uint32_t r) {
-				const uint32_t o1 = mad_u32(r, 16u * kRep1, off1), o2 = mad_u32(r, p2_stride, off2);
-				apply_row(lds128(o1), lds32(o2), s);
-			};
-			auto fold = [&]() { s.C0 = fold_twists(s.C0); s.C1 = fold_twists(s.C1); };
 			// as in k_scramble_macro3 the INVERSE moves are multiplied in REVERSE order (the tables are laid out for it): the last
 			// Philox block first, inside a block the last triple first, before everything the trailing rem moves
 			{                                                                    // the last block: may be partial, may hold the trailing moves
@@ -130,13 +109,12 @@ k_scramble_seeded(PhiloxKeys keys, uint64_t first_cube, int8_t* __restrict__ out
 				for (int k = 3; k >= 0; --k) {
 					const int q = 4 * j + k;
 					if (j < 0 || q > Q || (q == Q && rem == 0)) continue;
-					const uint32_t t = triple_of(x[k]);
+					const uint32_t tr = triple_of(x[k]);
 					if (q == Q) {                                                  // 1 or 2 moves: 2-move table, index = later + 13 * earlier (12 = none)
-						const uint32_t m0 = t / 144u, m1 = t / 12u % 12u;
-						const uint32_t r = smem_u32(tail) + (rem == 1 ? m0 + 13u * 12u : m1 + 13u * m0) * 32u;
-						apply_row(lds128(r), lds32(r + 16u), s);
+						const uint32_t m0 = tr / 144u, m1 = tr / 12u % 12u;
+						t.apply_tail(s, rem == 1 ? m0 + 13u * 12u : m1 + 13u * m0);
 					} else {
-						apply3(t);
+						t.apply3(s, tr);
 					}
 				}
 			}
@@ -144,10 +122,10 @@ k_scramble_seeded(PhiloxKeys keys, uint64_t first_cube, int8_t* __restrict__ out
 			for (int j = n_blocks - 2; j >= 0; --j) {
 				uint32_t x[4];
 				philox4x32_10((uint32_t)j, 0u, c2, c3, keys, x);
-				apply3(triple_of(x[3])); apply3(triple_of(x[2])); apply3(triple_of(x[1])); apply3(triple_of(x[0]));
-				if (++since == 2) { fold(); since = 0; }
+				t.apply3(s, triple_of(x[3])); t.apply3(s, triple_of(x[2])); t.apply3(s, triple_of(x[1])); t.apply3(s, triple_of(x[0]));
+				if (++since == 2) { fold(s); since = 0; }
 			}
-			fold();
+			fold(s);
 			cubie_major(s, res);
 		}
 		if ((int)lane < cnt) {
@@ -155,36 +133,20 @@ k_scramble_seeded(PhiloxKeys keys, uint64_t first_cube, int8_t* __restrict__ out
 			for (int k = 0; k < 5; ++k) stage[lane * 5 + k] = res[k];
 		}
 		__syncwarp();
-		uint8_t* dst = reinterpret_cast<uint8_t*>(out) + chunk * 32 * out_pitch;
-		const bool word_ok = (reinterpret_cast<uintptr_t>(out) & 3u) == 0 && (out_pitch & 3) == 0;
+		uint32_t outw[5];
 #pragma unroll
-		for (int t = 0; t < 5; ++t) {
-			const int j = lane + 32 * t, c = j / 5, k = j - 5 * c;
-			if (j < cnt * 5) {
-				const uint32_t w = stage[j];
-				if (word_ok) *reinterpret_cast<uint32_t*>(dst + c * out_pitch + 4 * k) = w;
-				else
-					for (int q = 0; q < 4; ++q) dst[c * out_pitch + 4 * k + q] = (uint8_t)(w >> (8 * q));
-			}
+		for (int k = 0; k < 5; ++k) {
+			const int j = lane + 32 * k;
+			outw[k] = j < cnt * 5 ? stage[j] : 0u;
 		}
 		__syncwarp();
+		store_results<32>(out, chunk * 32, out_pitch, cnt, lane, outw);
 	}
 }
 
-static int launch_seeded(uint64_t seed, uint64_t first_cube, int8_t* out, int64_t n, int depth, cudaStream_t st, int out_pitch = 20) {
+static int launch_seeded(uint64_t seed, uint64_t first_cube, int8_t* out, int64_t n, int depth, cudaStream_t st, int out_pitch) {
 	int rc = ensure_device();
 	if (rc != RB_OK) return rc;
-	{
-		static std::mutex mu;
-		static bool attr_done[64] = {};
-		int dev = 0;
-		RB_CUDA(cudaGetDevice(&dev));
-		std::lock_guard<std::mutex> lock(mu);
-		if (dev >= 0 && dev < 64 && !attr_done[dev]) {
-			RB_CUDA(cudaFuncSetAttribute(k_scramble_seeded, cudaFuncAttributeMaxDynamicSharedMemorySize, kSeedSmem));
-			attr_done[dev] = true;
-		}
-	}
 	const int64_t chunks = (n + 31) / 32;
 	int64_t warps = (chunks + RB_NUM_SMS - 1) / RB_NUM_SMS;                 // small n: one chunk per warp on as many SMs as possible
 	if (warps > kMaxThreads / 32) warps = kMaxThreads / 32;

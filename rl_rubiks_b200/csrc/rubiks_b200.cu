@@ -193,51 +193,43 @@ int rb_expand12_bf16(int rep, const int8_t* states, int8_t* children, uint16_t* 
 	return expand12_impl<uint16_t>(rep, states, children, children_oh, solved, n, stream);
 }
 
+// The rbs:: scramble kernels leave each cube's net 20x24 state at pitch 20, or parked at the head of its 6x8x6 output row; the
+// start state then goes in front of it (20x24: k_compose) or is rendered through it (6x8x6: one gather of its sticker records).
+static int scramble_pitch(int rep) { return rep == RB_REP_2024 ? 20 : rb686::kStateBytes; }
+static int scramble_finish(int rep, const int8_t* start, int8_t* out, int64_t n, cudaStream_t st) {
+	if (rep == RB_REP_2024) {
+		if (!start) return RB_OK;
+		rb2024::k_compose<<<rb_grid(n, 8, 8), rb2024::kThreads, 0, st>>>(out, start, n);   // start, then the sequence
+		RB_LAUNCHED("compose_2024");
+		return RB_OK;
+	}
+	rb686::k_render_from2024<<<rb_grid((n + 31) / 32, rb686::kWarps, 8), rb686::kThreads, 0, st>>>(out, start, n);
+	RB_LAUNCHED("render_686");
+	return RB_OK;
+}
+
 int rb_scramble(int rep, const uint8_t* actions, int64_t stride_cube, int64_t stride_move, const int8_t* start,
                 int8_t* out, int64_t n, int32_t depth, rb_stream_t stream) {
 	RB_REQUIRE(rep_ok(rep) && n >= 0 && depth >= 0, "bad rep or size");
 	if (n == 0) return RB_OK;
 	RB_REQUIRE(out && (actions || depth == 0), "null pointer");
 	RB_INIT();
+	if (rep != RB_REP_2024) RB_REQUIRE(aligned(out, 16) && aligned(start, 16), "6x8x6 states must be 16-byte aligned");
+	if (depth > 0 && start != out && (rep == RB_REP_2024 || rbt::host().stickers_ok)) {
+		// slot-major macro-move kernels: cube-major actions [n][depth], or move-major [depth][n] -- the reference's draw shape
+		// (cube.py:226-227) -- by 2-D tensor copies and in-register transposes
+		const bool cube_major = stride_move == 1 && stride_cube == depth && aligned(actions, 16) && rbs::warps_for(n, depth) > 0;
+		if (cube_major || (stride_cube == 1 && stride_move == n && rbs::can_transposed(actions, n, depth) && rbs::quads_for(n, depth) > 0)) {
+			const int rc = cube_major ? rbs::launch(actions, out, n, depth, S(stream), scramble_pitch(rep))
+			                          : rbs::launch_mm(actions, out, n, depth, S(stream), scramble_pitch(rep));
+			return rc != RB_OK ? rc : scramble_finish(rep, start, out, n, S(stream));
+		}
+	}
 	if (rep == RB_REP_2024) {
-		if (depth > 0 && stride_move == 1 && stride_cube == depth && aligned(actions, 16) && rbs::warps_for(n, depth) > 0 && start != out) {
-			int rc = rbs::launch(actions, out, n, depth, S(stream));    // slot-major macro-move kernel (cube-major actions)
-			if (rc != RB_OK || !start) return rc;
-			rb2024::k_compose<<<rb_grid(n, 8, 8), rb2024::kThreads, 0, S(stream)>>>(out, start, n);   // start, then the sequence
-			RB_LAUNCHED("compose_2024");
-			return RB_OK;
-		}
-		if (depth > 0 && stride_cube == 1 && stride_move == n && start != out && rbs::can_transposed(actions, n, depth) && rbs::quads_for(n, depth) > 0) {
-			// move-major actions [depth][n], the reference's draw shape (cube.py:226-227): 2-D tensor copies + in-register transposes
-			int rc = rbs::launch_mm(actions, out, n, depth, S(stream), 20);
-			if (rc != RB_OK || !start) return rc;
-			rb2024::k_compose<<<rb_grid(n, 8, 8), rb2024::kThreads, 0, S(stream)>>>(out, start, n);
-			RB_LAUNCHED("compose_2024");
-			return RB_OK;
-		}
 		rb2024::k_scramble<<<rb_grid(n, rb2024::kThreads, 8), rb2024::kThreads, 0, S(stream)>>>(
 			actions, stride_cube, stride_move, start, out, n, depth);
 		RB_LAUNCHED("scramble_2024");
 	} else {
-		RB_REQUIRE(aligned(out, 16) && aligned(start, 16), "6x8x6 states must be 16-byte aligned");
-		if (depth > 0 && stride_move == 1 && stride_cube == depth && aligned(actions, 16) && rbs::warps_for(n, depth) > 0 &&
-		    rbt::host().stickers_ok && start != out) {
-			// net permutation of the sequence on the slot-major macro-move kernel (20x24 state parked at the head of each
-			// output row), then one gather of the start state's sticker records through it
-			int rc = rbs::launch(actions, out, n, depth, S(stream), rb686::kStateBytes);
-			if (rc != RB_OK) return rc;
-			rb686::k_render_from2024<<<rb_grid((n + 31) / 32, rb686::kWarps, 8), rb686::kThreads, 0, S(stream)>>>(out, start, n);
-			RB_LAUNCHED("render_686");
-			return RB_OK;
-		}
-		if (depth > 0 && stride_cube == 1 && stride_move == n && start != out && rbt::host().stickers_ok && rbs::can_transposed(actions, n, depth) &&
-		    rbs::quads_for(n, depth) > 0) {
-			int rc = rbs::launch_mm(actions, out, n, depth, S(stream), rb686::kStateBytes);
-			if (rc != RB_OK) return rc;
-			rb686::k_render_from2024<<<rb_grid((n + 31) / 32, rb686::kWarps, 8), rb686::kThreads, 0, S(stream)>>>(out, start, n);
-			RB_LAUNCHED("render_686");
-			return RB_OK;
-		}
 		rb686::k_scramble<<<rb_grid(n, rb686::kWarps, 6), rb686::kThreads, 0, S(stream)>>>(
 			actions, stride_cube, stride_move, start, out, n, depth);
 		RB_LAUNCHED("scramble_686");
@@ -682,20 +674,12 @@ int rb_scramble_seeded(int rep, uint64_t seed, uint64_t first_cube, const int8_t
 	if (n == 0) return RB_OK;
 	RB_REQUIRE(out && start != out, "null output (or start aliases out)");
 	RB_INIT();
-	if (rep == RB_REP_2024) {
-		int rc = rbs::launch_seeded(seed, first_cube, out, n, depth, S(stream));
-		if (rc != RB_OK || !start) return rc;
-		rb2024::k_compose<<<rb_grid(n, 8, 8), rb2024::kThreads, 0, S(stream)>>>(out, start, n);       // start, then the sequence
-		RB_LAUNCHED("compose_2024");
-		return RB_OK;
+	if (rep != RB_REP_2024) {
+		RB_REQUIRE(aligned(out, 16) && aligned(start, 16), "6x8x6 states must be 16-byte aligned");
+		RB_REQUIRE(rbt::host().stickers_ok, "sticker tables: the 20x24 and 6x8x6 move tables disagree");
 	}
-	RB_REQUIRE(aligned(out, 16) && aligned(start, 16), "6x8x6 states must be 16-byte aligned");
-	RB_REQUIRE(rbt::host().stickers_ok, "sticker tables: the 20x24 and 6x8x6 move tables disagree");
-	int rc = rbs::launch_seeded(seed, first_cube, out, n, depth, S(stream), rb686::kStateBytes);    // 20x24 state parked at the row head
-	if (rc != RB_OK) return rc;
-	rb686::k_render_from2024<<<rb_grid((n + 31) / 32, rb686::kWarps, 8), rb686::kThreads, 0, S(stream)>>>(out, start, n);
-	RB_LAUNCHED("render_686");
-	return RB_OK;
+	int rc = rbs::launch_seeded(seed, first_cube, out, n, depth, S(stream), scramble_pitch(rep));
+	return rc != RB_OK ? rc : scramble_finish(rep, start, out, n, S(stream));
 }
 
 int rb_as2024(const int8_t* states686, int8_t* states2024, uint8_t* ok, int64_t n, rb_stream_t stream) {

@@ -592,38 +592,6 @@ def test_astar_cost_ties_and_infinities(case):
 
 
 # ---- 5. kernel variants selected by environment variables (read once per process: run in a child) --------------------
-SCRAMBLE_R2_DEPTHS = [20, 24, 36, 100, 228]
-
-
-def _check_scramble(is2024, n, depth, seed, start=False):
-	cube = _cube(is2024)
-	g = np.random.RandomState(seed)
-	acts = g.randint(0, 12, (n, depth)).astype(np.uint8)
-	f, d = O.indices_to_actions(acts)
-	st = O.scramble_many(g.randint(0, 6, (n, 4)), g.randint(0, 2, (n, 4)), is2024) if start else None
-	want = st.copy() if start else np.repeat(O.solved(is2024)[None], n, 0)
-	for m in range(depth):
-		want = O.multi_rotate(want, f[:, m], d[:, m], is2024)
-	got = cube.scramble_batch(acts, start=st) if depth else cube.scramble_batch(acts)
-	assert (got == want).all(), (is2024, n, depth, start)
-
-
-def _child_scramble_r2():
-	for is2024 in (True, False):
-		for depth in SCRAMBLE_R2_DEPTHS:
-			for start in (False, True):
-				_check_scramble(is2024, 4097, depth, depth, start)
-
-
-def _child_scramble_rows():
-	from tests.test_gpu_parity import SCRAMBLE_DEPTHS
-	for is2024 in (True, False):
-		for depth in SCRAMBLE_DEPTHS if is2024 else SCRAMBLE_DEPTHS[::2]:
-			if depth:
-				_check_scramble(is2024, 777, depth, depth)
-	_check_scramble(True, 4097, 100, 1, start=True)
-
-
 def _child_store_policy():
 	from rl_rubiks_b200 import adi
 	for is2024 in (True, False):
@@ -661,10 +629,6 @@ def _child_seq_units():
 
 
 ENV_CASES = {
-	"RB_SCRAMBLE_R2=2": ({"RB_SCRAMBLE_R2": "2"}, _child_scramble_r2),
-	"RB_SCRAMBLE_R2=4": ({"RB_SCRAMBLE_R2": "4"}, _child_scramble_r2),
-	"RB_SCRAMBLE_MOVES_PER_ROW=2": ({"RB_SCRAMBLE_MOVES_PER_ROW": "2"}, _child_scramble_rows),
-	"RB_SCRAMBLE_THREADS=256": ({"RB_SCRAMBLE_THREADS": "256"}, _child_scramble_rows),
 	"RB_STORE_POLICY=0": ({"RB_STORE_POLICY": "0"}, _child_store_policy),
 	"RB_STORE_POLICY=1": ({"RB_STORE_POLICY": "1"}, _child_store_policy),
 	"RB_SEQ_UNITS_PER_SM=1": ({"RB_SEQ_UNITS_PER_SM": "1"}, _child_seq_units),
