@@ -261,6 +261,39 @@ int rb_astar_expand(const rb_astar_view* v, int64_t max_states, int8_t* new_stat
 int rb_astar_commit(const rb_astar_view* v, const float* values, double lambda, const int32_t* new_search,
                     const int32_t* new_index, const int32_t* n_new_total, rb_stream_t stream);
 
+/* ---- batched breadth-first search on the device (BFS.search agents.py:96-123 for K cubes at once; 20x24 representation) ---
+ * K independent searches advance in lockstep.  Every buffer is caller-owned device memory; [K][M] arrays are indexed by the
+ * reference's state index (1-based in discovery order, 0 unused), M >= max_states + 1.  The FIFO of a search is its stored
+ * states: a step pops the next min(N, count - head + 1) of them, tests the budget `len(states) < max_states` before every
+ * pop (agents.py:104), dedups the children against the search's own states, numbers the new ones in (parent, action) order
+ * and stops the search at the first solved new child under a popped parent (not recorded, agents.py:112-118).  States
+ * numbered >= max_states are never popped and are not stored.  A search that runs out of budget stops unsolved. */
+typedef struct rb_bfs_view {
+	int32_t K, M, N;              /* searches (<= 65535), rows per search, pops per search and step */
+	int8_t*  states;              /* [K][M][20] */
+	int32_t* parents;             /* [K][M] FIFO index of the state's parent (agents.py:117) */
+	uint8_t* parent_actions;      /* [K][M] */
+	int32_t* count;               /* [K] states recorded (= len(agent); 0 for a solved start) */
+	int32_t* head;                /* [K] FIFO index of the next pop */
+	uint8_t* won;                 /* [K] */
+	uint8_t* done;                /* [K] */
+	int32_t* solved_parent;       /* [K] FIFO index of the solved child's parent (0: solved start) */
+	uint8_t* solved_action;       /* [K] action from that parent to the solved child */
+	void*    table;               /* shared seen-set, rb_hashset_bytes(capacity) bytes, cleared with rb_hashset_clear */
+	int64_t  capacity;            /* power of two, >= 2 K (M + 12 N) (checked: RB_ERR_CAPACITY below that) */
+	void*    scratch;             /* rb_bfs_scratch_bytes(K, N) bytes */
+} rb_bfs_view;
+/* agents.py:96-123: scratch bytes of a view with K searches and N pops per step. */
+int64_t rb_bfs_scratch_bytes(int32_t K, int32_t N);
+/* agents.py:99-103: roots int8 [K][20] become state 1 of every search (a solved root: found, len 0). */
+int rb_bfs_init(const rb_bfs_view* v, const int8_t* roots, rb_stream_t stream);
+/* agents.py:104-121, one step of every search: up to N pops each.  n_active (int32, device) receives the number of searches
+ * still running after the step; it is the one value a caller reads per step. */
+int rb_bfs_step(const rb_bfs_view* v, int64_t max_states, int32_t* n_active, rb_stream_t stream);
+/* agents.py:112-116: action queue of every search, uint8 [K][L]; lengths int32 [K] (0 when not found or solved at the start,
+ * -1 when the queue is longer than L). */
+int rb_bfs_paths(const rb_bfs_view* v, uint8_t* queues, int32_t* lengths, int32_t L, rb_stream_t stream);
+
 /* ---- host-buffer entry points (end-to-end: H2D + kernels + D2H inside the call) --------------- */
 /* rb_scramble on host buffers; actions uint8 [n][depth] (cube-major), out int8 [n][*shape].  Copies are
  * chunked and double-buffered on internal streams; pinned host memory makes them asynchronous. */

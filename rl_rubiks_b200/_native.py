@@ -67,6 +67,10 @@ SIGNATURES = {
 	"rb_astar_init": (C.c_int, [_p, _p, _p]),
 	"rb_astar_expand": (C.c_int, [_p, _i64, _p, _p, _p, _p, _p, _p]),
 	"rb_astar_commit": (C.c_int, [_p, _p, _f64, _p, _p, _p, _p]),
+	"rb_bfs_scratch_bytes": (_i64, [_i32, _i32]),
+	"rb_bfs_init": (C.c_int, [_p, _p, _p]),
+	"rb_bfs_step": (C.c_int, [_p, _i64, _p, _p]),
+	"rb_bfs_paths": (C.c_int, [_p, _p, _p, _i32, _p]),
 	"rb_as686": (C.c_int, [_p, _p, _i64, _p]),
 	"rb_as2024": (C.c_int, [_p, _p, _p, _i64, _p]),
 	"rb_scramble_seeded": (C.c_int, [C.c_int, C.c_uint64, C.c_uint64, _p, _p, _i64, _i32, _p]),
@@ -91,6 +95,13 @@ class AStarView(C.Structure):
 	_fields_ = [("K", _i32), ("M", _i32), ("N", _i32), ("states", _p), ("G", _p), ("parents", _p), ("parent_actions", _p),
 				("cost", _p), ("in_open", _p), ("count", _p), ("n_sel", _p), ("sel", _p), ("won", _p), ("solved_index", _p),
 				("table", _p), ("capacity", _i64), ("scratch", _p)]
+
+
+class BFSView(C.Structure):
+	"""rb_bfs_view (include/rubiks_b200.h)."""
+	_fields_ = [("K", _i32), ("M", _i32), ("N", _i32), ("states", _p), ("parents", _p), ("parent_actions", _p), ("count", _p),
+				("head", _p), ("won", _p), ("done", _p), ("solved_parent", _p), ("solved_action", _p), ("table", _p),
+				("capacity", _i64), ("scratch", _p)]
 
 
 class RubiksError(RuntimeError):

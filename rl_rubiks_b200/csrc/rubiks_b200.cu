@@ -9,6 +9,7 @@
 #include "rb_adi.cuh"
 #include "rb_frontier.cuh"
 #include "rb_astar.cuh"
+#include "rb_bfs.cuh"
 #include "rb_host.cuh"
 
 #define RB_INIT()                                   \
@@ -664,6 +665,99 @@ int rb_astar_commit(const rb_astar_view* a, const float* values, double lambda, 
 	RB_LAUNCHED("astar_relax_shortcuts");
 	rba::k_finish<<<grid, rba::kThreads, 0, st>>>(v);
 	RB_LAUNCHED("astar_finish");
+	return RB_OK;
+}
+
+// ---- batched BFS ---------------------------------------------------------------------------------------------------------
+int64_t rb_bfs_scratch_bytes(int32_t K, int32_t N) {
+	if (K <= 0 || N <= 0) return 0;
+	const int64_t k = K, P = 12 * (int64_t)N, nbx = (P + rbb::kThreads - 1) / rbb::kThreads;
+	return up16(k * 4) + up16(k * N * 4) + up16(k * P * 4) + up16(k * P) + up16(k * nbx * 4) + up16(k * 4) + up16((k + 1) * 4) +
+	       up16(k * 4) + up16(k * 8) + 64;
+}
+
+// Both views of one rb_bfs_view: the BFS kernels' own, and the A* view the shared probe / flag / totals kernels read (its
+// G / cost / in_open / tmp / solved_index stay null: those kernels never touch them).
+static int bfs_view(const rb_bfs_view* b, rbb::View& v, rba::View& a) {
+	RB_REQUIRE(b, "null view");
+	RB_REQUIRE(b->K > 0 && b->K <= 65535 && b->M > 1 && b->N > 0 && b->N <= (1 << 20), "bad K / M / N (K <= 65535, N <= 2^20)");
+	RB_REQUIRE(b->states && b->parents && b->parent_actions && b->count && b->head && b->won && b->done && b->solved_parent &&
+	           b->solved_action && b->table && b->scratch, "null buffer in view");
+	RB_REQUIRE_TABLE(b->table, b->capacity);
+	// the children of parents dropped by the budget are claimed before the cut is known: a search holds up to M + 12 N keys,
+	// and a full table would drop a child without an error word (k_probe stores slot -1)
+	if (b->capacity < 2 * (int64_t)b->K * (b->M + 12 * (int64_t)b->N))
+		return rb_fail(RB_ERR_CAPACITY, "BFS table capacity must be at least 2 K (M + 12 N) slots%s%s");
+	RB_REQUIRE(aligned(b->scratch, 16) && aligned(b->states, 4), "misaligned buffer");
+	const int64_t K = b->K, P = 12 * (int64_t)b->N, nbx = (P + rbb::kThreads - 1) / rbb::kThreads;
+	v.K = b->K; v.M = b->M; v.N = b->N;
+	v.states = b->states; v.parents = b->parents; v.parent_actions = b->parent_actions; v.count = b->count; v.head = b->head;
+	v.won = b->won; v.done = b->done; v.solved_parent = b->solved_parent; v.solved_action = b->solved_action;
+	v.table = b->table; v.capacity = b->capacity;
+	uint8_t* p = reinterpret_cast<uint8_t*>(b->scratch);
+	v.n_sel = reinterpret_cast<int32_t*>(p); p += up16(K * 4);
+	v.sel = reinterpret_cast<int32_t*>(p); p += up16(K * b->N * 4);
+	a.slot = reinterpret_cast<int32_t*>(p); p += up16(K * P * 4);
+	a.flags = p; p += up16(K * P);
+	a.block_new = reinterpret_cast<int32_t*>(p); p += up16(K * nbx * 4);
+	a.n_new = reinterpret_cast<int32_t*>(p); p += up16(K * 4);
+	a.off = reinterpret_cast<int32_t*>(p); p += up16((K + 1) * 4);
+	v.cut = reinterpret_cast<int32_t*>(p); p += up16(K * 4);
+	v.first_solved = reinterpret_cast<unsigned long long*>(p); p += up16(K * 8);
+	v.n_new_total = reinterpret_cast<int32_t*>(p);
+	a.K = v.K; a.M = v.M; a.N = v.N;
+	a.states = v.states; a.G = nullptr; a.parents = v.parents; a.parent_actions = v.parent_actions; a.cost = nullptr; a.in_open = nullptr;
+	a.count = v.count; a.n_sel = v.n_sel; a.sel = v.sel; a.won = v.won; a.solved_index = nullptr;
+	a.table = v.table; a.capacity = v.capacity; a.tmp = nullptr;
+	return RB_OK;
+}
+
+int rb_bfs_init(const rb_bfs_view* b, const int8_t* roots, rb_stream_t stream) {
+	rbb::View v;
+	rba::View a;
+	int rc = bfs_view(b, v, a);
+	if (rc != RB_OK) return rc;
+	RB_REQUIRE(roots && aligned(roots, 4), "roots must be a 4-byte aligned device pointer");
+	RB_INIT();
+	rbb::k_init<<<(v.K + rbb::kThreads - 1) / rbb::kThreads, rbb::kThreads, 0, S(stream)>>>(v, roots);
+	RB_LAUNCHED("bfs_init");
+	return RB_OK;
+}
+
+int rb_bfs_step(const rb_bfs_view* b, int64_t max_states, int32_t* n_active, rb_stream_t stream) {
+	rbb::View v;
+	rba::View a;
+	int rc = bfs_view(b, v, a);
+	if (rc != RB_OK) return rc;
+	RB_REQUIRE(n_active, "null n_active");
+	RB_REQUIRE(max_states >= 1 && max_states < v.M, "M must exceed max_states (index 0 is unused)");
+	RB_INIT();
+	cudaStream_t st = S(stream);
+	const dim3 grid(v.nbx(), v.K);
+	rbb::k_pop<<<dim3((v.N + rbb::kThreads - 1) / rbb::kThreads, v.K), rbb::kThreads, 0, st>>>(v, max_states, n_active);
+	RB_LAUNCHED("bfs_pop");
+	rba::k_probe<<<grid, rba::kThreads, 0, st>>>(a);
+	RB_LAUNCHED("bfs_probe");
+	rba::k_flag<<<grid, rba::kThreads, 0, st>>>(a);
+	RB_LAUNCHED("bfs_flag");
+	rba::k_totals<<<1, 1024, 0, st>>>(a, v.n_new_total);
+	RB_LAUNCHED("bfs_totals");
+	rbb::k_assign<<<grid, rbb::kThreads, 0, st>>>(v, a, max_states);
+	RB_LAUNCHED("bfs_assign");
+	rbb::k_finish<<<grid, rbb::kThreads, 0, st>>>(v, a, max_states, n_active);
+	RB_LAUNCHED("bfs_finish");
+	return RB_OK;
+}
+
+int rb_bfs_paths(const rb_bfs_view* b, uint8_t* queues, int32_t* lengths, int32_t L, rb_stream_t stream) {
+	rbb::View v;
+	rba::View a;
+	int rc = bfs_view(b, v, a);
+	if (rc != RB_OK) return rc;
+	RB_REQUIRE(queues && lengths && L > 0, "null output or L <= 0");
+	RB_INIT();
+	rbb::k_paths<<<(v.K + rbb::kThreads - 1) / rbb::kThreads, rbb::kThreads, 0, S(stream)>>>(v, queues, lengths, L);
+	RB_LAUNCHED("bfs_paths");
 	return RB_OK;
 }
 

@@ -4,8 +4,9 @@ Python dict keyed on `state.tostring()` (reference: librubiks/solving/agents.py:
 
 `StateHashSet` is an open-addressing hash set on the packed state in caller-owned (torch) device memory with the
 reference's index semantics: states are numbered 1, 2, ... in insertion order, a batch is numbered in batch order,
-in-batch duplicates resolve to their first occurrence (agents.py:286-306).  `BFS` (layer-synchronous) and `AStarBatch`
-(K searches in lockstep, open list and relaxation on the device) carry the reference agents' interface
+in-batch duplicates resolve to their first occurrence (agents.py:286-306).  `BFS` (layer-synchronous), `BFSBatch` (K
+breadth-first searches in lockstep on the device) and `AStarBatch` (K searches in lockstep, open list and relaxation on the
+device) carry the reference agents' interface
 (`search(state, time_limit, max_states) -> bool`, `action_queue`, `len(agent)`).  The reference's host-side agent loops
 (single-search A* around a heapq, MCTS' UCB walk) are not part of the product: tests/agent_harness.py replays them around
 `StateHashSet` to check the device primitives against traces recorded from the reference.
@@ -280,6 +281,22 @@ class BFS(Agent):
 		return "Breadth-first search"
 
 
+def _roots2024(states, is2024: bool, dev) -> torch.Tensor:
+	"""Start states (K, *shape) of a batched search as 20-byte device rows: the searches run on the 20x24 form, 6x8x6 starts
+	are converted (`rb_as2024`); an unreachable 6x8x6 start is an IndexError."""
+	s = states if isinstance(states, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(states, dtype=np.int8))
+	s = s.to(device=dev, dtype=torch.int8)
+	if is2024:
+		return s.reshape(-1, 20).contiguous()
+	s = s.reshape(-1, 6, 8, 6).contiguous()
+	roots = torch.empty(s.shape[0], 20, dtype=torch.int8, device=dev)
+	ok = torch.empty(s.shape[0], dtype=torch.uint8, device=dev)
+	N.check(N.lib.rb_as2024(N.ptr(s), N.ptr(roots), N.ptr(ok), s.shape[0], N.stream_handle()))
+	if not bool(ok.all().item()):
+		raise IndexError("a 6x8x6 start state is not a reachable cube")
+	return roots
+
+
 class AStarBatch:
 	"""Batched weighted A* (agents.py:171-413) for K cubes at once, entirely on the device (SURVEY 8f rows N2 + N3): open
 	list, seen-set, G / parent relaxation and the pop of the N cheapest states per search are kernels (csrc/rb_astar.cuh);
@@ -364,17 +381,7 @@ class AStarBatch:
 		return f"AStar (lambda={self.lambda_}, N={self.expansions})"
 
 	def _roots(self, states) -> torch.Tensor:
-		s = states if isinstance(states, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(states, dtype=np.int8))
-		s = s.to(device=self.dev, dtype=torch.int8)
-		if self.is2024:
-			return s.reshape(-1, 20).contiguous()
-		s = s.reshape(-1, 6, 8, 6).contiguous()
-		roots = torch.empty(s.shape[0], 20, dtype=torch.int8, device=self.dev)
-		ok = torch.empty(s.shape[0], dtype=torch.uint8, device=self.dev)
-		N.check(N.lib.rb_as2024(N.ptr(s), N.ptr(roots), N.ptr(ok), s.shape[0], N.stream_handle()))
-		if not bool(ok.all().item()):
-			raise IndexError("a 6x8x6 start state is not a reachable cube")
-		return roots
+		return _roots2024(states, self.is2024, self.dev)
 
 	def _step_calls(self, max_states: int):
 		"""The two halves of a step as callables: plain C-ABI calls, or replays of their CUDA graphs (captured once per buffer set
@@ -471,3 +478,99 @@ class AStarBatch:
 					i = int(parents[i])
 			queues.append(q)
 		return won, queues, count
+
+
+class BFSBatch:
+	"""Breadth-first search (agents.py:92-129) for K cubes at once, entirely on the device (csrc/rb_bfs.cuh): every search pops
+	up to `_step` parents of its FIFO per step, with the reference's budget test before every pop, and all searches share one
+	seen-set.  The host reads one counter per step (searches still running).  Each search's found flag, `len(agent)` and
+	action queue are `BFS.search`'s for the same start and `max_states` (tests/golden/bfs_budget.npz).
+
+	Both representations (the module flag, or `is2024`): the searches run on the 20-byte states, 6x8x6 starts are converted
+	on the way in (`rb_as2024`)."""
+
+	_step = 2048                                   # parents popped per search and step (changes no result)
+	_queue_len = 16                                # a FIFO index below 2^29 has BFS depth <= 9
+	_default_max_states = 1 << 20                  # buffers are sized by the state budget: a search limited by time only gets this one
+
+	def __init__(self, is2024: bool | None = None):
+		N.require_cuda()
+		self.is2024 = cube.get_is2024() if is2024 is None else bool(is2024)
+		self.dev = torch.device("cuda", torch.cuda.current_device())
+		self.action_queue = deque()
+		self._explored_states = 0
+
+	def __len__(self):
+		return self._explored_states
+
+	def __str__(self):
+		return "Breadth-first search (batched)"
+
+	def _alloc(self, K: int, max_states: int):
+		dev, Nx = self.dev, self._step
+		M = max_states + 1
+		if getattr(self, "_shape", None) == (K, M, Nx):           # every field a search reads is re-initialised by rb_bfs_init /
+			return                                                # rb_hashset_clear
+		self._shape = (K, M, Nx)
+		self.K, self.M = K, M
+		self.states = torch.empty(K, M, 20, dtype=torch.int8, device=dev)
+		self.parents = torch.zeros(K, M, dtype=torch.int32, device=dev)
+		self.parent_actions = torch.zeros(K, M, dtype=torch.uint8, device=dev)
+		self.count = torch.zeros(K, dtype=torch.int32, device=dev)
+		self.head = torch.zeros(K, dtype=torch.int32, device=dev)
+		self.won = torch.zeros(K, dtype=torch.uint8, device=dev)
+		self.done = torch.zeros(K, dtype=torch.uint8, device=dev)
+		self.solved_parent = torch.zeros(K, dtype=torch.int32, device=dev)
+		self.solved_action = torch.zeros(K, dtype=torch.uint8, device=dev)
+		# load <= 1/2: a search holds at most M states plus the children of one step's dropped parents
+		self.capacity = _pow2_at_least(2 * K * (M + 12 * Nx))
+		self.table = torch.empty(N.lib.rb_hashset_bytes(self.capacity), dtype=torch.uint8, device=dev)
+		self.scratch = torch.empty(N.lib.rb_bfs_scratch_bytes(K, Nx), dtype=torch.uint8, device=dev)
+		self.n_active = torch.zeros(1, dtype=torch.int32, device=dev)
+		self.n_active_host = torch.zeros(1, dtype=torch.int32, pin_memory=True)
+		self.queues = torch.zeros(K, self._queue_len, dtype=torch.uint8, device=dev)
+		self.lengths = torch.zeros(K, dtype=torch.int32, device=dev)
+		self.view = N.BFSView(K, M, Nx, *(N.ptr(t) for t in (self.states, self.parents, self.parent_actions, self.count, self.head, self.won,
+															 self.done, self.solved_parent, self.solved_action, self.table)),
+							  self.capacity, N.ptr(self.scratch))
+
+	def search(self, state, time_limit: float = None, max_states: int = None) -> bool:
+		"""`BFS.search(state, time_limit, max_states)` for one cube on the batched machinery (K = 1): fills `action_queue` and
+		`len(agent)`.  The time limit is tested before every step."""
+		assert time_limit or max_states
+		won, queues, count = self.search_many(np.asarray(state)[None] if not isinstance(state, torch.Tensor) else state[None],
+											  int(max_states or self._default_max_states), time_limit=time_limit)
+		self.action_queue = deque(queues[0])
+		self._explored_states = int(count[0])
+		return bool(won[0])
+
+	@torch.no_grad()
+	def search_many(self, states, max_states: int, time_limit: float | None = None):
+		"""states: (K, *shape) int8 (numpy or CUDA tensor).  Returns (found bool (K,), action queues: list of K lists,
+		len per search int (K,)), the three things `BFS.search` leaves behind for one cube (len 0 for a solved start)."""
+		import ctypes as C
+		t0 = perf_counter()
+		roots = _roots2024(states, self.is2024, self.dev)
+		self._alloc(roots.shape[0], int(max_states))
+		sh = N.stream_handle()
+		v = C.byref(self.view)
+		N.check(N.lib.rb_hashset_clear(N.ptr(self.table), self.capacity, sh))
+		N.check(N.lib.rb_bfs_init(v, N.ptr(roots), sh))
+		self.steps = 0
+		l0 = N.lib.rb_launch_count()
+		while time_limit is None or perf_counter() - t0 < time_limit:
+			N.check(N.lib.rb_bfs_step(v, int(max_states), N.ptr(self.n_active), sh))
+			self.steps += 1
+			self.n_active_host.copy_(self.n_active, non_blocking=True)          # the one host read of a step
+			torch.cuda.current_stream().synchronize()
+			if int(self.n_active_host[0]) == 0:
+				break
+		N.check(N.lib.rb_bfs_paths(v, N.ptr(self.queues), N.ptr(self.lengths), self._queue_len, sh))
+		self.launches = N.lib.rb_launch_count() - l0
+		won = self.won.bool().cpu().numpy()
+		count = self.count.cpu().numpy().astype(int)
+		lengths = self.lengths.cpu().numpy()
+		if (lengths < 0).any():
+			raise N.RubiksError(f"an action queue is longer than {self._queue_len} moves")
+		queues = self.queues.cpu().numpy()
+		return won, [queues[s, :lengths[s]].tolist() for s in range(len(won))], count
