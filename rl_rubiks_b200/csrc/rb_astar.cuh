@@ -7,21 +7,19 @@
 //     relaxations never re-push: agents.py:316-317, 333-367); popping the N smallest (cost, index) tuples of a heapq is
 //     selecting and sorting the N smallest keys, done per search by one block (chunked bitonic sort + merge with a running
 //     threshold);
-//   * children of the popped parents are generated in (parent order, action order), deduplicated against the search's own
-//     seen-set with the reference's batch-order numbering (same probe / flag / assign scheme as rb_frontier.cuh; the hash
-//     key carries the search id in the 24 free bits of its high word, so all searches share one table);
+//   * children of the popped parents are deduplicated and numbered by the lockstep expansion core (rb_search.cuh: probe,
+//     flag, totals, then k_assign here);
 //   * costs are lambda * G (f64) + H (f32 widened), H = -value, as agents.py:380-383;
 //   * the two relaxation passes are vectorised numpy statements: all right-hand sides are evaluated before any write, and a
 //     duplicate target keeps the LAST assignment (numpy fancy assignment).  They are therefore four small kernels:
 //     evaluate / write "new ways" (targets unique), evaluate "shortcuts", write them per parent in action order.
 // 20x24 representation only.  Buffers are caller-owned (rb_astar_view, include/rubiks_b200.h).
 #pragma once
-#include "rb_common.cuh"
-#include "rb_frontier.cuh"
+#include "rb_search.cuh"
 
 namespace rba {
 
-constexpr int kThreads = 256;
+using rbl::kThreads;
 constexpr int kSelThreads = 1024;
 constexpr unsigned long long kInfKey = ~0ull;
 
@@ -34,30 +32,12 @@ __device__ __forceinline__ unsigned long long sortable(double c) {
 	return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
 }
 
-struct View {                       // device-side copy of rb_astar_view
-	int K, M, N;
-	int8_t* states;
+struct View : rbl::Core {           // device-side copy of rb_astar_view
 	double* G;
-	int32_t* parents;
-	uint8_t* parent_actions;
 	double* cost;
 	uint8_t* in_open;
-	int32_t* count;
-	int32_t* n_sel;
-	int32_t* sel;
-	uint8_t* won;
 	int32_t* solved_index;
-	void* table;
-	int64_t capacity;
-	// scratch, [K][P] with P = 12 N
-	int32_t* slot;
-	uint8_t* flags;                 // bit 0 new, bit 1 old (first & seen), bit 2 relax flag of the running pass
-	double* tmp;
-	int32_t* block_new;             // [K][nbx]
-	int32_t* n_new;                 // [K]
-	int32_t* off;                   // [K + 1]
-	__host__ __device__ int P() const { return 12 * N; }
-	__host__ __device__ int nbx() const { return (12 * N + kThreads - 1) / kThreads; }
+	double* tmp;                    // scratch, [K][P]: the relaxation passes' right-hand sides
 };
 
 __device__ __forceinline__ bool lex_less(unsigned long long ka, uint32_t ia, unsigned long long kb, uint32_t ib) {
@@ -171,122 +151,28 @@ k_select(View v, int64_t max_states, int32_t* __restrict__ n_active) {
 	}
 }
 
-// ---- expansion: probe / flag / totals / assign ----------------------------------------------------------------------------
-__device__ __forceinline__ void child_words(const View& v, int s, int i, const uint8_t* s_lut, uint32_t (&w)[5], int& parent) {
-	parent = v.sel[(int64_t)s * v.N + i / 12];
-	const uint32_t* p = reinterpret_cast<const uint32_t*>(v.states + ((int64_t)s * v.M + parent) * 20);
-#pragma unroll
-	for (int k = 0; k < 5; ++k) w[k] = p[k];
-	rb_move2024(s_lut, (uint32_t)(i % 12), w);
-}
-
-__global__ void __launch_bounds__(kThreads) k_probe(View v) {
-	__shared__ __align__(16) uint8_t s_lut[RB_LUT_BYTES];
-	rb_stage_lut2024(s_lut);
-	__syncthreads();
-	const int s = blockIdx.y, i = blockIdx.x * kThreads + threadIdx.x;
-	if (i >= v.n_sel[s] * 12) return;
-	uint32_t w[5]; int parent;
-	child_words(v, s, i, s_lut, w, parent);
-	rbf::Key k = rbf::pack2024(w);
-	k.hi |= (unsigned long long)s << 40;
-	const rbf::Table t = rbf::table_of(v.table, v.capacity);
-	const int64_t slot = rbf::find_or_claim(t, k);
-	v.slot[(int64_t)s * v.P() + i] = (int32_t)slot;
-	if (slot >= 0) atomicMin(&t.firstpos(slot), (uint32_t)i);
-}
-
-__global__ void __launch_bounds__(kThreads) k_flag(View v) {
-	const int s = blockIdx.y, i = blockIdx.x * kThreads + threadIdx.x;
-	const rbf::Table t = rbf::table_of(v.table, v.capacity);
-	bool is_new = false;
-	if (i < v.n_sel[s] * 12) {
-		const int32_t slot = v.slot[(int64_t)s * v.P() + i];
-		bool seen = false, first = false;
-		if (slot >= 0) { seen = t.val(slot) != 0; first = t.firstpos(slot) == (uint32_t)i; }
-		is_new = first && !seen;
-		v.flags[(int64_t)s * v.P() + i] = (uint8_t)((is_new ? 1 : 0) | ((first && seen) ? 2 : 0));
-	}
-	const int c = __syncthreads_count(is_new);
-	if (threadIdx.x == 0) v.block_new[s * v.nbx() + blockIdx.x] = c;
-}
-
-// n_new[s], exclusive offsets over the searches, grand total.  One block.
-__global__ void __launch_bounds__(1024) k_totals(View v, int32_t* __restrict__ n_new_total) {
-	__shared__ int32_t s_carry, s_warp[32];
-	if (threadIdx.x == 0) s_carry = 0;
-	__syncthreads();
-	for (int base = 0; base < v.K; base += 1024) {
-		const int s = base + threadIdx.x;
-		int32_t x = 0;
-		if (s < v.K) {
-			const int nb = (v.n_sel[s] * 12 + kThreads - 1) / kThreads;
-			for (int b = 0; b < nb; ++b) x += v.block_new[s * v.nbx() + b];
-			v.n_new[s] = x;
-		}
-		int32_t incl = x;
-#pragma unroll
-		for (int o = 1; o < 32; o <<= 1) {
-			const int32_t y = __shfl_up_sync(0xffffffffu, incl, o);
-			if ((threadIdx.x & 31) >= o) incl += y;
-		}
-		if ((threadIdx.x & 31) == 31) s_warp[threadIdx.x >> 5] = incl;
-		__syncthreads();
-		if (threadIdx.x < 32) {
-			int32_t wv = s_warp[threadIdx.x];
-#pragma unroll
-			for (int o = 1; o < 32; o <<= 1) {
-				const int32_t y = __shfl_up_sync(0xffffffffu, wv, o);
-				if (threadIdx.x >= o) wv += y;
-			}
-			s_warp[threadIdx.x] = wv;
-		}
-		__syncthreads();
-		incl += threadIdx.x >= 32 ? s_warp[(threadIdx.x >> 5) - 1] : 0;
-		const int32_t carry = s_carry;
-		if (s < v.K) v.off[s] = carry + incl - x;
-		__syncthreads();
-		if (threadIdx.x == 1023) s_carry = carry + incl;
-		__syncthreads();
-	}
-	if (threadIdx.x == 0) { v.off[v.K] = s_carry; *n_new_total = s_carry; }
-}
-
+// ---- expansion: assign, after rbl::k_probe / k_flag / k_totals ------------------------------------------------------------
 // New children get index count + rank + 1 in batch order, are stored with G / parent / action, tested for solved and
 // appended to the contiguous cost batch (state + search + index) the value net runs on.
 __global__ void __launch_bounds__(kThreads)
 k_assign(View v, int8_t* __restrict__ new_states, int32_t* __restrict__ new_search, int32_t* __restrict__ new_index) {
-	__shared__ __align__(16) uint8_t s_lut[RB_LUT_BYTES];
-	__shared__ int32_t s_warp[kThreads / 32];
-	rb_stage_lut2024(s_lut);
 	const int s = blockIdx.y, i = blockIdx.x * kThreads + threadIdx.x;
-	const bool live = i < v.n_sel[s] * 12;
-	const bool is_new = live && (v.flags[(int64_t)s * v.P() + i] & 1);
-	const int r = rbf::block_rank(is_new, s_warp);               // also orders the LUT staging before use
-	if (!is_new) return;
-	int32_t prefix = 0;
-	for (int b = 0; b < (int)blockIdx.x; ++b) prefix += v.block_new[s * v.nbx() + b];
-	const int k = prefix + r;
-	const int idx = v.count[s] + k + 1;
-	const rbf::Table t = rbf::table_of(v.table, v.capacity);
-	t.val(v.slot[(int64_t)s * v.P() + i]) = idx;
-	uint32_t w[5]; int parent;
-	child_words(v, s, i, s_lut, w, parent);
-	const int64_t row = (int64_t)s * v.M + idx;
+	rbl::NewChild c;
+	if (!rbl::number_new_child(v, s, i, c)) return;
+	const int64_t row = (int64_t)s * v.M + c.idx;
 	uint32_t* dst = reinterpret_cast<uint32_t*>(v.states + row * 20);
-	const int64_t j = (int64_t)v.off[s] + k;
+	const int64_t j = (int64_t)v.off[s] + c.k;
 	uint32_t* dst2 = reinterpret_cast<uint32_t*>(new_states + j * 20);
 #pragma unroll
-	for (int q = 0; q < 5; ++q) { dst[q] = w[q]; dst2[q] = w[q]; }
-	v.G[row] = v.G[(int64_t)s * v.M + parent] + 1.0;
+	for (int q = 0; q < 5; ++q) { dst[q] = c.w[q]; dst2[q] = c.w[q]; }
+	v.G[row] = v.G[(int64_t)s * v.M + c.parent] + 1.0;
 	v.parent_actions[row] = (uint8_t)(i % 12);
-	v.parents[row] = parent;
+	v.parents[row] = c.parent;
 	new_search[j] = s;
-	new_index[j] = idx;
-	const uint32_t* sv = reinterpret_cast<const uint32_t*>(g_solved2024);
-	if ((w[0] == sv[0]) & (w[1] == sv[1]) & (w[2] == sv[2]) & (w[3] == sv[3]) & (w[4] == sv[4])) {
+	new_index[j] = c.idx;
+	if (rbl::is_solved(c.w)) {
 		v.won[s] = 1;
-		v.solved_index[s] = idx;
+		v.solved_index[s] = c.idx;
 	}
 }
 
@@ -348,37 +234,21 @@ __global__ void __launch_bounds__(kThreads) k_relax_shortcuts(View v) {
 
 __global__ void __launch_bounds__(kThreads) k_finish(View v) {
 	const int s = blockIdx.y, i = blockIdx.x * kThreads + threadIdx.x;
-	if (i < v.n_sel[s] * 12) {
-		const int32_t slot = v.slot[(int64_t)s * v.P() + i];
-		if (slot >= 0) rbf::table_of(v.table, v.capacity).firstpos(slot) = 0xffffffffu;
-	}
-	if (i == 0) v.count[s] += v.n_sel[s] ? v.n_new[s] : 0;
+	const int n = v.n_sel[s];
+	rbl::rearm_firstpos(v, s, i, n);
+	if (i == 0) v.count[s] += n ? v.n_new[s] : 0;
 }
 
 // roots: state 1 of every search, G = 0, in the open list with cost 0 (agents.py:233-234)
 __global__ void __launch_bounds__(kThreads) k_init(View v, const int8_t* __restrict__ roots) {
 	const int s = blockIdx.x * kThreads + threadIdx.x;
 	if (s >= v.K) return;
-	uint32_t w[5];
-	const uint32_t* p = reinterpret_cast<const uint32_t*>(roots + (int64_t)s * 20);
-	uint32_t* dst = reinterpret_cast<uint32_t*>(v.states + ((int64_t)s * v.M + 1) * 20);
-#pragma unroll
-	for (int k = 0; k < 5; ++k) { w[k] = p[k]; dst[k] = w[k]; }
-	rbf::Key k = rbf::pack2024(w);
-	k.hi |= (unsigned long long)s << 40;
-	const rbf::Table t = rbf::table_of(v.table, v.capacity);
-	const int64_t slot = rbf::find_or_claim(t, k);
-	if (slot >= 0) t.val(slot) = 1;
-	const uint32_t* sv = reinterpret_cast<const uint32_t*>(g_solved2024);
-	const bool solved = (w[0] == sv[0]) & (w[1] == sv[1]) & (w[2] == sv[2]) & (w[3] == sv[3]) & (w[4] == sv[4]);
+	const bool solved = rbl::init_root(v, s, roots);            // agents.py:230: a solved start returns True at once
 	const int64_t row = (int64_t)s * v.M + 1;
 	v.G[row] = 0.0;
 	v.cost[row] = 0.0;
 	v.in_open[row] = solved ? 0 : 1;
-	v.parents[row] = 0;
-	v.parent_actions[row] = 0;
 	v.count[s] = 1;
-	v.won[s] = solved ? 1 : 0;                                  // agents.py:230: a solved start returns True at once
 	v.solved_index[s] = solved ? 1 : 0;
 	v.n_sel[s] = 0;
 }

@@ -6,8 +6,8 @@
 //   * the FIFO is the stored states themselves: state i of a search is the i-th state its dict records (root = 1, children
 //     numbered in (parent, action) order), so popping is taking head, head + 1, ...; a step pops
 //     take = min(N, count - head + 1) of them;
-//   * children are deduplicated against the search's own seen-set with the batch-order numbering of rb_frontier.cuh, by the
-//     batched A*'s probe / flag / totals kernels (rba::, the search id in the 24 free bits of the key, one shared table);
+//   * children are deduplicated and numbered by the lockstep expansion core the batched A* uses too (rb_search.cuh: probe,
+//     flag, totals, then k_assign here);
 //   * the budget `len(states) < max_states` is tested before every pop (agents.py:104): parent j of the step is admitted iff
 //     count + (new states recorded by the step's parents before j) < max_states.  The admitted parents are a prefix, and the
 //     last one records new state number max_states - count (the cut); later parents' children are dropped;
@@ -16,66 +16,31 @@
 // States numbered >= max_states are never popped: they are counted and entered into the table, not stored.
 // 20x24 representation only.  Buffers are caller-owned (rb_bfs_view, include/rubiks_b200.h).
 #pragma once
-#include "rb_common.cuh"
-#include "rb_frontier.cuh"
-#include "rb_astar.cuh"
+#include "rb_search.cuh"
 
 namespace rbb {
 
-constexpr int kThreads = 256;
-static_assert(kThreads == rba::kThreads, "block_new is laid out by the A* kernels' block size");
+using rbl::kThreads;
 constexpr int32_t kNoCut = 0x7fffffff;
 constexpr unsigned long long kNoSolved = ~0ull;
 
-struct View {                       // device-side copy of rb_bfs_view
-	int K, M, N;
-	int8_t* states;
-	int32_t* parents;
-	uint8_t* parent_actions;
-	int32_t* count;
+struct View : rbl::Core {           // device-side copy of rb_bfs_view; n_sel, sel, cut, first_solved, n_new_total: scratch
 	int32_t* head;
-	uint8_t* won;
 	uint8_t* done;
 	int32_t* solved_parent;
 	uint8_t* solved_action;
-	void* table;
-	int64_t capacity;
-	// scratch
-	int32_t* n_sel;                 // [K]
-	int32_t* sel;                   // [K][N]
 	int32_t* cut;                   // [K] batch position of the child numbered max_states (kNoCut: none this step)
 	unsigned long long* first_solved;   // [K] (rank << 32 | batch position) of the first solved new child
-	int32_t* n_new_total;           // [1] written by rba::k_totals, unused here
-	__host__ __device__ int P() const { return 12 * N; }
-	__host__ __device__ int nbx() const { return (12 * N + kThreads - 1) / kThreads; }
+	int32_t* n_new_total;           // [1] written by rbl::k_totals, unused here
 };
-
-__device__ __forceinline__ bool is_solved2024(const uint32_t (&w)[5]) {
-	const uint32_t* sv = reinterpret_cast<const uint32_t*>(g_solved2024);
-	return (w[0] == sv[0]) & (w[1] == sv[1]) & (w[2] == sv[2]) & (w[3] == sv[3]) & (w[4] == sv[4]);
-}
 
 // roots: state 1 of every search; a solved root is found at once with len 0 (agents.py:99-100)
 __global__ void __launch_bounds__(kThreads) k_init(View v, const int8_t* __restrict__ roots) {
 	const int s = blockIdx.x * kThreads + threadIdx.x;
 	if (s >= v.K) return;
-	uint32_t w[5];
-	const uint32_t* p = reinterpret_cast<const uint32_t*>(roots + (int64_t)s * 20);
-	uint32_t* dst = reinterpret_cast<uint32_t*>(v.states + ((int64_t)s * v.M + 1) * 20);
-#pragma unroll
-	for (int k = 0; k < 5; ++k) { w[k] = p[k]; dst[k] = w[k]; }
-	rbf::Key k = rbf::pack2024(w);
-	k.hi |= (unsigned long long)s << 40;
-	const rbf::Table t = rbf::table_of(v.table, v.capacity);
-	const int64_t slot = rbf::find_or_claim(t, k);
-	if (slot >= 0) t.val(slot) = 1;
-	const bool solved = is_solved2024(w);
-	const int64_t row = (int64_t)s * v.M + 1;
-	v.parents[row] = 0;
-	v.parent_actions[row] = 0;
+	const bool solved = rbl::init_root(v, s, roots);
 	v.count[s] = solved ? 0 : 1;
 	v.head[s] = 1;
-	v.won[s] = solved ? 1 : 0;
 	v.done[s] = solved ? 1 : 0;
 	v.solved_parent[s] = 0;
 	v.solved_action[s] = 0;
@@ -100,45 +65,28 @@ __global__ void __launch_bounds__(kThreads) k_pop(View v, int64_t max_states, in
 
 // New children get index count + rank + 1 in batch order; those that can be popped later (index < M) are stored with parent
 // and action.  The child numbered max_states marks the cut, and the first solved new child is kept by (rank, position).
-__global__ void __launch_bounds__(kThreads) k_assign(View v, rba::View a, int64_t max_states) {
-	__shared__ __align__(16) uint8_t s_lut[RB_LUT_BYTES];
-	__shared__ int32_t s_warp[kThreads / 32];
-	rb_stage_lut2024(s_lut);
+__global__ void __launch_bounds__(kThreads) k_assign(View v, int64_t max_states) {
 	const int s = blockIdx.y, i = blockIdx.x * kThreads + threadIdx.x;
-	const bool live = i < v.n_sel[s] * 12;
-	const bool is_new = live && (a.flags[(int64_t)s * v.P() + i] & 1);
-	const int r = rbf::block_rank(is_new, s_warp);               // also orders the LUT staging before use
-	if (!is_new) return;
-	int32_t prefix = 0;
-	for (int b = 0; b < (int)blockIdx.x; ++b) prefix += a.block_new[s * v.nbx() + b];
-	const int k = prefix + r;
-	const int cnt = v.count[s];
-	const int idx = cnt + k + 1;
-	const rbf::Table t = rbf::table_of(v.table, v.capacity);
-	t.val(a.slot[(int64_t)s * v.P() + i]) = idx;
-	uint32_t w[5]; int parent;
-	rba::child_words(a, s, i, s_lut, w, parent);
-	if (idx < v.M) {
-		const int64_t row = (int64_t)s * v.M + idx;
+	rbl::NewChild c;
+	if (!rbl::number_new_child(v, s, i, c)) return;
+	if (c.idx < v.M) {
+		const int64_t row = (int64_t)s * v.M + c.idx;
 		uint32_t* dst = reinterpret_cast<uint32_t*>(v.states + row * 20);
 #pragma unroll
-		for (int q = 0; q < 5; ++q) dst[q] = w[q];
-		v.parents[row] = parent;
+		for (int q = 0; q < 5; ++q) dst[q] = c.w[q];
+		v.parents[row] = c.parent;
 		v.parent_actions[row] = (uint8_t)(i % 12);
 	}
-	if ((int64_t)k == max_states - cnt - 1) v.cut[s] = i;
-	if (is_solved2024(w)) atomicMin(&v.first_solved[s], ((unsigned long long)k << 32) | (unsigned)i);
+	if ((int64_t)c.idx == max_states) v.cut[s] = i;
+	if (rbl::is_solved(c.w)) atomicMin(&v.first_solved[s], ((unsigned long long)c.k << 32) | (unsigned)i);
 }
 
 // Firstpos re-arm of every probed slot; one thread per search applies the cut and the first-solved rule, advances count and
 // head and counts the searches still running.
-__global__ void __launch_bounds__(kThreads) k_finish(View v, rba::View a, int64_t max_states, int32_t* __restrict__ n_active) {
+__global__ void __launch_bounds__(kThreads) k_finish(View v, int64_t max_states, int32_t* __restrict__ n_active) {
 	const int s = blockIdx.y, i = blockIdx.x * kThreads + threadIdx.x;
 	const int take = v.n_sel[s];
-	if (i < take * 12) {
-		const int32_t slot = a.slot[(int64_t)s * v.P() + i];
-		if (slot >= 0) rbf::table_of(v.table, v.capacity).firstpos(slot) = 0xffffffffu;
-	}
+	rbl::rearm_firstpos(v, s, i, take);
 	if (i != 0 || take == 0) return;
 	const int cnt = v.count[s];
 	const int cut = v.cut[s];
@@ -157,13 +105,13 @@ __global__ void __launch_bounds__(kThreads) k_finish(View v, rba::View a, int64_
 	if (cut != kNoCut) {
 		// the parent of the cut records all its new children; no later parent is popped
 		int adm = (int)(max_states - cnt);
-		const uint8_t* f = a.flags + (int64_t)s * v.P();
+		const uint8_t* f = v.flags + (int64_t)s * v.P();
 		for (int q = cut + 1; q < (cut / 12 + 1) * 12; ++q) adm += f[q] & 1;
 		v.count[s] = cnt + adm;
 		v.done[s] = 1;
 		return;
 	}
-	const int c2 = cnt + a.n_new[s], h2 = v.head[s] + take;
+	const int c2 = cnt + v.n_new[s], h2 = v.head[s] + take;
 	v.count[s] = c2;
 	v.head[s] = h2;
 	if ((int64_t)c2 >= max_states || h2 > c2) { v.done[s] = 1; return; }

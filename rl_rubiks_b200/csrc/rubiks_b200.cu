@@ -8,6 +8,7 @@
 #include "rb_cube686.cuh"
 #include "rb_adi.cuh"
 #include "rb_frontier.cuh"
+#include "rb_search.cuh"
 #include "rb_astar.cuh"
 #include "rb_bfs.cuh"
 #include "rb_host.cuh"
@@ -563,39 +564,72 @@ int rb_check_range(int rep, const int8_t* states, int64_t n_states, const uint8_
 	return RB_OK;
 }
 
-// ---- batched A* ----------------------------------------------------------------------------------------------------------
-static inline int64_t up16(int64_t x) { return (x + 15) / 16 * 16; }
+// ---- batched searches: view checks and scratch layouts ------------------------------------------------------------------
+// A search's scratch: its arrays one after the other at 16-byte boundaries, then 64 spare bytes.  With a null base only the
+// size is counted, so sizing and carving share one layout per search.
+extern "C++" {
+template <class T> static void carve(T*& dst, uint8_t* base, int64_t& used, int64_t n) {
+	dst = base ? reinterpret_cast<T*>(base + used) : nullptr;
+	used += rbf::up16(n * (int64_t)sizeof(T));
+}
 
+static int64_t carve_expansion(rbl::Core& v, uint8_t* base) {
+	const int64_t K = v.K, P = 12 * (int64_t)v.N;
+	int64_t used = 0;
+	carve(v.slot, base, used, K * P);
+	carve(v.flags, base, used, K * P);
+	carve(v.block_new, base, used, K * ((P + rbl::kThreads - 1) / rbl::kThreads));
+	carve(v.n_new, base, used, K);
+	carve(v.off, base, used, K + 1);
+	return used;
+}
+
+static int64_t scratch(rba::View& v, uint8_t* base) {
+	int64_t used = carve_expansion(v, base);
+	carve(v.tmp, base, used, (int64_t)v.K * 12 * v.N);
+	return used + 64;
+}
+
+static int64_t scratch(rbb::View& v, uint8_t* base) {
+	int64_t used = carve_expansion(v, base);
+	carve(v.n_sel, base, used, v.K);
+	carve(v.sel, base, used, (int64_t)v.K * v.N);
+	carve(v.cut, base, used, v.K);
+	carve(v.first_solved, base, used, v.K);
+	carve(v.n_new_total, base, used, 0);                        // written by k_totals, unused: the first of the spare bytes
+	return used + 64;
+}
+
+// The checks both views share, in order; then the Core is filled and the scratch carved.  An entry point checks its own
+// arguments only after this, so a bad view is what a call reports first.  keys: slots one search can claim (a full table drops
+// a child without an error word, k_probe stores slot -1: 2 K keys slots keep every search at load <= 1/2).
+template <class AbiView, class View>
+static int core_view(const AbiView* a, bool n_ok, int64_t keys, bool own_set, bool own_aligned, View& v) {
+	RB_REQUIRE(a->K > 0 && a->K <= 65535 && a->M > 1 && a->N > 0 && n_ok, "bad K / M / N (K <= 65535; N <= 1024 for A*, 2^20 for BFS)");
+	RB_REQUIRE(a->states && a->parents && a->parent_actions && a->count && a->won && a->table && a->scratch && own_set, "null buffer in view");
+	RB_REQUIRE_TABLE(a->table, a->capacity);
+	if (a->capacity < 2 * (int64_t)a->K * keys)
+		return rb_fail(RB_ERR_CAPACITY, "table capacity must be at least 2 K M slots for A*, 2 K (M + 12 N) for BFS%s%s");
+	RB_REQUIRE(aligned(a->scratch, 16) && aligned(a->states, 4) && own_aligned, "misaligned buffer");
+	v.K = a->K; v.M = a->M; v.N = a->N;
+	v.states = a->states; v.parents = a->parents; v.parent_actions = a->parent_actions; v.count = a->count; v.won = a->won;
+	v.table = a->table; v.capacity = a->capacity;
+	scratch(v, static_cast<uint8_t*>(a->scratch));
+	return RB_OK;
+}
+}  // extern "C++"
+
+// ---- batched A* ----------------------------------------------------------------------------------------------------------
 int64_t rb_astar_scratch_bytes(int32_t K, int32_t N) {
-	if (K <= 0 || N <= 0) return 0;
-	const int64_t P = 12 * (int64_t)N, nbx = (P + rba::kThreads - 1) / rba::kThreads;
-	return up16(K * P * 4) + up16(K * P) + up16(K * P * 8) + up16(K * nbx * 4) + up16((int64_t)K * 4) + up16((int64_t)(K + 1) * 4) + 64;
+	rba::View v{{K, 0, N}};
+	return K > 0 && N > 0 ? scratch(v, nullptr) : 0;
 }
 
 static int astar_view(const rb_astar_view* a, rba::View& v) {
 	RB_REQUIRE(a, "null view");
-	RB_REQUIRE(a->K > 0 && a->K <= 65535 && a->M > 1 && a->N > 0 && a->N <= 1024, "bad K / M / N (K <= 65535, N <= 1024)");
-	RB_REQUIRE(a->states && a->G && a->parents && a->parent_actions && a->cost && a->in_open && a->count && a->n_sel && a->sel && a->won &&
-	           a->solved_index && a->table && a->scratch, "null buffer in view");
-	RB_REQUIRE_TABLE(a->table, a->capacity);
-	// a full table drops a child without an error word (k_probe stores slot -1): at least 2 K M slots keep every search's
-	// M states at load <= 1/2
-	if (a->capacity < 2 * (int64_t)a->K * a->M)
-		return rb_fail(RB_ERR_CAPACITY, "A* table capacity must be at least 2 K M slots%s%s");
-	RB_REQUIRE(aligned(a->scratch, 16) && aligned(a->states, 4) && aligned(a->G, 8) && aligned(a->cost, 8), "misaligned buffer");
-	const int64_t K = a->K, P = 12 * (int64_t)a->N, nbx = (P + rba::kThreads - 1) / rba::kThreads;
-	v.K = a->K; v.M = a->M; v.N = a->N;
-	v.states = a->states; v.G = a->G; v.parents = a->parents; v.parent_actions = a->parent_actions; v.cost = a->cost; v.in_open = a->in_open;
-	v.count = a->count; v.n_sel = a->n_sel; v.sel = a->sel; v.won = a->won; v.solved_index = a->solved_index;
-	v.table = a->table; v.capacity = a->capacity;
-	uint8_t* p = reinterpret_cast<uint8_t*>(a->scratch);
-	v.slot = reinterpret_cast<int32_t*>(p); p += up16(K * P * 4);
-	v.flags = p; p += up16(K * P);
-	v.tmp = reinterpret_cast<double*>(p); p += up16(K * P * 8);
-	v.block_new = reinterpret_cast<int32_t*>(p); p += up16(K * nbx * 4);
-	v.n_new = reinterpret_cast<int32_t*>(p); p += up16(K * 4);
-	v.off = reinterpret_cast<int32_t*>(p);
-	return RB_OK;
+	v.G = a->G; v.cost = a->cost; v.in_open = a->in_open; v.n_sel = a->n_sel; v.sel = a->sel; v.solved_index = a->solved_index;
+	return core_view(a, a->N <= 1024, a->M, a->G && a->cost && a->in_open && a->n_sel && a->sel && a->solved_index,
+	                 aligned(a->G, 8) && aligned(a->cost, 8), v);
 }
 
 int rb_astar_init(const rb_astar_view* a, const int8_t* roots, rb_stream_t stream) {
@@ -604,7 +638,7 @@ int rb_astar_init(const rb_astar_view* a, const int8_t* roots, rb_stream_t strea
 	if (rc != RB_OK) return rc;
 	RB_REQUIRE(roots && aligned(roots, 4), "roots must be a 4-byte aligned device pointer");
 	RB_INIT();
-	rba::k_init<<<(v.K + rba::kThreads - 1) / rba::kThreads, rba::kThreads, 0, S(stream)>>>(v, roots);
+	rba::k_init<<<(v.K + rbl::kThreads - 1) / rbl::kThreads, rbl::kThreads, 0, S(stream)>>>(v, roots);
 	RB_LAUNCHED("astar_init");
 	return RB_OK;
 }
@@ -633,13 +667,13 @@ int rb_astar_expand(const rb_astar_view* a, int64_t max_states, int8_t* new_stat
 	}
 	rba::k_select<<<v.K, rba::kSelThreads, rba::kSelSmem, st>>>(v, max_states, n_active);
 	RB_LAUNCHED("astar_select");
-	rba::k_probe<<<grid, rba::kThreads, 0, st>>>(v);
+	rbl::k_probe<<<grid, rbl::kThreads, 0, st>>>(v);
 	RB_LAUNCHED("astar_probe");
-	rba::k_flag<<<grid, rba::kThreads, 0, st>>>(v);
+	rbl::k_flag<<<grid, rbl::kThreads, 0, st>>>(v);
 	RB_LAUNCHED("astar_flag");
-	rba::k_totals<<<1, 1024, 0, st>>>(v, n_new_total);
+	rbl::k_totals<<<1, 1024, 0, st>>>(v, n_new_total);
 	RB_LAUNCHED("astar_totals");
-	rba::k_assign<<<grid, rba::kThreads, 0, st>>>(v, new_states, new_search, new_index);
+	rba::k_assign<<<grid, rbl::kThreads, 0, st>>>(v, new_states, new_search, new_index);
 	RB_LAUNCHED("astar_assign");
 	return RB_OK;
 }
@@ -653,110 +687,76 @@ int rb_astar_commit(const rb_astar_view* a, const float* values, double lambda, 
 	cudaStream_t st = S(stream);
 	const dim3 grid(v.nbx(), v.K);
 	const int64_t worst = (int64_t)v.K * v.P();
-	rba::k_push<<<(unsigned)((worst + rba::kThreads - 1) / rba::kThreads), rba::kThreads, 0, st>>>(v, values, lambda, new_search, new_index, n_new_total);
+	rba::k_push<<<(unsigned)((worst + rbl::kThreads - 1) / rbl::kThreads), rbl::kThreads, 0, st>>>(v, values, lambda, new_search, new_index, n_new_total);
 	RB_LAUNCHED("astar_push");
-	rba::k_relax_eval<<<grid, rba::kThreads, 0, st>>>(v, 0);
+	rba::k_relax_eval<<<grid, rbl::kThreads, 0, st>>>(v, 0);
 	RB_LAUNCHED("astar_relax_eval0");
-	rba::k_relax_new_ways<<<grid, rba::kThreads, 0, st>>>(v);
+	rba::k_relax_new_ways<<<grid, rbl::kThreads, 0, st>>>(v);
 	RB_LAUNCHED("astar_relax_new_ways");
-	rba::k_relax_eval<<<grid, rba::kThreads, 0, st>>>(v, 1);
+	rba::k_relax_eval<<<grid, rbl::kThreads, 0, st>>>(v, 1);
 	RB_LAUNCHED("astar_relax_eval1");
-	rba::k_relax_shortcuts<<<dim3((v.N + rba::kThreads - 1) / rba::kThreads, v.K), rba::kThreads, 0, st>>>(v);
+	rba::k_relax_shortcuts<<<dim3((v.N + rbl::kThreads - 1) / rbl::kThreads, v.K), rbl::kThreads, 0, st>>>(v);
 	RB_LAUNCHED("astar_relax_shortcuts");
-	rba::k_finish<<<grid, rba::kThreads, 0, st>>>(v);
+	rba::k_finish<<<grid, rbl::kThreads, 0, st>>>(v);
 	RB_LAUNCHED("astar_finish");
 	return RB_OK;
 }
 
 // ---- batched BFS ---------------------------------------------------------------------------------------------------------
 int64_t rb_bfs_scratch_bytes(int32_t K, int32_t N) {
-	if (K <= 0 || N <= 0) return 0;
-	const int64_t k = K, P = 12 * (int64_t)N, nbx = (P + rbb::kThreads - 1) / rbb::kThreads;
-	return up16(k * 4) + up16(k * N * 4) + up16(k * P * 4) + up16(k * P) + up16(k * nbx * 4) + up16(k * 4) + up16((k + 1) * 4) +
-	       up16(k * 4) + up16(k * 8) + 64;
+	rbb::View v{{K, 0, N}};
+	return K > 0 && N > 0 ? scratch(v, nullptr) : 0;
 }
 
-// Both views of one rb_bfs_view: the BFS kernels' own, and the A* view the shared probe / flag / totals kernels read (its
-// G / cost / in_open / tmp / solved_index stay null: those kernels never touch them).
-static int bfs_view(const rb_bfs_view* b, rbb::View& v, rba::View& a) {
+static int bfs_view(const rb_bfs_view* b, rbb::View& v) {
 	RB_REQUIRE(b, "null view");
-	RB_REQUIRE(b->K > 0 && b->K <= 65535 && b->M > 1 && b->N > 0 && b->N <= (1 << 20), "bad K / M / N (K <= 65535, N <= 2^20)");
-	RB_REQUIRE(b->states && b->parents && b->parent_actions && b->count && b->head && b->won && b->done && b->solved_parent &&
-	           b->solved_action && b->table && b->scratch, "null buffer in view");
-	RB_REQUIRE_TABLE(b->table, b->capacity);
-	// the children of parents dropped by the budget are claimed before the cut is known: a search holds up to M + 12 N keys,
-	// and a full table would drop a child without an error word (k_probe stores slot -1)
-	if (b->capacity < 2 * (int64_t)b->K * (b->M + 12 * (int64_t)b->N))
-		return rb_fail(RB_ERR_CAPACITY, "BFS table capacity must be at least 2 K (M + 12 N) slots%s%s");
-	RB_REQUIRE(aligned(b->scratch, 16) && aligned(b->states, 4), "misaligned buffer");
-	const int64_t K = b->K, P = 12 * (int64_t)b->N, nbx = (P + rbb::kThreads - 1) / rbb::kThreads;
-	v.K = b->K; v.M = b->M; v.N = b->N;
-	v.states = b->states; v.parents = b->parents; v.parent_actions = b->parent_actions; v.count = b->count; v.head = b->head;
-	v.won = b->won; v.done = b->done; v.solved_parent = b->solved_parent; v.solved_action = b->solved_action;
-	v.table = b->table; v.capacity = b->capacity;
-	uint8_t* p = reinterpret_cast<uint8_t*>(b->scratch);
-	v.n_sel = reinterpret_cast<int32_t*>(p); p += up16(K * 4);
-	v.sel = reinterpret_cast<int32_t*>(p); p += up16(K * b->N * 4);
-	a.slot = reinterpret_cast<int32_t*>(p); p += up16(K * P * 4);
-	a.flags = p; p += up16(K * P);
-	a.block_new = reinterpret_cast<int32_t*>(p); p += up16(K * nbx * 4);
-	a.n_new = reinterpret_cast<int32_t*>(p); p += up16(K * 4);
-	a.off = reinterpret_cast<int32_t*>(p); p += up16((K + 1) * 4);
-	v.cut = reinterpret_cast<int32_t*>(p); p += up16(K * 4);
-	v.first_solved = reinterpret_cast<unsigned long long*>(p); p += up16(K * 8);
-	v.n_new_total = reinterpret_cast<int32_t*>(p);
-	a.K = v.K; a.M = v.M; a.N = v.N;
-	a.states = v.states; a.G = nullptr; a.parents = v.parents; a.parent_actions = v.parent_actions; a.cost = nullptr; a.in_open = nullptr;
-	a.count = v.count; a.n_sel = v.n_sel; a.sel = v.sel; a.won = v.won; a.solved_index = nullptr;
-	a.table = v.table; a.capacity = v.capacity; a.tmp = nullptr;
-	return RB_OK;
+	v.head = b->head; v.done = b->done; v.solved_parent = b->solved_parent; v.solved_action = b->solved_action;
+	// the children of parents dropped by the budget are claimed before the cut is known: a search holds up to M + 12 N keys
+	return core_view(b, b->N <= (1 << 20), b->M + 12 * (int64_t)b->N, b->head && b->done && b->solved_parent && b->solved_action, true, v);
 }
 
 int rb_bfs_init(const rb_bfs_view* b, const int8_t* roots, rb_stream_t stream) {
 	rbb::View v;
-	rba::View a;
-	int rc = bfs_view(b, v, a);
+	int rc = bfs_view(b, v);
 	if (rc != RB_OK) return rc;
 	RB_REQUIRE(roots && aligned(roots, 4), "roots must be a 4-byte aligned device pointer");
 	RB_INIT();
-	rbb::k_init<<<(v.K + rbb::kThreads - 1) / rbb::kThreads, rbb::kThreads, 0, S(stream)>>>(v, roots);
+	rbb::k_init<<<(v.K + rbl::kThreads - 1) / rbl::kThreads, rbl::kThreads, 0, S(stream)>>>(v, roots);
 	RB_LAUNCHED("bfs_init");
 	return RB_OK;
 }
 
 int rb_bfs_step(const rb_bfs_view* b, int64_t max_states, int32_t* n_active, rb_stream_t stream) {
 	rbb::View v;
-	rba::View a;
-	int rc = bfs_view(b, v, a);
+	int rc = bfs_view(b, v);
 	if (rc != RB_OK) return rc;
 	RB_REQUIRE(n_active, "null n_active");
 	RB_REQUIRE(max_states >= 1 && max_states < v.M, "M must exceed max_states (index 0 is unused)");
 	RB_INIT();
 	cudaStream_t st = S(stream);
 	const dim3 grid(v.nbx(), v.K);
-	rbb::k_pop<<<dim3((v.N + rbb::kThreads - 1) / rbb::kThreads, v.K), rbb::kThreads, 0, st>>>(v, max_states, n_active);
+	rbb::k_pop<<<dim3((v.N + rbl::kThreads - 1) / rbl::kThreads, v.K), rbl::kThreads, 0, st>>>(v, max_states, n_active);
 	RB_LAUNCHED("bfs_pop");
-	rba::k_probe<<<grid, rba::kThreads, 0, st>>>(a);
+	rbl::k_probe<<<grid, rbl::kThreads, 0, st>>>(v);
 	RB_LAUNCHED("bfs_probe");
-	rba::k_flag<<<grid, rba::kThreads, 0, st>>>(a);
+	rbl::k_flag<<<grid, rbl::kThreads, 0, st>>>(v);
 	RB_LAUNCHED("bfs_flag");
-	rba::k_totals<<<1, 1024, 0, st>>>(a, v.n_new_total);
+	rbl::k_totals<<<1, 1024, 0, st>>>(v, v.n_new_total);
 	RB_LAUNCHED("bfs_totals");
-	rbb::k_assign<<<grid, rbb::kThreads, 0, st>>>(v, a, max_states);
+	rbb::k_assign<<<grid, rbl::kThreads, 0, st>>>(v, max_states);
 	RB_LAUNCHED("bfs_assign");
-	rbb::k_finish<<<grid, rbb::kThreads, 0, st>>>(v, a, max_states, n_active);
+	rbb::k_finish<<<grid, rbl::kThreads, 0, st>>>(v, max_states, n_active);
 	RB_LAUNCHED("bfs_finish");
 	return RB_OK;
 }
 
 int rb_bfs_paths(const rb_bfs_view* b, uint8_t* queues, int32_t* lengths, int32_t L, rb_stream_t stream) {
 	rbb::View v;
-	rba::View a;
-	int rc = bfs_view(b, v, a);
+	int rc = bfs_view(b, v);
 	if (rc != RB_OK) return rc;
 	RB_REQUIRE(queues && lengths && L > 0, "null output or L <= 0");
 	RB_INIT();
-	rbb::k_paths<<<(v.K + rbb::kThreads - 1) / rbb::kThreads, rbb::kThreads, 0, S(stream)>>>(v, queues, lengths, L);
+	rbb::k_paths<<<(v.K + rbl::kThreads - 1) / rbl::kThreads, rbl::kThreads, 0, S(stream)>>>(v, queues, lengths, L);
 	RB_LAUNCHED("bfs_paths");
 	return RB_OK;
 }

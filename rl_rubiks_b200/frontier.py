@@ -13,6 +13,7 @@ device) carry the reference agents' interface
 """
 from __future__ import annotations
 
+import ctypes as C
 from collections import deque
 from time import perf_counter
 
@@ -380,13 +381,9 @@ class AStarBatch:
 	def __str__(self):
 		return f"AStar (lambda={self.lambda_}, N={self.expansions})"
 
-	def _roots(self, states) -> torch.Tensor:
-		return _roots2024(states, self.is2024, self.dev)
-
 	def _step_calls(self, max_states: int):
 		"""The two halves of a step as callables: plain C-ABI calls, or replays of their CUDA graphs (captured once per buffer set
 		and budget; the graphs hold kernel launches only -- the value net runs between them, on however many new states there are)."""
-		import ctypes as C
 		v = C.byref(self.view)
 		n_total_ptr, n_active_ptr = C.c_void_p(self.counters.data_ptr()), C.c_void_p(self.counters.data_ptr() + 4)
 
@@ -414,11 +411,10 @@ class AStarBatch:
 		"""states: (K, *shape) int8 (numpy or CUDA tensor).  Returns (solved bool (K,), action queues: list of K lists,
 		len per search int (K,)), the three things `AStar.search` leaves behind for one cube."""
 		t0 = perf_counter()
-		roots = self._roots(states)
+		roots = _roots2024(states, self.is2024, self.dev)
 		self._alloc(roots.shape[0], int(max_states))
 		self.net.eval()
 		sh = N.stream_handle()
-		import ctypes as C
 		def start():
 			N.check(N.lib.rb_hashset_clear(N.ptr(self.table), self.capacity, sh))
 			N.check(N.lib.rb_astar_init(C.byref(self.view), N.ptr(roots), sh))
@@ -548,7 +544,6 @@ class BFSBatch:
 	def search_many(self, states, max_states: int, time_limit: float | None = None):
 		"""states: (K, *shape) int8 (numpy or CUDA tensor).  Returns (found bool (K,), action queues: list of K lists,
 		len per search int (K,)), the three things `BFS.search` leaves behind for one cube (len 0 for a solved start)."""
-		import ctypes as C
 		t0 = perf_counter()
 		roots = _roots2024(states, self.is2024, self.dev)
 		self._alloc(roots.shape[0], int(max_states))

@@ -56,7 +56,7 @@ def keys(states, is2024):
 
 
 def astar_key(states, search):
-	"""rba::k_probe / k_init: the search id in bits 40-55 of the 20x24 key's high word."""
+	"""rbl::key (k_probe, root init): the search id in bits 40-55 of the 20x24 key's high word."""
 	lo, hi = key2024(states)
 	return lo, hi | (np.asarray(search, dtype=np.uint64) << np.uint64(40))
 

@@ -135,9 +135,11 @@ def test_store_policy_threshold_and_big_outputs():
 	assert 12 * games * depth == S.BIG_ONE_HOT["adi_generate_2024_f32"][0]
 
 
-def test_astar_rounds():
+def test_astar_rounds_in_search_core():
+	"""k_totals lives in the lockstep expansion core both batched searches share (rb_search.cuh)."""
 	src = _read("rb_astar.cuh")
-	body = src[src.index("k_totals("):]
+	body = _read("rb_search.cuh")
+	body = body[body.index("k_totals("):]
 	step = int(re.search(r"for \(int base = 0; base < v\.K; base \+= (\d+)\)", body).group(1))
 	assert step == 1024
 	assert [-(-k // step) for k in (1100, 2085)] == [2, 3]
