@@ -617,36 +617,61 @@ static int core_view(const AbiView* a, bool n_ok, int64_t keys, bool own_set, bo
 	scratch(v, static_cast<uint8_t*>(a->scratch));
 	return RB_OK;
 }
-}  // extern "C++"
 
-// ---- batched A* ----------------------------------------------------------------------------------------------------------
-int64_t rb_astar_scratch_bytes(int32_t K, int32_t N) {
-	rba::View v{{K, 0, N}};
+template <class View> static int64_t scratch_bytes(int32_t K, int32_t N) {
+	View v{{K, 0, N}};
 	return K > 0 && N > 0 ? scratch(v, nullptr) : 0;
 }
 
-static int astar_view(const rb_astar_view* a, rba::View& v) {
+static int search_view(const rb_astar_view* a, rba::View& v) {
 	RB_REQUIRE(a, "null view");
 	v.G = a->G; v.cost = a->cost; v.in_open = a->in_open; v.n_sel = a->n_sel; v.sel = a->sel; v.solved_index = a->solved_index;
 	return core_view(a, a->N <= 1024, a->M, a->G && a->cost && a->in_open && a->n_sel && a->sel && a->solved_index,
 	                 aligned(a->G, 8) && aligned(a->cost, 8), v);
 }
 
-int rb_astar_init(const rb_astar_view* a, const int8_t* roots, rb_stream_t stream) {
-	rba::View v;
-	int rc = astar_view(a, v);
+static int search_view(const rb_bfs_view* b, rbb::View& v) {
+	RB_REQUIRE(b, "null view");
+	v.head = b->head; v.done = b->done; v.solved_parent = b->solved_parent; v.solved_action = b->solved_action;
+	// the children of parents dropped by the budget are claimed before the cut is known: a search holds up to M + 12 N keys
+	return core_view(b, b->N <= (1 << 20), b->M + 12 * (int64_t)b->N, b->head && b->done && b->solved_parent && b->solved_action, true, v);
+}
+
+// state 1 of every search: its root
+template <class AbiView, class View>
+static int init_search(const AbiView* a, const int8_t* roots, void (*k_init)(View, const int8_t*), rb_stream_t stream) {
+	View v;
+	int rc = search_view(a, v);
 	if (rc != RB_OK) return rc;
 	RB_REQUIRE(roots && aligned(roots, 4), "roots must be a 4-byte aligned device pointer");
 	RB_INIT();
-	rba::k_init<<<(v.K + rbl::kThreads - 1) / rbl::kThreads, rbl::kThreads, 0, S(stream)>>>(v, roots);
-	RB_LAUNCHED("astar_init");
+	k_init<<<(v.K + rbl::kThreads - 1) / rbl::kThreads, rbl::kThreads, 0, S(stream)>>>(v, roots);
+	RB_LAUNCHED("search_init");
 	return RB_OK;
 }
+
+// the children of the selected parents, deduplicated and counted: the part of a step between a search's select and its assign
+static int expand_children(const rbl::Core& v, int32_t* n_new_total, cudaStream_t st) {
+	const dim3 grid(v.nbx(), v.K);
+	rbl::k_probe<<<grid, rbl::kThreads, 0, st>>>(v);
+	RB_LAUNCHED("search_probe");
+	rbl::k_flag<<<grid, rbl::kThreads, 0, st>>>(v);
+	RB_LAUNCHED("search_flag");
+	rbl::k_totals<<<1, 1024, 0, st>>>(v, n_new_total);
+	RB_LAUNCHED("search_totals");
+	return RB_OK;
+}
+}  // extern "C++"
+
+// ---- batched A* ----------------------------------------------------------------------------------------------------------
+int64_t rb_astar_scratch_bytes(int32_t K, int32_t N) { return scratch_bytes<rba::View>(K, N); }
+
+int rb_astar_init(const rb_astar_view* a, const int8_t* roots, rb_stream_t stream) { return init_search(a, roots, rba::k_init, stream); }
 
 int rb_astar_expand(const rb_astar_view* a, int64_t max_states, int8_t* new_states, int32_t* new_search, int32_t* new_index,
                     int32_t* n_new_total, int32_t* n_active, rb_stream_t stream) {
 	rba::View v;
-	int rc = astar_view(a, v);
+	int rc = search_view(a, v);
 	if (rc != RB_OK) return rc;
 	RB_REQUIRE(new_states && new_search && new_index && n_new_total && n_active && aligned(new_states, 4), "null or misaligned output");
 	RB_REQUIRE(max_states < v.M, "M must exceed max_states (index 0 is unused)");
@@ -667,12 +692,8 @@ int rb_astar_expand(const rb_astar_view* a, int64_t max_states, int8_t* new_stat
 	}
 	rba::k_select<<<v.K, rba::kSelThreads, rba::kSelSmem, st>>>(v, max_states, n_active);
 	RB_LAUNCHED("astar_select");
-	rbl::k_probe<<<grid, rbl::kThreads, 0, st>>>(v);
-	RB_LAUNCHED("astar_probe");
-	rbl::k_flag<<<grid, rbl::kThreads, 0, st>>>(v);
-	RB_LAUNCHED("astar_flag");
-	rbl::k_totals<<<1, 1024, 0, st>>>(v, n_new_total);
-	RB_LAUNCHED("astar_totals");
+	rc = expand_children(v, n_new_total, st);
+	if (rc != RB_OK) return rc;
 	rba::k_assign<<<grid, rbl::kThreads, 0, st>>>(v, new_states, new_search, new_index);
 	RB_LAUNCHED("astar_assign");
 	return RB_OK;
@@ -681,7 +702,7 @@ int rb_astar_expand(const rb_astar_view* a, int64_t max_states, int8_t* new_stat
 int rb_astar_commit(const rb_astar_view* a, const float* values, double lambda, const int32_t* new_search, const int32_t* new_index,
                     const int32_t* n_new_total, rb_stream_t stream) {
 	rba::View v;
-	int rc = astar_view(a, v);
+	int rc = search_view(a, v);
 	if (rc != RB_OK) return rc;
 	RB_REQUIRE(values && new_search && new_index && n_new_total, "null input");
 	cudaStream_t st = S(stream);
@@ -703,32 +724,13 @@ int rb_astar_commit(const rb_astar_view* a, const float* values, double lambda, 
 }
 
 // ---- batched BFS ---------------------------------------------------------------------------------------------------------
-int64_t rb_bfs_scratch_bytes(int32_t K, int32_t N) {
-	rbb::View v{{K, 0, N}};
-	return K > 0 && N > 0 ? scratch(v, nullptr) : 0;
-}
+int64_t rb_bfs_scratch_bytes(int32_t K, int32_t N) { return scratch_bytes<rbb::View>(K, N); }
 
-static int bfs_view(const rb_bfs_view* b, rbb::View& v) {
-	RB_REQUIRE(b, "null view");
-	v.head = b->head; v.done = b->done; v.solved_parent = b->solved_parent; v.solved_action = b->solved_action;
-	// the children of parents dropped by the budget are claimed before the cut is known: a search holds up to M + 12 N keys
-	return core_view(b, b->N <= (1 << 20), b->M + 12 * (int64_t)b->N, b->head && b->done && b->solved_parent && b->solved_action, true, v);
-}
-
-int rb_bfs_init(const rb_bfs_view* b, const int8_t* roots, rb_stream_t stream) {
-	rbb::View v;
-	int rc = bfs_view(b, v);
-	if (rc != RB_OK) return rc;
-	RB_REQUIRE(roots && aligned(roots, 4), "roots must be a 4-byte aligned device pointer");
-	RB_INIT();
-	rbb::k_init<<<(v.K + rbl::kThreads - 1) / rbl::kThreads, rbl::kThreads, 0, S(stream)>>>(v, roots);
-	RB_LAUNCHED("bfs_init");
-	return RB_OK;
-}
+int rb_bfs_init(const rb_bfs_view* b, const int8_t* roots, rb_stream_t stream) { return init_search(b, roots, rbb::k_init, stream); }
 
 int rb_bfs_step(const rb_bfs_view* b, int64_t max_states, int32_t* n_active, rb_stream_t stream) {
 	rbb::View v;
-	int rc = bfs_view(b, v);
+	int rc = search_view(b, v);
 	if (rc != RB_OK) return rc;
 	RB_REQUIRE(n_active, "null n_active");
 	RB_REQUIRE(max_states >= 1 && max_states < v.M, "M must exceed max_states (index 0 is unused)");
@@ -737,12 +739,8 @@ int rb_bfs_step(const rb_bfs_view* b, int64_t max_states, int32_t* n_active, rb_
 	const dim3 grid(v.nbx(), v.K);
 	rbb::k_pop<<<dim3((v.N + rbl::kThreads - 1) / rbl::kThreads, v.K), rbl::kThreads, 0, st>>>(v, max_states, n_active);
 	RB_LAUNCHED("bfs_pop");
-	rbl::k_probe<<<grid, rbl::kThreads, 0, st>>>(v);
-	RB_LAUNCHED("bfs_probe");
-	rbl::k_flag<<<grid, rbl::kThreads, 0, st>>>(v);
-	RB_LAUNCHED("bfs_flag");
-	rbl::k_totals<<<1, 1024, 0, st>>>(v, v.n_new_total);
-	RB_LAUNCHED("bfs_totals");
+	rc = expand_children(v, v.n_new_total, st);
+	if (rc != RB_OK) return rc;
 	rbb::k_assign<<<grid, rbl::kThreads, 0, st>>>(v, max_states);
 	RB_LAUNCHED("bfs_assign");
 	rbb::k_finish<<<grid, rbl::kThreads, 0, st>>>(v, max_states, n_active);
@@ -752,7 +750,7 @@ int rb_bfs_step(const rb_bfs_view* b, int64_t max_states, int32_t* n_active, rb_
 
 int rb_bfs_paths(const rb_bfs_view* b, uint8_t* queues, int32_t* lengths, int32_t L, rb_stream_t stream) {
 	rbb::View v;
-	int rc = bfs_view(b, v);
+	int rc = search_view(b, v);
 	if (rc != RB_OK) return rc;
 	RB_REQUIRE(queues && lengths && L > 0, "null output or L <= 0");
 	RB_INIT();

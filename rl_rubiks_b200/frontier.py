@@ -6,7 +6,7 @@ Python dict keyed on `state.tostring()` (reference: librubiks/solving/agents.py:
 reference's index semantics: states are numbered 1, 2, ... in insertion order, a batch is numbered in batch order,
 in-batch duplicates resolve to their first occurrence (agents.py:286-306).  `BFS` (layer-synchronous), `BFSBatch` (K
 breadth-first searches in lockstep on the device) and `AStarBatch` (K searches in lockstep, open list and relaxation on the
-device) carry the reference agents' interface
+device; the two batched agents share their host driver, `_BatchAgent`) carry the reference agents' interface
 (`search(state, time_limit, max_states) -> bool`, `action_queue`, `len(agent)`).  The reference's host-side agent loops
 (single-search A* around a heapq, MCTS' UCB walk) are not part of the product: tests/agent_harness.py replays them around
 `StateHashSet` to check the device primitives against traces recorded from the reference.
@@ -284,75 +284,136 @@ class BFS(Agent):
 
 def _roots2024(states, is2024: bool, dev) -> torch.Tensor:
 	"""Start states (K, *shape) of a batched search as 20-byte device rows: the searches run on the 20x24 form, 6x8x6 starts
-	are converted (`rb_as2024`); an unreachable 6x8x6 start is an IndexError."""
+	are converted (`cube.to_2024`: an unreachable start is an IndexError)."""
 	s = states if isinstance(states, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(states, dtype=np.int8))
 	s = s.to(device=dev, dtype=torch.int8)
-	if is2024:
-		return s.reshape(-1, 20).contiguous()
-	s = s.reshape(-1, 6, 8, 6).contiguous()
-	roots = torch.empty(s.shape[0], 20, dtype=torch.int8, device=dev)
-	ok = torch.empty(s.shape[0], dtype=torch.uint8, device=dev)
-	N.check(N.lib.rb_as2024(N.ptr(s), N.ptr(roots), N.ptr(ok), s.shape[0], N.stream_handle()))
-	if not bool(ok.all().item()):
-		raise IndexError("a 6x8x6 start state is not a reachable cube")
-	return roots
+	return s.reshape(-1, 20).contiguous() if is2024 else cube.to_2024(s)
 
 
-class AStarBatch:
+class _BatchAgent(Agent):
+	"""K searches in lockstep on the device (csrc/rb_search.cuh), the part every such search has: the state rows, parents,
+	counts and shared seen-set, the one-cube `search` of the reference agents' interface and the step loop of `search_many`.
+	Both representations (the module flag, or `is2024`): the searches run on the 20-byte states, 6x8x6 starts are converted
+	on the way in.  A subclass brings its buffers and C view (`_alloc`), its C calls for the scratch size and the init
+	(`_c_scratch_bytes`, `_c_init`), one step (`_advance`) and the read-back (`_results`)."""
+
+	_default_max_states = 1 << 20              # buffers are sized by the state budget: a search limited by time only gets this one
+
+	def __init__(self, is2024: bool | None = None):
+		super().__init__()
+		N.require_cuda()
+		self.is2024 = cube.get_is2024() if is2024 is None else bool(is2024)
+		self.dev = torch.device("cuda", torch.cuda.current_device())
+
+	def search(self, state, time_limit: float = None, max_states: int = None) -> bool:
+		"""The reference agent's `search(state, time_limit, max_states)` for one cube on the batched machinery (K = 1): fills
+		`action_queue`, and `len(agent)` is the number of states stored (0 for a solved start).  The time limit is tested before
+		every step."""
+		assert time_limit or max_states
+		won, queues, count = self.search_many(np.asarray(state)[None] if not isinstance(state, torch.Tensor) else state[None],
+											  int(max_states or self._default_max_states), time_limit=time_limit)
+		self.action_queue = deque(queues[0])
+		self._explored_states = 0 if won[0] and not queues[0] and count[0] <= 1 else int(count[0])
+		return bool(won[0])
+
+	def _alloc_core(self, K: int, M: int, Nx: int, keys: int) -> bool:
+		"""The buffers every search has, for K searches of M state rows and up to Nx parents per step; `keys`: entries one search
+		can hold in the seen-set, which is kept at load <= 1/2.  False when the previous call's buffers (same K, M, Nx) are
+		reused: every field a search reads is re-initialised by its init and `rb_hashset_clear`."""
+		if getattr(self, "_shape", None) == (K, M, Nx):
+			return False
+		self._shape = (K, M, Nx)
+		self.K, self.M = K, M
+		dev = self.dev
+		self.states = torch.empty(K, M, 20, dtype=torch.int8, device=dev)
+		self.parents = torch.zeros(K, M, dtype=torch.int32, device=dev)
+		self.parent_actions = torch.zeros(K, M, dtype=torch.uint8, device=dev)
+		self.count = torch.zeros(K, dtype=torch.int32, device=dev)
+		self.won = torch.zeros(K, dtype=torch.uint8, device=dev)
+		self.capacity = _pow2_at_least(2 * K * keys)
+		self.table = torch.empty(N.lib.rb_hashset_bytes(self.capacity), dtype=torch.uint8, device=dev)
+		self.scratch = torch.empty(self._c_scratch_bytes(K, Nx), dtype=torch.uint8, device=dev)
+		self.counters = torch.zeros(2, dtype=torch.int32, device=dev)          # new states of the step (A* only), searches active
+		self.counters_host = torch.zeros(2, dtype=torch.int32, pin_memory=True)
+		return True
+
+	def _start(self, roots: torch.Tensor, max_states: int):
+		sh = N.stream_handle()
+		N.check(N.lib.rb_hashset_clear(N.ptr(self.table), self.capacity, sh))
+		N.check(self._c_init(C.byref(self.view), N.ptr(roots), sh))
+
+	def _read(self):
+		"""The one host read of a step: `counters` through the pinned buffer."""
+		self.counters_host.copy_(self.counters, non_blocking=True)
+		torch.cuda.current_stream().synchronize()
+		return self.counters_host.tolist()
+
+	@torch.no_grad()
+	def _run(self, states, max_states: int, max_steps: int | None, time_limit: float | None):
+		"""`search_many`: steps until `_advance` reports no search active, or `max_steps` / the time limit ends the call.
+		`steps` counts the steps that ran, `launches` the library's kernel launches outside CUDA graphs from the first step to
+		the end of the read-back."""
+		t0 = perf_counter()
+		max_states = int(max_states)
+		roots = _roots2024(states, self.is2024, self.dev)
+		self._alloc(roots.shape[0], max_states)
+		self._start(roots, max_states)
+		self.steps = 0
+		l0 = N.lib.rb_launch_count()
+		while (max_steps is None or self.steps < max_steps) and (time_limit is None or perf_counter() - t0 < time_limit):
+			ran, active = self._advance(max_states)
+			self.steps += ran
+			if not active:
+				break
+		out = self._results()
+		self.launches = N.lib.rb_launch_count() - l0
+		return out
+
+
+class AStarBatch(_BatchAgent):
 	"""Batched weighted A* (agents.py:171-413) for K cubes at once, entirely on the device (SURVEY 8f rows N2 + N3): open
 	list, seen-set, G / parent relaxation and the pop of the N cheapest states per search are kernels (csrc/rb_astar.cuh);
 	the host only runs the value net on the contiguous batch of new states of all searches and reads two counters per step.
 	Every search follows the reference's trace exactly (same pops, same state numbering, same G / parents / action queue).
 
-	Both representations (the module flag, or `is2024`): the searches always run on the 20-byte states -- the two
-	representations describe the same cube, children come in the same action order, so the trace is the same -- and with the
-	6x8x6 representation the roots are converted on the way in (`rb_as2024`) and the new states are rendered as 6x8x6 rows
-	(`rb_as686`) only to feed the value net its 288-wide one-hot.
+	Both representations describe the same cube and children come in the same action order, so the trace is the same; with
+	the 6x8x6 representation the new states are rendered as 6x8x6 rows (`rb_as686`) only to feed the value net its 288-wide
+	one-hot.
 
 	The launches of a step are two CUDA graphs (expand: 6 kernels + 1 memset, commit: 6 kernels), captured once per buffer set."""
 
+	_c_scratch_bytes, _c_init = N.lib.rb_astar_scratch_bytes, N.lib.rb_astar_init
+
 	def __init__(self, net, lambda_: float, expansions: int, oh_dtype=torch.float32, is2024: bool | None = None, use_graphs: bool = True):
-		N.require_cuda()
+		super().__init__(is2024)
 		if not 0 < expansions <= 1024:
 			raise ValueError("expansions must be in 1..1024")
 		self.net, self.lambda_, self.expansions = net, float(lambda_), int(expansions)
-		self.is2024 = cube.get_is2024() if is2024 is None else bool(is2024)
 		# torch.bfloat16 (opt-in, not the reference's dtype): bf16 one-hot rows and a bf16-autocast forward of the value net
 		self.oh_dtype = oh_dtype
 		self._as_oh = cube._oh_fn("rb_as_oh", oh_dtype)
-		self.dev = torch.device("cuda", torch.cuda.current_device())
 		self.use_graphs = use_graphs
-		self.action_queue = deque()
+
+	def __str__(self):
+		return f"AStar (lambda={self.lambda_}, N={self.expansions})"
 
 	def _alloc(self, K: int, max_states: int):
 		dev, Nx = self.dev, self.expansions
 		M = max_states + 1
-		if getattr(self, "_shape", None) == (K, M, Nx):           # buffers of the previous search_many are reused (everything that
-			self.parents.zero_(); self.parent_actions.zero_()     # matters is re-initialised by rb_astar_init / rb_hashset_clear)
+		if not self._alloc_core(K, M, Nx, M):    # a search stores at most M states
+			self.parents.zero_(); self.parent_actions.zero_()     # reused buffers: rb_astar_init does not clear these
 			self.in_open.zero_()
 			return
-		self._shape = (K, M, Nx)
-		self.K, self.M = K, M
-		self.states = torch.empty(K, M, 20, dtype=torch.int8, device=dev)
 		self.G = torch.empty(K, M, dtype=torch.float64, device=dev)
-		self.parents = torch.zeros(K, M, dtype=torch.int32, device=dev)
-		self.parent_actions = torch.zeros(K, M, dtype=torch.uint8, device=dev)
 		self.cost = torch.empty(K, M, dtype=torch.float64, device=dev)
 		self.in_open = torch.zeros(K, M, dtype=torch.uint8, device=dev)
-		self.count = torch.zeros(K, dtype=torch.int32, device=dev)
 		self.n_sel = torch.zeros(K, dtype=torch.int32, device=dev)
 		self.sel = torch.zeros(K, Nx, dtype=torch.int32, device=dev)
-		self.won = torch.zeros(K, dtype=torch.uint8, device=dev)
 		self.solved_index = torch.zeros(K, dtype=torch.int32, device=dev)
-		self.capacity = _pow2_at_least(2 * K * M)                 # load <= 1/2 by construction: a search stores at most M states
-		self.table = torch.empty(N.lib.rb_hashset_bytes(self.capacity), dtype=torch.uint8, device=dev)
-		self.scratch = torch.empty(N.lib.rb_astar_scratch_bytes(K, Nx), dtype=torch.uint8, device=dev)
 		P = 12 * Nx
 		self.new_states = torch.empty(K * P, 20, dtype=torch.int8, device=dev)
 		self.new_search = torch.empty(K * P, dtype=torch.int32, device=dev)
 		self.new_index = torch.empty(K * P, dtype=torch.int32, device=dev)
-		self.counters = torch.zeros(2, dtype=torch.int32, device=dev)          # n_new_total, n_active
-		self.counters_host = torch.zeros(2, dtype=torch.int32, pin_memory=True)
 		self.values = torch.zeros(K * P, dtype=torch.float32, device=dev)      # the net's output lands here: fixed address for the commit graph
 		self.oh = torch.empty(K * P, 480 if self.is2024 else 288, dtype=self.oh_dtype, device=dev)
 		self.new_states686 = None if self.is2024 else torch.empty(K * P, 6, 8, 6, dtype=torch.int8, device=dev)
@@ -361,87 +422,52 @@ class AStarBatch:
 								self.capacity, N.ptr(self.scratch))
 		self._graphs = None
 
-	# ---- the reference agents' interface, one cube (agents.py:221-252) ----
-	_default_max_states = 1 << 20              # buffers are sized by the state budget: a search limited by time only gets this one
-
-	def search(self, state, time_limit: float = None, max_states: int = None) -> bool:
-		"""`AStar.search(state, time_limit, max_states)` for one cube on the batched machinery (K = 1): fills `action_queue`,
-		`len(agent)` is the number of states stored.  The time limit is tested before every expansion step, like
-		agents.py:238."""
-		assert time_limit or max_states
-		won, queues, count = self.search_many(np.asarray(state)[None] if not isinstance(state, torch.Tensor) else state[None],
-											  int(max_states or self._default_max_states), time_limit=time_limit)
-		self.action_queue = deque(queues[0])
-		self._explored_states = int(count[0]) if not (won[0] and count[0] == 1 and not queues[0]) else 0      # solved start: nothing stored
-		return bool(won[0])
-
-	def __len__(self):
-		return getattr(self, "_explored_states", 0)
-
-	def __str__(self):
-		return f"AStar (lambda={self.lambda_}, N={self.expansions})"
-
-	def _step_calls(self, max_states: int):
-		"""The two halves of a step as callables: plain C-ABI calls, or replays of their CUDA graphs (captured once per buffer set
-		and budget; the graphs hold kernel launches only -- the value net runs between them, on however many new states there are)."""
+	def _start(self, roots: torch.Tensor, max_states: int):
+		"""Also readies the two halves of a step: plain C-ABI calls, or replays of their CUDA graphs (captured once per buffer set;
+		the graphs hold kernel launches only -- the value net runs between them, on however many new states there are)."""
 		v = C.byref(self.view)
-		n_total_ptr, n_active_ptr = C.c_void_p(self.counters.data_ptr()), C.c_void_p(self.counters.data_ptr() + 4)
+		n_total, n_active = N.ptr(self.counters[:1]), N.ptr(self.counters[1:])
 
 		def expand():
-			N.check(N.lib.rb_astar_expand(v, int(max_states), N.ptr(self.new_states), N.ptr(self.new_search), N.ptr(self.new_index),
-										  n_total_ptr, n_active_ptr, N.stream_handle()))
-
-		def commit():
-			N.check(N.lib.rb_astar_commit(v, N.ptr(self.values), self.lambda_, N.ptr(self.new_search), N.ptr(self.new_index), n_total_ptr,
+			N.check(N.lib.rb_astar_expand(v, max_states, N.ptr(self.new_states), N.ptr(self.new_search), N.ptr(self.new_index), n_total, n_active,
 										  N.stream_handle()))
 
-		if not self.use_graphs:
-			return expand, commit
-		if self._graphs is None or self._graphs[0] != int(max_states):
-			ge, gc = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
-			with torch.cuda.graph(ge):
-				expand()
-			with torch.cuda.graph(gc):
-				commit()
-			self._graphs = (int(max_states), ge, gc)
-		return self._graphs[1].replay, self._graphs[2].replay
-
-	@torch.no_grad()
-	def search_many(self, states, max_states: int, max_steps: int | None = None, time_limit: float | None = None):
-		"""states: (K, *shape) int8 (numpy or CUDA tensor).  Returns (solved bool (K,), action queues: list of K lists,
-		len per search int (K,)), the three things `AStar.search` leaves behind for one cube."""
-		t0 = perf_counter()
-		roots = _roots2024(states, self.is2024, self.dev)
-		self._alloc(roots.shape[0], int(max_states))
-		self.net.eval()
-		sh = N.stream_handle()
-		def start():
-			N.check(N.lib.rb_hashset_clear(N.ptr(self.table), self.capacity, sh))
-			N.check(N.lib.rb_astar_init(C.byref(self.view), N.ptr(roots), sh))
+		def commit():
+			N.check(N.lib.rb_astar_commit(v, N.ptr(self.values), self.lambda_, N.ptr(self.new_search), N.ptr(self.new_index), n_total,
+										  N.stream_handle()))
 
 		if self.use_graphs and self._graphs is None:
 			# one plain expansion before the capture (tables uploaded, function attributes set: nothing of that may happen inside
 			# a capture), then everything is initialised again
-			start()
-			N.check(N.lib.rb_astar_expand(C.byref(self.view), int(max_states), N.ptr(self.new_states), N.ptr(self.new_search), N.ptr(self.new_index),
-										  C.c_void_p(self.counters.data_ptr()), C.c_void_p(self.counters.data_ptr() + 4), sh))
-			torch.cuda.current_stream().synchronize()
-		start()
-		expand, commit = self._step_calls(max_states)
-		self.steps = self.launches = 0
-		l0 = N.lib.rb_launch_count()
-		while (max_steps is None or self.steps < max_steps) and (time_limit is None or perf_counter() - t0 < time_limit):
+			super()._start(roots, max_states)
 			expand()
-			self.counters_host.copy_(self.counters, non_blocking=True)           # the one host sync of a step
 			torch.cuda.current_stream().synchronize()
-			n_total, n_active = (int(x) for x in self.counters_host.tolist())
-			if n_active == 0:
-				break
-			self._values(n_total)
-			commit()
-			self.steps += 1
-		self.launches = N.lib.rb_launch_count() - l0
-		return self._results()
+		super()._start(roots, max_states)
+		if self.use_graphs:
+			if self._graphs is None:
+				ge, gc = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
+				with torch.cuda.graph(ge):
+					expand()
+				with torch.cuda.graph(gc):
+					commit()
+				self._graphs = ge, gc
+			expand, commit = self._graphs[0].replay, self._graphs[1].replay
+		self._expand, self._commit = expand, commit
+
+	def search_many(self, states, max_states: int, max_steps: int | None = None, time_limit: float | None = None):
+		"""states: (K, *shape) int8 (numpy or CUDA tensor).  Returns (solved bool (K,), action queues: list of K lists,
+		len per search int (K,)), the three things `AStar.search` leaves behind for one cube."""
+		self.net.eval()
+		return self._run(states, max_states, max_steps, time_limit)
+
+	def _advance(self, max_states: int):
+		self._expand()
+		n_total, n_active = self._read()
+		if n_active == 0:
+			return False, False
+		self._values(n_total)
+		self._commit()
+		return True, True
 
 	def _values(self, n: int):
 		"""agents.py:379-381: one-hot born on the device, value head only; the f32 values land in `self.values[:n]`."""
@@ -476,28 +502,15 @@ class AStarBatch:
 		return won, queues, count
 
 
-class BFSBatch:
+class BFSBatch(_BatchAgent):
 	"""Breadth-first search (agents.py:92-129) for K cubes at once, entirely on the device (csrc/rb_bfs.cuh): every search pops
 	up to `_step` parents of its FIFO per step, with the reference's budget test before every pop, and all searches share one
 	seen-set.  The host reads one counter per step (searches still running).  Each search's found flag, `len(agent)` and
-	action queue are `BFS.search`'s for the same start and `max_states` (tests/golden/bfs_budget.npz).
-
-	Both representations (the module flag, or `is2024`): the searches run on the 20-byte states, 6x8x6 starts are converted
-	on the way in (`rb_as2024`)."""
+	action queue are `BFS.search`'s for the same start and `max_states` (tests/golden/bfs_budget.npz)."""
 
 	_step = 2048                                   # parents popped per search and step (changes no result)
 	_queue_len = 16                                # a FIFO index below 2^29 has BFS depth <= 9
-	_default_max_states = 1 << 20                  # buffers are sized by the state budget: a search limited by time only gets this one
-
-	def __init__(self, is2024: bool | None = None):
-		N.require_cuda()
-		self.is2024 = cube.get_is2024() if is2024 is None else bool(is2024)
-		self.dev = torch.device("cuda", torch.cuda.current_device())
-		self.action_queue = deque()
-		self._explored_states = 0
-
-	def __len__(self):
-		return self._explored_states
+	_c_scratch_bytes, _c_init = N.lib.rb_bfs_scratch_bytes, N.lib.rb_bfs_init
 
 	def __str__(self):
 		return "Breadth-first search (batched)"
@@ -505,63 +518,30 @@ class BFSBatch:
 	def _alloc(self, K: int, max_states: int):
 		dev, Nx = self.dev, self._step
 		M = max_states + 1
-		if getattr(self, "_shape", None) == (K, M, Nx):           # every field a search reads is re-initialised by rb_bfs_init /
-			return                                                # rb_hashset_clear
-		self._shape = (K, M, Nx)
-		self.K, self.M = K, M
-		self.states = torch.empty(K, M, 20, dtype=torch.int8, device=dev)
-		self.parents = torch.zeros(K, M, dtype=torch.int32, device=dev)
-		self.parent_actions = torch.zeros(K, M, dtype=torch.uint8, device=dev)
-		self.count = torch.zeros(K, dtype=torch.int32, device=dev)
+		# a search holds at most M states plus the children of one step's dropped parents
+		if not self._alloc_core(K, M, Nx, M + 12 * Nx):
+			return
 		self.head = torch.zeros(K, dtype=torch.int32, device=dev)
-		self.won = torch.zeros(K, dtype=torch.uint8, device=dev)
 		self.done = torch.zeros(K, dtype=torch.uint8, device=dev)
 		self.solved_parent = torch.zeros(K, dtype=torch.int32, device=dev)
 		self.solved_action = torch.zeros(K, dtype=torch.uint8, device=dev)
-		# load <= 1/2: a search holds at most M states plus the children of one step's dropped parents
-		self.capacity = _pow2_at_least(2 * K * (M + 12 * Nx))
-		self.table = torch.empty(N.lib.rb_hashset_bytes(self.capacity), dtype=torch.uint8, device=dev)
-		self.scratch = torch.empty(N.lib.rb_bfs_scratch_bytes(K, Nx), dtype=torch.uint8, device=dev)
-		self.n_active = torch.zeros(1, dtype=torch.int32, device=dev)
-		self.n_active_host = torch.zeros(1, dtype=torch.int32, pin_memory=True)
 		self.queues = torch.zeros(K, self._queue_len, dtype=torch.uint8, device=dev)
 		self.lengths = torch.zeros(K, dtype=torch.int32, device=dev)
 		self.view = N.BFSView(K, M, Nx, *(N.ptr(t) for t in (self.states, self.parents, self.parent_actions, self.count, self.head, self.won,
 															 self.done, self.solved_parent, self.solved_action, self.table)),
 							  self.capacity, N.ptr(self.scratch))
 
-	def search(self, state, time_limit: float = None, max_states: int = None) -> bool:
-		"""`BFS.search(state, time_limit, max_states)` for one cube on the batched machinery (K = 1): fills `action_queue` and
-		`len(agent)`.  The time limit is tested before every step."""
-		assert time_limit or max_states
-		won, queues, count = self.search_many(np.asarray(state)[None] if not isinstance(state, torch.Tensor) else state[None],
-											  int(max_states or self._default_max_states), time_limit=time_limit)
-		self.action_queue = deque(queues[0])
-		self._explored_states = int(count[0])
-		return bool(won[0])
-
-	@torch.no_grad()
 	def search_many(self, states, max_states: int, time_limit: float | None = None):
 		"""states: (K, *shape) int8 (numpy or CUDA tensor).  Returns (found bool (K,), action queues: list of K lists,
 		len per search int (K,)), the three things `BFS.search` leaves behind for one cube (len 0 for a solved start)."""
-		t0 = perf_counter()
-		roots = _roots2024(states, self.is2024, self.dev)
-		self._alloc(roots.shape[0], int(max_states))
-		sh = N.stream_handle()
-		v = C.byref(self.view)
-		N.check(N.lib.rb_hashset_clear(N.ptr(self.table), self.capacity, sh))
-		N.check(N.lib.rb_bfs_init(v, N.ptr(roots), sh))
-		self.steps = 0
-		l0 = N.lib.rb_launch_count()
-		while time_limit is None or perf_counter() - t0 < time_limit:
-			N.check(N.lib.rb_bfs_step(v, int(max_states), N.ptr(self.n_active), sh))
-			self.steps += 1
-			self.n_active_host.copy_(self.n_active, non_blocking=True)          # the one host read of a step
-			torch.cuda.current_stream().synchronize()
-			if int(self.n_active_host[0]) == 0:
-				break
-		N.check(N.lib.rb_bfs_paths(v, N.ptr(self.queues), N.ptr(self.lengths), self._queue_len, sh))
-		self.launches = N.lib.rb_launch_count() - l0
+		return self._run(states, max_states, None, time_limit)
+
+	def _advance(self, max_states: int):
+		N.check(N.lib.rb_bfs_step(C.byref(self.view), max_states, N.ptr(self.counters[1:]), N.stream_handle()))
+		return True, self._read()[1] > 0
+
+	def _results(self):
+		N.check(N.lib.rb_bfs_paths(C.byref(self.view), N.ptr(self.queues), N.ptr(self.lengths), self._queue_len, N.stream_handle()))
 		won = self.won.bool().cpu().numpy()
 		count = self.count.cpu().numpy().astype(int)
 		lengths = self.lengths.cpu().numpy()
