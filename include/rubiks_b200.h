@@ -294,6 +294,59 @@ int rb_bfs_step(const rb_bfs_view* v, int64_t max_states, int32_t* n_active, rb_
  * -1 when the queue is longer than L). */
 int rb_bfs_paths(const rb_bfs_view* v, uint8_t* queues, int32_t* lengths, int32_t L, rb_stream_t stream);
 
+/* ---- batched Monte Carlo tree search on the device (MCTS.search agents.py:461-633 for K cubes at once; 20x24) -------------
+ * K independent searches advance in lockstep, one leaf expansion per search and step.  Every buffer is caller-owned device
+ * memory; [K][M] arrays are indexed by the reference's node index (1-based in numbering order, 0 unused), M >= max_states + 1.
+ *   rb_mcts_init     roots become node 1 (a solved root: found, len 1, empty queue)
+ *   [caller: net on the roots; P = softmax(policy) f32 [K][12], values f32 [K]]
+ *   rb_mcts_commit   with new_search = 0 .. K-1, new_index = 1, *n_new_total = K: the roots' P and V, the first walks
+ *   then per step:
+ *   rb_mcts_expand   the leaf of every running search: children deduplicated, numbered in action order and stored, neighbour
+ *                    links both ways, solved test; the new states go to one contiguous batch for the net
+ *   [caller: net on new_states[0 .. *n_new_total), softmax]
+ *   rb_mcts_commit   P and V of the new nodes, the backup along the walk, the next walk (UCB, virtual loss) and the budget test
+ *                    len + 12 <= max_states; *n_active receives the searches that expand in the next step, *overflow 1 when a
+ *                    walk needed more than max_path moves (that search stops; its results are not the reference's)
+ *   rb_mcts_finish   once: graph mode completes the neighbour table of the won searches and shortens their queues by BFS;
+ *                    then the action queue of every search.
+ * A row is written in full when its node is numbered; no buffer needs clearing between calls. */
+typedef struct rb_mcts_view {
+	int32_t K, M, max_path;       /* searches (<= 65535), rows per search (<= 2^27), walk length cap (>= 1) */
+	int8_t*  states;              /* [K][M][20] */
+	int32_t* parents;             /* [K][M] the node a node was generated from; graph mode: the shortening's scratch */
+	uint8_t* parent_actions;      /* [K][M] the action that generated it */
+	int32_t* neighbors;           /* [K][M][12] */
+	uint8_t* leaves;              /* [K][M] */
+	float*   P;                   /* [K][M][12] prior (softmax of the policy) */
+	float*   V;                   /* [K][M] value */
+	int32_t* N;                   /* [K][M][12] visit counts */
+	float*   W;                   /* [K][M][12] */
+	int32_t* L;                   /* [K][M][12] virtual loss in units of nu = 100 (zero outside the running walk) */
+	int32_t* count;               /* [K] nodes stored (= len(agent)) */
+	uint8_t* won;                 /* [K] */
+	int32_t* solved_index;        /* [K] the solved node (0: none, or a solved start) */
+	int32_t* path_node;           /* [K][max_path] the last walk: node j ... */
+	uint8_t* path_action;         /* [K][max_path] ... and the action taken there */
+	int32_t* path_len;            /* [K] */
+	int32_t* order;               /* [K][M] scratch of the graph shortening */
+	void*    table;               /* shared seen-set, rb_hashset_bytes(capacity) bytes, cleared with rb_hashset_clear */
+	int64_t  capacity;            /* power of two, >= 2 K M (checked: RB_ERR_CAPACITY below that) */
+	void*    scratch;             /* rb_mcts_scratch_bytes(K) bytes */
+} rb_mcts_view;
+int64_t rb_mcts_scratch_bytes(int32_t K);
+/* roots int8 [K][20]. */
+int rb_mcts_init(const rb_mcts_view* v, const int8_t* roots, rb_stream_t stream);
+/* new_states int8 [12K][20], new_search / new_index int32 [12K]; n_new_total: int32 on the device. */
+int rb_mcts_expand(const rb_mcts_view* v, int8_t* new_states, int32_t* new_search, int32_t* new_index, int32_t* n_new_total,
+                   rb_stream_t stream);
+/* probs f32 [*n_new_total][12], values f32 [*n_new_total]: softmax(policy) and value of new_states, in order.  n_active,
+ * overflow: int32 on the device. */
+int rb_mcts_commit(const rb_mcts_view* v, const float* probs, const float* values, const int32_t* new_search,
+                   const int32_t* new_index, const int32_t* n_new_total, double c, int64_t max_states, int32_t* n_active,
+                   int32_t* overflow, rb_stream_t stream);
+/* graph != 0: agents.py:597-633 for the won searches.  Queues uint8 [K][L], lengths int32 [K] (-1: longer than L). */
+int rb_mcts_finish(const rb_mcts_view* v, int32_t graph, uint8_t* queues, int32_t* lengths, int32_t L, rb_stream_t stream);
+
 /* ---- host-buffer entry points (end-to-end: H2D + kernels + D2H inside the call) --------------- */
 /* rb_scramble on host buffers; actions uint8 [n][depth] (cube-major), out int8 [n][*shape].  Copies are
  * chunked and double-buffered on internal streams; pinned host memory makes them asynchronous. */

@@ -71,6 +71,11 @@ SIGNATURES = {
 	"rb_bfs_init": (C.c_int, [_p, _p, _p]),
 	"rb_bfs_step": (C.c_int, [_p, _i64, _p, _p]),
 	"rb_bfs_paths": (C.c_int, [_p, _p, _p, _i32, _p]),
+	"rb_mcts_scratch_bytes": (_i64, [_i32]),
+	"rb_mcts_init": (C.c_int, [_p, _p, _p]),
+	"rb_mcts_expand": (C.c_int, [_p, _p, _p, _p, _p, _p]),
+	"rb_mcts_commit": (C.c_int, [_p, _p, _p, _p, _p, _p, _f64, _i64, _p, _p, _p]),
+	"rb_mcts_finish": (C.c_int, [_p, _i32, _p, _p, _i32, _p]),
 	"rb_as686": (C.c_int, [_p, _p, _i64, _p]),
 	"rb_as2024": (C.c_int, [_p, _p, _p, _i64, _p]),
 	"rb_scramble_seeded": (C.c_int, [C.c_int, C.c_uint64, C.c_uint64, _p, _p, _i64, _i32, _p]),
@@ -102,6 +107,13 @@ class BFSView(C.Structure):
 	_fields_ = [("K", _i32), ("M", _i32), ("N", _i32), ("states", _p), ("parents", _p), ("parent_actions", _p), ("count", _p),
 				("head", _p), ("won", _p), ("done", _p), ("solved_parent", _p), ("solved_action", _p), ("table", _p),
 				("capacity", _i64), ("scratch", _p)]
+
+
+class MCTSView(C.Structure):
+	"""rb_mcts_view (include/rubiks_b200.h)."""
+	_fields_ = [("K", _i32), ("M", _i32), ("max_path", _i32), ("states", _p), ("parents", _p), ("parent_actions", _p), ("neighbors", _p),
+				("leaves", _p), ("P", _p), ("V", _p), ("N", _p), ("W", _p), ("L", _p), ("count", _p), ("won", _p), ("solved_index", _p),
+				("path_node", _p), ("path_action", _p), ("path_len", _p), ("order", _p), ("table", _p), ("capacity", _i64), ("scratch", _p)]
 
 
 class RubiksError(RuntimeError):

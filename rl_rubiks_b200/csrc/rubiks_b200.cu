@@ -11,6 +11,7 @@
 #include "rb_search.cuh"
 #include "rb_astar.cuh"
 #include "rb_bfs.cuh"
+#include "rb_mcts.cuh"
 #include "rb_host.cuh"
 
 #define RB_INIT()                                   \
@@ -600,16 +601,23 @@ static int64_t scratch(rbb::View& v, uint8_t* base) {
 	return used + 64;
 }
 
+static int64_t scratch(rbm::View& v, uint8_t* base) {
+	int64_t used = carve_expansion(v, base);
+	carve(v.n_sel, base, used, v.K);
+	carve(v.sel, base, used, v.K);
+	return used + 64;
+}
+
 // The checks both views share, in order; then the Core is filled and the scratch carved.  An entry point checks its own
 // arguments only after this, so a bad view is what a call reports first.  keys: slots one search can claim (a full table drops
 // a child without an error word, k_probe stores slot -1: 2 K keys slots keep every search at load <= 1/2).
 template <class AbiView, class View>
 static int core_view(const AbiView* a, bool n_ok, int64_t keys, bool own_set, bool own_aligned, View& v) {
-	RB_REQUIRE(a->K > 0 && a->K <= 65535 && a->M > 1 && a->N > 0 && n_ok, "bad K / M / N (K <= 65535; N <= 1024 for A*, 2^20 for BFS)");
+	RB_REQUIRE(a->K > 0 && a->K <= 65535 && a->M > 1 && a->N > 0 && n_ok, "bad K / M / N (K <= 65535; N <= 1024 for A*, 2^20 for BFS; M <= 2^27 and max_path >= 1 for MCTS)");
 	RB_REQUIRE(a->states && a->parents && a->parent_actions && a->count && a->won && a->table && a->scratch && own_set, "null buffer in view");
 	RB_REQUIRE_TABLE(a->table, a->capacity);
 	if (a->capacity < 2 * (int64_t)a->K * keys)
-		return rb_fail(RB_ERR_CAPACITY, "table capacity must be at least 2 K M slots for A*, 2 K (M + 12 N) for BFS%s%s");
+		return rb_fail(RB_ERR_CAPACITY, "table capacity must be at least 2 K M slots for A* and MCTS, 2 K (M + 12 N) for BFS%s%s");
 	RB_REQUIRE(aligned(a->scratch, 16) && aligned(a->states, 4) && own_aligned, "misaligned buffer");
 	v.K = a->K; v.M = a->M; v.N = a->N;
 	v.states = a->states; v.parents = a->parents; v.parent_actions = a->parent_actions; v.count = a->count; v.won = a->won;
@@ -635,6 +643,22 @@ static int search_view(const rb_bfs_view* b, rbb::View& v) {
 	v.head = b->head; v.done = b->done; v.solved_parent = b->solved_parent; v.solved_action = b->solved_action;
 	// the children of parents dropped by the budget are claimed before the cut is known: a search holds up to M + 12 N keys
 	return core_view(b, b->N <= (1 << 20), b->M + 12 * (int64_t)b->N, b->head && b->done && b->solved_parent && b->solved_action, true, v);
+}
+
+static int search_view(const rb_mcts_view* m, rbm::View& v) {
+	RB_REQUIRE(m, "null view");
+	struct {                                                   // the Core fields, with N = 1: one leaf per search and step
+		int32_t K, M, N;
+		int8_t* states; int32_t* parents; uint8_t* parent_actions; int32_t* count; uint8_t* won; void* table; int64_t capacity; void* scratch;
+	} a{m->K, m->M, 1, m->states, m->parents, m->parent_actions, m->count, m->won, m->table, m->capacity, m->scratch};
+	v.neighbors = m->neighbors; v.leaves = m->leaves; v.Pv = m->P; v.V = m->V; v.Nv = m->N; v.W = m->W; v.L = m->L;
+	v.solved_index = m->solved_index; v.path_node = m->path_node; v.path_action = m->path_action; v.path_len = m->path_len;
+	v.order = m->order; v.max_path = m->max_path;
+	// discovery keys of the graph shortening, 12 M, stay below 2^31
+	return core_view(&a, m->M <= (1 << 27) && m->max_path >= 1, m->M,
+	                 m->neighbors && m->leaves && m->P && m->V && m->N && m->W && m->L && m->solved_index && m->path_node && m->path_action &&
+	                 m->path_len && m->order,
+	                 aligned(m->neighbors, 4) && aligned(m->P, 4) && aligned(m->V, 4) && aligned(m->N, 4) && aligned(m->W, 4) && aligned(m->L, 4), v);
 }
 
 // state 1 of every search: its root
@@ -756,6 +780,61 @@ int rb_bfs_paths(const rb_bfs_view* b, uint8_t* queues, int32_t* lengths, int32_
 	RB_INIT();
 	rbb::k_paths<<<(v.K + rbl::kThreads - 1) / rbl::kThreads, rbl::kThreads, 0, S(stream)>>>(v, queues, lengths, L);
 	RB_LAUNCHED("bfs_paths");
+	return RB_OK;
+}
+
+// ---- batched MCTS --------------------------------------------------------------------------------------------------------
+int64_t rb_mcts_scratch_bytes(int32_t K) { return scratch_bytes<rbm::View>(K, 1); }
+
+int rb_mcts_init(const rb_mcts_view* m, const int8_t* roots, rb_stream_t stream) { return init_search(m, roots, rbm::k_init, stream); }
+
+int rb_mcts_expand(const rb_mcts_view* m, int8_t* new_states, int32_t* new_search, int32_t* new_index, int32_t* n_new_total,
+                   rb_stream_t stream) {
+	rbm::View v;
+	int rc = search_view(m, v);
+	if (rc != RB_OK) return rc;
+	RB_REQUIRE(new_states && new_search && new_index && n_new_total && aligned(new_states, 4), "null or misaligned output");
+	RB_INIT();
+	cudaStream_t st = S(stream);
+	rc = expand_children(v, n_new_total, st);
+	if (rc != RB_OK) return rc;
+	rbm::k_assign<<<dim3(1, v.K), rbl::kThreads, 0, st>>>(v, new_states, new_search, new_index);
+	RB_LAUNCHED("mcts_assign");
+	return RB_OK;
+}
+
+int rb_mcts_commit(const rb_mcts_view* m, const float* probs, const float* values, const int32_t* new_search, const int32_t* new_index,
+                   const int32_t* n_new_total, double c, int64_t max_states, int32_t* n_active, int32_t* overflow, rb_stream_t stream) {
+	rbm::View v;
+	int rc = search_view(m, v);
+	if (rc != RB_OK) return rc;
+	RB_REQUIRE(probs && values && new_search && new_index && n_new_total && n_active && overflow, "null input or output");
+	RB_REQUIRE(max_states < v.M, "M must exceed max_states (index 0 is unused)");
+	RB_INIT();
+	cudaStream_t st = S(stream);
+	const int64_t worst = 12 * (int64_t)v.K;
+	rbm::k_values<<<(unsigned)((worst + rbl::kThreads - 1) / rbl::kThreads), rbl::kThreads, 0, st>>>(v, probs, values, new_search, new_index,
+	                                                                                                  n_new_total, n_active, overflow);
+	RB_LAUNCHED("mcts_values");
+	rbm::k_walk<<<(v.K + rbm::kWalkWarps - 1) / rbm::kWalkWarps, rbl::kThreads, 0, st>>>(v, c, max_states, n_active, overflow);
+	RB_LAUNCHED("mcts_walk");
+	return RB_OK;
+}
+
+int rb_mcts_finish(const rb_mcts_view* m, int32_t graph, uint8_t* queues, int32_t* lengths, int32_t L, rb_stream_t stream) {
+	rbm::View v;
+	int rc = search_view(m, v);
+	if (rc != RB_OK) return rc;
+	RB_REQUIRE(queues && lengths && L > 0, "null output or L <= 0");
+	RB_INIT();
+	cudaStream_t st = S(stream);
+	if (graph) {
+		const int64_t bx = (12 * (int64_t)v.M + rbl::kThreads - 1) / rbl::kThreads;
+		rbm::k_complete<<<dim3((unsigned)(bx < 64 ? bx : 64), v.K), rbl::kThreads, 0, st>>>(v);
+		RB_LAUNCHED("mcts_complete");
+	}
+	rbm::k_queue<<<v.K, rbl::kThreads, 0, st>>>(v, graph ? 1 : 0, queues, lengths, L);
+	RB_LAUNCHED("mcts_queue");
 	return RB_OK;
 }
 

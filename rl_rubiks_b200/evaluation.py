@@ -8,9 +8,9 @@ solve (-1 unsolved), states explored (`len(agent)`) and seconds per game.
 
 `Evaluator.eval_batched(agent)` draws exactly the same scrambles from the global numpy stream (same order of
 `np.random` calls, evaluation.py:74-76 and cube.py:206-216), then hands ALL cubes of the evaluation to a batched agent
-(`frontier.AStarBatch.search_many` or `frontier.BFSBatch.search_many`) in one call, so that a B200 advances every search
-in lockstep instead of one cube at a time.  A* (given the net) and BFS are deterministic given the start state and a
-`max_states` budget, so `results` and `states` equal the sequential loop's; `times` is the wall time of the batch divided
+(`frontier.AStarBatch`, `frontier.BFSBatch` or `frontier.MCTSBatch`, through `search_many`) in one call, so that a B200
+advances every search in lockstep instead of one cube at a time.  A* and MCTS (given the net) and BFS are deterministic given
+the start state and a `max_states` budget, so `results` and `states` equal the sequential loop's; `times` is the wall time of the batch divided
 evenly.  With one process per GPU the cubes are sharded by rank (searches are independent, no collective on the path) and
 the three arrays gathered at the end.
 """
@@ -84,7 +84,7 @@ class Evaluator:
 		return np.reshape(res, shape), np.reshape(states, shape), np.reshape(times, shape)
 
 	def eval_batched(self, agent, shard: bool = True):
-		"""All cubes of the evaluation in one `agent.search_many(states, max_states)` call (`AStarBatch`, `BFSBatch`; this rank's
+		"""All cubes of the evaluation in one `agent.search_many(states, max_states)` call (`AStarBatch`, `BFSBatch`, `MCTSBatch`; this rank's
 		share of them when a process group is up and `shard` is set).  Requires `max_states` (a wall-clock limit has no batched
 		meaning)."""
 		if not self.max_states:

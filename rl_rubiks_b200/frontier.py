@@ -5,11 +5,12 @@ Python dict keyed on `state.tostring()` (reference: librubiks/solving/agents.py:
 `StateHashSet` is an open-addressing hash set on the packed state in caller-owned (torch) device memory with the
 reference's index semantics: states are numbered 1, 2, ... in insertion order, a batch is numbered in batch order,
 in-batch duplicates resolve to their first occurrence (agents.py:286-306).  `BFS` (layer-synchronous), `BFSBatch` (K
-breadth-first searches in lockstep on the device) and `AStarBatch` (K searches in lockstep, open list and relaxation on the
-device; the two batched agents share their host driver, `_BatchAgent`) carry the reference agents' interface
-(`search(state, time_limit, max_states) -> bool`, `action_queue`, `len(agent)`).  The reference's host-side agent loops
-(single-search A* around a heapq, MCTS' UCB walk) are not part of the product: tests/agent_harness.py replays them around
-`StateHashSet` to check the device primitives against traces recorded from the reference.
+breadth-first searches in lockstep on the device), `AStarBatch` (K searches in lockstep, open list and relaxation on the
+device) and `MCTSBatch` (K Monte Carlo tree searches in lockstep, node arrays and UCB walk on the device; the three batched
+agents share their host driver, `_BatchAgent`) carry the reference agents' interface (`search(state, time_limit, max_states)
+-> bool`, `action_queue`, `len(agent)`).  The reference's single-search host loops (A* around a heapq, MCTS' UCB walk) are
+replayed statement by statement in tests/agent_harness.py around `StateHashSet`, as the test reference of the device
+primitives and the batched agents.
 """
 from __future__ import annotations
 
@@ -547,5 +548,139 @@ class BFSBatch(_BatchAgent):
 		lengths = self.lengths.cpu().numpy()
 		if (lengths < 0).any():
 			raise N.RubiksError(f"an action queue is longer than {self._queue_len} moves")
+		queues = self.queues.cpu().numpy()
+		return won, [queues[s, :lengths[s]].tolist() for s in range(len(won))], count
+
+
+class MCTSBatch(_BatchAgent):
+	"""Monte Carlo tree search (agents.py:415-645) for K cubes at once, entirely on the device (csrc/rb_mcts.cuh): every search
+	expands one leaf per step, and the node arrays, the UCB walk with its virtual loss, the backup and, in graph mode
+	(`search_graph`), the graph completion and the BFS that shortens the action queue are kernels.  The host runs the net on
+	the contiguous batch of new states of all searches (`p, v = net(oh)`, P = `p.softmax(dim=1)`) and reads three counters
+	per step.  Every search equals `MCTS.search` for the same start, net, `c`, `search_graph` and `max_states` node for node
+	(`states`, `neighbors`, `leaves`, `N`, `W`, `V`, `P`; `L` counts the virtual loss in units of nu = 100), found flag,
+	`len(agent)` and action queue.  Both representations, as `AStarBatch`: 6x8x6 rows are rendered only for the net's
+	288-wide one-hot.
+
+	A walk longer than `max_path` moves raises RubiksError.  A step is 6 plain kernel launches (expand: 4, commit: 2): capturing
+	the two halves as CUDA graphs, as A* does, measured no faster (tools/mcts_batch_bench.py), since the net and the host read
+	of each step dominate."""
+
+	def __init__(self, net, c: float, search_graph: bool, is2024: bool | None = None, max_path: int = 1024):
+		super().__init__(is2024)
+		if max_path < 1:
+			raise ValueError("max_path must be at least 1")
+		self.net, self.c, self.search_graph, self.max_path = net, float(c), bool(search_graph), int(max_path)
+
+	def __str__(self):
+		return ("BFS" if self.search_graph else "Naive") + f" MCTS (c={self.c}, batched)"
+
+	@staticmethod
+	def _c_scratch_bytes(K: int, Nx: int):
+		return N.lib.rb_mcts_scratch_bytes(K)
+
+	_c_init = N.lib.rb_mcts_init
+
+	def _alloc(self, K: int, max_states: int):
+		dev = self.dev
+		M = max_states + 1
+		if not self._alloc_core(K, M, 1, M):        # a search stores at most M nodes; every row is written when numbered
+			return
+		self.neighbors = torch.empty(K, M, 12, dtype=torch.int32, device=dev)
+		self.leaves = torch.empty(K, M, dtype=torch.uint8, device=dev)
+		self.P = torch.empty(K, M, 12, dtype=torch.float32, device=dev)
+		self.V = torch.empty(K, M, dtype=torch.float32, device=dev)
+		self.N = torch.empty(K, M, 12, dtype=torch.int32, device=dev)
+		self.W = torch.empty(K, M, 12, dtype=torch.float32, device=dev)
+		self.L = torch.empty(K, M, 12, dtype=torch.int32, device=dev)
+		self.solved_index = torch.zeros(K, dtype=torch.int32, device=dev)
+		self.path_node = torch.zeros(K, self.max_path, dtype=torch.int32, device=dev)
+		self.path_action = torch.zeros(K, self.max_path, dtype=torch.uint8, device=dev)
+		self.path_len = torch.zeros(K, dtype=torch.int32, device=dev)
+		self.order = torch.empty(K, M, dtype=torch.int32, device=dev)
+		self.new_states = torch.empty(12 * K, 20, dtype=torch.int8, device=dev)
+		self.new_search = torch.empty(12 * K, dtype=torch.int32, device=dev)
+		self.new_index = torch.empty(12 * K, dtype=torch.int32, device=dev)
+		self.new_states686 = None if self.is2024 else torch.empty(12 * K, 6, 8, 6, dtype=torch.int8, device=dev)
+		self.oh = torch.empty(12 * K, 480 if self.is2024 else 288, dtype=torch.float32, device=dev)
+		self.probs = torch.zeros(12 * K, 12, dtype=torch.float32, device=dev)       # the net's outputs land here
+		self.values = torch.zeros(12 * K, dtype=torch.float32, device=dev)
+		self.root_search = torch.arange(K, dtype=torch.int32, device=dev)
+		self.root_index = torch.ones(K, dtype=torch.int32, device=dev)
+		self.root_total = torch.full((1,), K, dtype=torch.int32, device=dev)
+		self.queues = torch.zeros(K, self.max_path + 1, dtype=torch.uint8, device=dev)
+		self.lengths = torch.zeros(K, dtype=torch.int32, device=dev)
+		# new states of the step, searches expanding in the next step, walk overflow
+		self.counters = torch.zeros(3, dtype=torch.int32, device=dev)
+		self.counters_host = torch.zeros(3, dtype=torch.int32, pin_memory=True)
+		self.view = N.MCTSView(K, M, self.max_path, *(N.ptr(t) for t in (
+			self.states, self.parents, self.parent_actions, self.neighbors, self.leaves, self.P, self.V, self.N, self.W, self.L, self.count,
+			self.won, self.solved_index, self.path_node, self.path_action, self.path_len, self.order, self.table)), self.capacity, N.ptr(self.scratch))
+
+	def _net_rows(self, src: torch.Tensor, n: int):
+		"""agents.py:470-472, 546-552: the net on the 20-byte rows src[:n]; softmax(policy) and value land in `probs[:n]` and
+		`values[:n]`."""
+		if n == 0:
+			return
+		oh, rep = self.oh[:n], N.REP_2024
+		if not self.is2024:
+			N.check(N.lib.rb_as686(N.ptr(src), N.ptr(self.new_states686), n, N.stream_handle()))
+			src, rep = self.new_states686, N.REP_686
+		N.check(N.lib.rb_as_oh(rep, N.ptr(src), N.ptr(oh), n, N.stream_handle()))
+		p, v = self.net(oh)
+		self.probs[:n].copy_(p.softmax(dim=1))
+		self.values[:n].copy_(v.reshape(-1))
+
+	def _start(self, roots: torch.Tensor, max_states: int):
+		"""Roots, their net call, their P and V and the first walks."""
+		self._max_states = max_states
+		super()._start(roots, max_states)
+		self._net_rows(roots, roots.shape[0])
+		self._commit(self.root_search, self.root_index, self.root_total)
+
+	def _expand(self):
+		N.check(N.lib.rb_mcts_expand(C.byref(self.view), N.ptr(self.new_states), N.ptr(self.new_search), N.ptr(self.new_index),
+									 N.ptr(self.counters[0:1]), N.stream_handle()))
+
+	def _commit(self, search: torch.Tensor, index: torch.Tensor, total: torch.Tensor):
+		N.check(N.lib.rb_mcts_commit(C.byref(self.view), N.ptr(self.probs), N.ptr(self.values), N.ptr(search), N.ptr(index), N.ptr(total), self.c,
+									 self._max_states, N.ptr(self.counters[1:2]), N.ptr(self.counters[2:3]), N.stream_handle()))
+
+	def search_many(self, states, max_states: int, max_steps: int | None = None, time_limit: float | None = None):
+		"""states: (K, *shape) int8 (numpy or CUDA tensor).  Returns (found bool (K,), action queues: list of K lists, len per
+		search int (K,)), the three things `MCTS.search` leaves behind for one cube (len 1 for a solved start).  A search cut
+		off by the budget returns the actions of its last walk."""
+		self.net.eval()
+		return self._run(states, max_states, max_steps, time_limit)
+
+	def search(self, state, time_limit: float = None, max_states: int = None) -> bool:
+		"""`_BatchAgent.search`, with MCTS' len: the nodes stored, 1 for a solved start (agents.py:466-468 store the root first)."""
+		won = super().search(state, time_limit, max_states)
+		self._explored_states = int(self._count[0])
+		return won
+
+	def _check_overflow(self, flag: int):
+		if flag:
+			raise N.RubiksError(f"an MCTS walk needs more than max_path = {self.max_path} moves")
+
+	def _advance(self, max_states: int):
+		self._expand()
+		n_total, n_active, overflow = self._read()
+		self._check_overflow(overflow)
+		if n_active == 0:
+			return False, False
+		self._net_rows(self.new_states, n_total)
+		self._commit(self.new_search, self.new_index, self.counters[0:1])
+		return True, True
+
+	def _results(self):
+		N.check(N.lib.rb_mcts_finish(C.byref(self.view), int(self.search_graph), N.ptr(self.queues), N.ptr(self.lengths), self.max_path + 1,
+									 N.stream_handle()))
+		self._check_overflow(int(self.counters[2].item()))
+		won = self.won.bool().cpu().numpy()
+		self._count = count = self.count.cpu().numpy().astype(int)
+		lengths = self.lengths.cpu().numpy()
+		if (lengths < 0).any():
+			raise N.RubiksError(f"an action queue is longer than {self.max_path + 1} moves")
 		queues = self.queues.cpu().numpy()
 		return won, [queues[s, :lengths[s]].tolist() for s in range(len(won))], count
